@@ -2,6 +2,7 @@
 """Benchmark of the MAFED distillation hot path (fused forward + backward) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C2|C3|C1] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): distill fwd+bwd tokens*layers/sec, and the fraction of HBM peak.
 A "step" is one pass of the hot path (forward over all selected layers, loss algebra, backward) over one
@@ -35,6 +36,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # a run leaves the tree as it found it (it may be read-only): no __pycache__ there
 
 METRIC = "distill fwd+bwd tokens*layers/sec"
 UNIT = "tokens*layers/s"
@@ -342,6 +344,45 @@ def emit(line):
     out.flush()
 
 
+DUMP_GRAD_BYTES = 32 << 20      # budget of the sampled gradient rows; every dump stays under 64 MB
+
+
+def dump_outputs(out_dir, loss, fd, leaves, batch):
+    """Write what the caller of the timed path received from its last step, as ``out_dir/<name>.npy``:
+
+      loss             float64 ()           the returned loss
+      layer_losses     float32 (L,)         the per-layer values the step logs (W&B payload)
+      lang_masks       float32 (B, T)       the masks the step leaves in ``batch``
+      image_masks      float32 (B, T)
+      grad_rows        float32 (L, R, D)    rows ``grad_row_index`` of every distilled layer's gradient, flattened to
+                                            (B*T, D): a fixed sample (seed 0) of R rows, R set by DUMP_GRAD_BYTES
+      grad_row_index   float64 (R,)
+      grad_row_sums    float64 (L, B, T)    the sum over D of every gradient row, so that no element goes unchecked
+
+    The inputs depend only on the arguments, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    L = len(fd.last_layers)
+    grads = [leaves[l].grad for l in fd.last_layers]
+    B, T, D = grads[0].shape
+    rows = min(B * T, max(1, DUMP_GRAD_BYTES // (L * D * 4)))
+    index = torch.randperm(B * T, generator=torch.Generator().manual_seed(0))[:rows].sort().values
+    idx_dev = index.to(grads[0].device)
+    arrays = {
+        "loss": np.asarray(float(loss.detach()), dtype=np.float64),
+        "layer_losses": fd.last_layer_losses[:L].float().cpu().numpy(),
+        "lang_masks": batch["lang_masks"].float().cpu().numpy(),
+        "image_masks": batch["image_masks"].float().cpu().numpy(),
+        "grad_rows": torch.stack([g.reshape(B * T, D)[idx_dev].float() for g in grads]).cpu().numpy(),
+        "grad_row_index": index.double().numpy(),
+        "grad_row_sums": torch.stack([g.double().sum(-1) for g in grads]).cpu().numpy(),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- helpers of the main arm
 class Ctx:
     """Process-wide facts of one bench run."""
@@ -413,7 +454,8 @@ class ApiLoop:
         for s in self.leaves:
             s.grad = None
         n = len(self.masks)
-        loss = fd.distill(self.out, {"attention_mask": self.masks[i % n]})
+        self.batch = {"attention_mask": self.masks[i % n]}
+        loss = fd.distill(self.out, self.batch)
         loss.backward()
         if self.prefetch and fd.process_group is not False:
             fd.prefetch_counts({"attention_mask": self.masks[(i + 2) % n]})
@@ -791,7 +833,11 @@ def main():
     ap.add_argument("--no-other-workloads", action="store_true")
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--e2e-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # plain `python bench.py --gpus N`: relaunch as one process per GPU (what the driver does itself)
         os.dup2(_REAL_STDOUT.fileno(), 1)
@@ -963,6 +1009,8 @@ def run_main(ctx):
     snapshot = (lambda k: peer.trace_into(trace_buf[k])) if peer is not None else None
     sampler = ClockSampler(ctx.local_rank)
     api_ms, host_us, loss = loop.timed(args.steps, args.warmup, sampler, snapshot)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, fd, leaves, loop.batch)
     trace0, trace1 = (trace_buf[0].tolist(), trace_buf[1].tolist()) if peer is not None else (None, None)
     cold_ms = loop.cold_ms_per_step
     start_skew = None

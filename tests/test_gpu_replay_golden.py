@@ -24,12 +24,20 @@ def _golden():
     return z, json.loads(str(z["meta"]))
 
 
+def _generator():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("make_golden_replay", os.path.join(HERE, "golden", "make_golden_replay.py"))
+    gen = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(gen)
+    return gen
+
+
 def _models(z, device):
-    from tiny_vl import TinyVL
-    n_vis = 8
-    student, teacher = TinyVL(n_vis=n_vis, fp32_island=True), TinyVL(n_vis=n_vis, fp32_island=True)
-    student.load_state_dict({k[len("student/"):]: torch.from_numpy(z[k]) for k in z.files if k.startswith("student/")})
-    teacher.load_state_dict({k[len("teacher/"):]: torch.from_numpy(z[k]) for k in z.files if k.startswith("teacher/")})
+    """The two models the goldens were made with, regenerated from their seeds and checked against the stored digests."""
+    gen = _generator()
+    student, teacher = gen.models()
+    assert gen.weights_digest(student) == str(z["student_sha256"]), "regenerated student weights differ from the goldens'"
+    assert gen.weights_digest(teacher) == str(z["teacher_sha256"]), "regenerated teacher weights differ from the goldens'"
     return student.to(device), teacher.to(device).eval()
 
 
@@ -175,14 +183,10 @@ def test_replay_goldens_are_what_the_reference_produces_here():
     from oracle import ref_harness as R
     if not R.available():
         pytest.skip("the reference is not available on this machine")
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("make_golden_replay", os.path.join(HERE, "golden", "make_golden_replay.py"))
-    gen = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(gen)
+    gen = _generator()
     z, meta = _golden()
     student, teacher = gen.models()
-    for k, v in student.state_dict().items():
-        assert np.array_equal(z[f"student/{k}"], v.numpy()), k
+    assert gen.weights_digest(student) == str(z["student_sha256"])
     batch = gen.make_batch(seed=0)
     for case in gen.REPLAY_CASES[:3]:
         fd = gen.make_method(case)
