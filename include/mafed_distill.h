@@ -30,7 +30,7 @@
  * launch; without one the stages are available separately for an NCCL sequence:
  * mafed_distill_fwd | mafed_distill_fused -> mafed_distill_scalar_stage(REDUCE|COUNTS) -> allreduce(sums) ->
  * mafed_distill_scalar_stage(LOSSES|SCALE).
- * The library has no process-global knobs: experiment knobs travel with the call (mafed_shape_t::tuning).  What it
+ * The library has no process-global knobs: the few overrides travel with the call (mafed_shape_t::tuning).  What it
  * remembers between calls is bookkeeping only (per-device attribute caches, the round-robin index of its arrival
  * counters, and which streams a gate was last sent to -- see mafed_distill_bwd).
  */
@@ -67,8 +67,13 @@ enum {
 /* flags of mafed_distill_scalar_stage */
 enum { MAFED_STAGE_REDUCE = 1, MAFED_STAGE_COUNTS = 2, MAFED_STAGE_LOSSES = 4, MAFED_STAGE_SCALE = 8 };
 
-/* Experiment knobs of ONE call (benchmarks and A/B measurements; keys in mafed_b200/cabi.py).  All zero = the
- * library's defaults, which is also what a NULL mafed_shape_t::tuning means. */
+/* Overrides of ONE call, for tests and benchmarks that compare a default launch with another form of it.  All zero =
+ * the library's defaults, which is also what a NULL mafed_shape_t::tuning means.  Three indices of v are read; every
+ * other index is ignored (the layout is kept for callers built against earlier versions of this header):
+ *   v[MAFED_TUNE_NO_TAIL]     1: the losses come from a separate scalar-stage launch instead of the last CTA
+ *   v[MAFED_TUNE_VARIANT_ALL] kernel family of every pass: 1 register-staged (LDG), 2 TMA ring (0: default)
+ *   v[MAFED_TUNE_NO_GATE]     1: the backward fix-up is a full grid whose CTAs return at once instead of a gate */
+enum { MAFED_TUNE_NO_TAIL = 17, MAFED_TUNE_VARIANT_ALL = 18, MAFED_TUNE_NO_GATE = 19 };
 typedef struct mafed_tuning {
   int32_t v[24];
 } mafed_tuning_t;

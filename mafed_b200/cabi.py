@@ -17,16 +17,11 @@ VARIANT_DEFAULT, VARIANT_LDG, VARIANT_TMA = 0, 1, 2
 STAGE_REDUCE, STAGE_COUNTS, STAGE_LOSSES, STAGE_SCALE = 1, 2, 4, 8
 COMM_SUMS, COMM_COUNTS = 1, 2
 ABI_VERSION = 4
-# keys of mafed_tuning_t (benchmark knobs of ONE call); the first three are per pass: key + PASS_*
-PASS_FWD, PASS_BWD, PASS_FUSED = 0, 1, 2
-TUNE_TMA_STAGES, TUNE_TMA_ROWS, TUNE_VARIANT = 0, 3, 6
-TUNE_TMA_WARPS, TUNE_LDG_BLOCKS_PER_SM, TUNE_BWD_FORWARD_ORDER, TUNE_GRID_MUL = 9, 10, 11, 12
-TUNE_LOAD_POLICY, TUNE_STORE_POLICY = 13, 14   # 0 none, 1 evict_first, 2 evict_last, 3 evict_normal
-TUNE_NO_PDL = 15
-TUNE_NO_INLINE_SCALE, TUNE_NO_TAIL = 16, 17   # 1: separate prologue launch / separate epilogue launch
-TUNE_VARIANT_ALL = 18                          # kernel family of every pass: 1 ldg, 2 tma (0 = default)
-TUNE_NO_GATE = 19                              # 1: backward fix-up as a full grid that returns at once (round-1 form)
-TUNE_PACE_NS = 20                              # TMA producer: nanoseconds between a free slot and its refill (experiment)
+# indices of mafed_tuning_t::v the library reads (MAFED_TUNE_* of the header; it ignores every other index)
+TUNE_NO_TAIL = 17       # 1: separate epilogue launch instead of the in-kernel tail
+TUNE_VARIANT_ALL = 18   # kernel family of every pass: 1 ldg, 2 tma (0 = default)
+TUNE_NO_GATE = 19       # 1: backward fix-up as a full grid that returns at once (round-1 form)
+TUNE_KEYS = {"TUNE_NO_TAIL": TUNE_NO_TAIL, "TUNE_VARIANT_ALL": TUNE_VARIANT_ALL, "TUNE_NO_GATE": TUNE_NO_GATE}
 N_TUNE_KEYS = 24
 
 # MAFED_B200_LIB: another build of the same C ABI (A/B measurements of two kernel versions, tools/ab_lib.py)
@@ -58,7 +53,7 @@ class Shape(ctypes.Structure):
                [("tuning", ctypes.POINTER(Tuning))]
 
 
-# Experiment knobs travel with each call (mafed_shape_t::tuning); the library itself keeps no mutable state.
+# Overrides travel with each call (mafed_shape_t::tuning); the library itself keeps no mutable state.
 # Benchmarks and tests install a Tuning for the calls made inside a `with cabi.tuning(...)` block of THIS process.
 _active_tuning = None
 
@@ -70,19 +65,19 @@ def active_tuning_address() -> int:
 
 @contextlib.contextmanager
 def tuning(variant: int = 0, **keys):
-    """``with cabi.tuning(variant=cabi.VARIANT_LDG, TUNE_NO_TAIL=1): ...`` -- knobs for the calls inside the block.
-    Keys are the TUNE_* names of this module (or integers via ``raw={key: value}``)."""
+    """``with cabi.tuning(variant=cabi.VARIANT_LDG, TUNE_NO_TAIL=1): ...`` -- overrides for the calls inside the block.
+    Keys are the names of TUNE_KEYS; any other keyword raises TypeError."""
     global _active_tuning
+    unknown = sorted(set(keys) - set(TUNE_KEYS))
+    if unknown:
+        raise TypeError(f"unknown tuning key(s) {unknown}; the library reads {sorted(TUNE_KEYS)}")
     t = Tuning()
     if _active_tuning is not None:
         ctypes.memmove(ctypes.addressof(t), ctypes.addressof(_active_tuning), ctypes.sizeof(Tuning))
     if variant:
         t.v[TUNE_VARIANT_ALL] = int(variant)
-    raw = keys.pop("raw", None) or {}
     for name, value in keys.items():
-        t.v[globals()[name]] = int(value)
-    for key, value in raw.items():
-        t.v[int(key)] = int(value)
+        t.v[TUNE_KEYS[name]] = int(value)
     prev, _active_tuning = _active_tuning, t
     try:
         yield t

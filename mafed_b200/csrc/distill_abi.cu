@@ -19,14 +19,9 @@ namespace {
 
 // May this launch be a programmatic dependent of its predecessor in `stream`?  Not right behind a gate
 // (distill_gate.cu: the gate may have started a backward from the device that needs the SMs first).
-bool pdl_allowed(const mafed_shape_t& sh, void* stream) {
-  const bool after_gate = mafed_gate::consume_gate_mark(stream);
-  return tune(sh, kTuneNoPdl) == 0 && !after_gate;
-}
+bool pdl_allowed(void* stream) { return !mafed_gate::consume_gate_mark(stream); }
 
-HostLaunch host_launch(const mafed_shape_t& sh, void* stream) {
-  return HostLaunch{(cudaStream_t)stream, pdl_allowed(sh, stream)};
-}
+HostLaunch host_launch(void* stream) { return HostLaunch{(cudaStream_t)stream, pdl_allowed(stream)}; }
 
 // Arrival counters of the in-kernel tail (distill_tma.cuh).  A counter is zero whenever no kernel is using it
 // (the last CTA resets it), so launches take them round-robin: two kernels can only share one if 128 tailed
@@ -116,7 +111,7 @@ int launch_scalar_stage(const mafed_shape_t& sh, const mafed_weights_t* w, int f
   e.a.loss_kind = sh.loss_kind;
   e.a.flags = flags;
   if (w != nullptr) e.w = *w;
-  launch_pdl(k_epilogue, 1, kEpiThreads, 0, st, pdl_allowed(sh, st), e);
+  launch_pdl(k_epilogue, 1, kEpiThreads, 0, st, pdl_allowed(st), e);
   return (int)cudaPeekAtLastError();
 }
 
@@ -143,10 +138,9 @@ int fused_impl(const mafed_shape_t* shape, const void* const* student_ptrs, cons
   p.ws = reinterpret_cast<float*>(ws);
   const bool sharded = comm != nullptr && comm->world > 1;
   const bool tma = uses_tma(*shape, p, kPassFused);
-  const bool want_tail = tail != nullptr && weights != nullptr && tma && !tune(*shape, kTuneNoTail);
+  const bool want_tail = tail != nullptr && weights != nullptr && tma && !tune(*shape, MAFED_TUNE_NO_TAIL);
   // with a ticket nobody sums the mask inside the streaming kernel, so the mask size does not matter
-  const bool want_inline = weights != nullptr && tma && !tune(*shape, kTuneNoInlineScale) &&
-                           (counts_ticket != nullptr || mask_entries(*shape) <= 16384);
+  const bool want_inline = weights != nullptr && tma && (counts_ticket != nullptr || mask_entries(*shape) <= 16384);
   // The arrival counter: needed for the tail and, in a sharded step without a ticket, for the in-kernel counts
   // exchange (the last CTA advances the device-side epoch).
   unsigned int* done = nullptr;
@@ -185,7 +179,7 @@ int fused_impl(const mafed_shape_t* shape, const void* const* student_ptrs, cons
       if (rc) return rc;
     }
   }
-  return dispatch<kPassFused>(*shape, p, host_launch(*shape, stream));
+  return dispatch<kPassFused>(*shape, p, host_launch(stream));
 }
 
 }  // namespace
@@ -224,7 +218,7 @@ int mafed_distill_fwd(const mafed_shape_t* shape, const void* const* student_ptr
   if (rc) return rc;
   if (!ws) return MAFED_E_ARG;
   p.ws = reinterpret_cast<float*>(ws);
-  return dispatch<kPassFwd>(*shape, p, host_launch(*shape, stream));
+  return dispatch<kPassFwd>(*shape, p, host_launch(stream));
 }
 
 int mafed_distill_token_norm_sums(const mafed_shape_t* shape, const void* const* tensor_ptrs, const int64_t* attn_mask,
@@ -235,7 +229,7 @@ int mafed_distill_token_norm_sums(const mafed_shape_t* shape, const void* const*
   if (!ws) return MAFED_E_ARG;
   p.ws = reinterpret_cast<float*>(ws);
   p.single_input = 1;
-  return dispatch<kPassFwd>(*shape, p, host_launch(*shape, stream), kLossL2Norm);
+  return dispatch<kPassFwd>(*shape, p, host_launch(stream), kLossL2Norm);
 }
 
 int mafed_distill_scalar_stage(const mafed_shape_t* shape, const mafed_weights_t* weights, int flags,
@@ -367,7 +361,7 @@ int mafed_distill_prefetch_counts(const mafed_shape_t* shape, const int64_t* att
   pp.n_vis_rows = vis_rows(*shape);
   pp.ticket = reinterpret_cast<long long*>(ticket);
   pp.comm = comm_dev(comm);
-  launch_pdl(k_prefetch_counts, 1, kEpiThreads, 0, (cudaStream_t)stream, pdl_allowed(*shape, stream), pp);
+  launch_pdl(k_prefetch_counts, 1, kEpiThreads, 0, (cudaStream_t)stream, pdl_allowed(stream), pp);
   return (int)cudaPeekAtLastError();
 }
 
@@ -375,26 +369,25 @@ int mafed_distill_bwd(const mafed_shape_t* shape, const void* const* student_ptr
                       void* const* grad_ptrs, const int64_t* attn_mask, const float* bwd_scale, const float* grad_out,
                       float grad_out_scale, const float* skip_if_equals, float* grad_out_seen, void* stream) {
   if (!grad_ptrs || !bwd_scale) return MAFED_E_ARG;
-  if (skip_if_equals != nullptr && !tune(*shape, kTuneNoGate)) {
+  int rc = check_shape(shape);
+  if (rc) return rc;
+  if (skip_if_equals != nullptr && !tune(*shape, MAFED_TUNE_NO_GATE)) {
     // the one-pass step's gate: a 1-CTA launch that starts the backward from the device only if it is needed
     // (distill_gate.cu, the relocatable-device-code unit of the library)
-    int rc = check_shape(shape);
-    if (rc) return rc;
     return mafed_gate::gated_backward(shape, student_ptrs, teacher_ptrs, grad_ptrs, attn_mask, bwd_scale, grad_out,
                                       grad_out_scale, *skip_if_equals, grad_out_seen, stream);
   }
   PathParams p;
-  int rc = fill_params(shape, student_ptrs, teacher_ptrs, grad_ptrs, attn_mask, p);
+  rc = fill_params(shape, student_ptrs, teacher_ptrs, grad_ptrs, attn_mask, p);
   if (rc) return rc;
   p.bwd_scale = bwd_scale;
   p.grad_out = grad_out;
   p.gout_scale = grad_out_scale;
-  if (skip_if_equals != nullptr) {   // kTuneNoGate: the round-1 form, a full grid whose CTAs return at once
+  if (skip_if_equals != nullptr) {   // MAFED_TUNE_NO_GATE: the round-1 form, a full grid whose CTAs return at once
     p.skip_if_gout_equals = 1;
     p.fixed_gout = *skip_if_equals;
   }
-  p.reverse = tune(*shape, kTuneBwdForward) ? 0 : 1;
-  return dispatch<kPassBwd>(*shape, p, host_launch(*shape, stream));
+  return dispatch<kPassBwd>(*shape, p, host_launch(stream));
 }
 
 int mafed_distill_fused(const mafed_shape_t* shape, const void* const* student_ptrs, const void* const* teacher_ptrs,
@@ -444,7 +437,7 @@ int mafed_distill_fwd_step(const mafed_shape_t* shape, const void* const* studen
   p.ws = reinterpret_cast<float*>(ws);
   const int flags = MAFED_STAGE_REDUCE | MAFED_STAGE_COUNTS | MAFED_STAGE_LOSSES | (bwd_scale ? MAFED_STAGE_SCALE : 0);
   unsigned int* done = nullptr;
-  if (!tune(*shape, kTuneNoTail) && uses_tma(*shape, p, kPassFwd)) done = next_tail_counter((cudaStream_t)stream);
+  if (!tune(*shape, MAFED_TUNE_NO_TAIL) && uses_tma(*shape, p, kPassFwd)) done = next_tail_counter((cudaStream_t)stream);
   if (done != nullptr) {
     p.tail_flags = flags;
     p.tail_done = done;
@@ -459,9 +452,9 @@ int mafed_distill_fwd_step(const mafed_shape_t* shape, const void* const* studen
       p.comm = comm_dev(comm);
       p.tail_comm = 1;
     }
-    return dispatch<kPassFwd>(*shape, p, host_launch(*shape, stream));
+    return dispatch<kPassFwd>(*shape, p, host_launch(stream));
   }
-  rc = dispatch<kPassFwd>(*shape, p, host_launch(*shape, stream));
+  rc = dispatch<kPassFwd>(*shape, p, host_launch(stream));
   if (rc) return rc;
   return launch_scalar_stage(*shape, weights, flags, attn_mask, ws, sums, out, bwd_scale, (cudaStream_t)stream,
                              sharded ? comm : nullptr, MAFED_COMM_SUMS | MAFED_COMM_COUNTS);
@@ -474,7 +467,7 @@ int mafed_distill_modality_masks(const mafed_shape_t* shape, const int64_t* attn
   if (!lang_mask || !image_mask || (needs_mask(*shape) && !attn_mask)) return MAFED_E_ARG;
   const long long n = (long long)shape->B * shape->T;
   const unsigned grid = (unsigned)clamp_grid((n + 255) / 256, 1 << 20);
-  launch_pdl(k_modality_masks, grid > 1184 ? 1184u : grid, 256, 0, (cudaStream_t)stream, pdl_allowed(*shape, stream),
+  launch_pdl(k_modality_masks, grid > 1184 ? 1184u : grid, 256, 0, (cudaStream_t)stream, pdl_allowed(stream),
              attn_mask, lang_mask, image_mask, n, (int)shape->T, (int)shape->n_vis);
   return (int)cudaPeekAtLastError();
 }

@@ -59,7 +59,6 @@ struct PathParams {
   int txt;                       // T - n_vis
   int D;
   int n_chunks;                  // 16-byte chunks per row (vector kernels)
-  int reverse;                   // backward: walk work items last-to-first (L2 reuse after forward)
   float fixed_gout;              // fused pass: upstream gradient assumed at forward time (host value)
   float gout_scale;              // backward: host factor on *grad_out (e.g. world_size to undo DDP's averaging)
   int skip_if_gout_equals;       // backward fix-up: return at once when *grad_out == fixed_gout
@@ -77,8 +76,6 @@ struct PathParams {
   int comm_counts;               // 1: exchange the counts in this kernel (epoch = device-side counter + 1)
   const long long* counts_ticket;  // counts sent ahead of the step (k_prefetch_counts): {epoch, bits(n_text), bits(n_vis rows)}
   CommDev comm;
-  int load_policy;               // L2 eviction hint for student/teacher reads (CachePolicy)
-  int store_policy;              // L2 eviction hint for gradient writes
   // In-kernel tail (TMA kernels): the last CTA to finish runs the scalar stage on the partial sums, so the step
   // needs no epilogue launch.  Needs w / loss_kind / n_mask / n_vis_rows above (and comm for a sharded step).
   int tail_flags;                // 0: no tail; else EpiFlags of the stage to run
@@ -92,17 +89,6 @@ struct PathParams {
   int64_t* lang_mask_out;
   int64_t* image_mask_out;
 };
-
-// L2 eviction-priority hints (createpolicy); kPolicyNone issues the plain instruction.
-enum CachePolicy { kPolicyNone = 0, kPolicyEvictFirst = 1, kPolicyEvictLast = 2, kPolicyEvictNormal = 3 };
-
-__device__ __forceinline__ uint64_t make_policy(int kind) {
-  uint64_t pol = 0;
-  if (kind == kPolicyEvictFirst) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  else if (kind == kPolicyEvictLast) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  else if (kind == kPolicyEvictNormal) asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
 
 // What a "backward-shaped" kernel does: kBackward writes gradients only; kFused also accumulates
 // the loss sums in the same pass over student and teacher (3*D*e bytes per token*layer instead of 5).
@@ -196,19 +182,6 @@ __device__ __forceinline__ uint4 ldg_stream(const void* p) {
 __device__ __forceinline__ void stg_128(void* p, const uint4& v) {
   asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};"
                :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-// Variants carrying an L2 eviction hint (`kind` is warp-uniform; kPolicyNone -> the plain instruction).
-__device__ __forceinline__ uint4 ldg_stream(const void* p, int kind, uint64_t pol) {
-  if (kind == kPolicyNone) return ldg_stream(p);
-  uint4 r;
-  asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;"
-               : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(pol));
-  return r;
-}
-__device__ __forceinline__ void stg_128(void* p, const uint4& v, int kind, uint64_t pol) {
-  if (kind == kPolicyNone) { stg_128(p, v); return; }
-  asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1, %2, %3, %4}, %5;"
-               :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "l"(pol) : "memory");
 }
 
 // ---------------------------------------------------------------- programmatic dependent launch

@@ -5,7 +5,7 @@
 // kernel is started is a `Launcher` policy: HostLaunch enqueues it on the stream, GateLaunch (distill_gate.cu)
 // enqueues a gate that starts it from the device only when it has work to do.
 //
-// Nothing here is process-global: experiment knobs arrive per call (mafed_shape_t::tuning) and the caches of
+// Nothing here is process-global: overrides arrive per call (mafed_shape_t::tuning) and the caches of
 // occupancy / opt-in shared memory are per kernel and per device.
 #pragma once
 #include <cstring>
@@ -19,12 +19,7 @@ namespace MAFED_NS {
 enum Pass { kPassFwd = 0, kPassBwd = 1, kPassFused = 2 };
 constexpr int kMaxDevices = 64;
 
-// keys of mafed_tuning_t::v (see include/mafed_distill.h); the first three are per pass: key + Pass
-enum TuneKey { kTuneTmaStages = 0, kTuneTmaRows = 3, kTuneVariant = 6, kTuneTmaWarps = 9, kTuneLdgBlocksPerSm = 10,
-               kTuneBwdForward = 11, kTuneGridMul = 12, kTuneLoadPolicy = 13, kTuneStorePolicy = 14, kTuneNoPdl = 15,
-               kTuneNoInlineScale = 16, kTuneNoTail = 17, kTuneVariantAll = 18, kTuneNoGate = 19,
-               kTunePaceNs = 20 };
-
+// key: MAFED_TUNE_* (include/mafed_distill.h)
 inline int tune(const mafed_shape_t& sh, int key) { return sh.tuning != nullptr ? sh.tuning->v[key] : 0; }
 
 // Launch with programmatic dependent launch enabled: the kernel may start its prologue while its
@@ -186,20 +181,20 @@ struct LdgKernel<T, CPL, RPI, LOSS, kPassFused> {
   static auto host() { return &k_bwd_ldg<T, CPL, RPI, LOSS, kFused>; }
 };
 
-template <typename T, int LOSS, int NCW, int PASS>
+template <typename T, int LOSS, int PASS>
 struct TmaKernel;
-template <typename T, int LOSS, int NCW>
-struct TmaKernel<T, LOSS, NCW, kPassFwd> {
-  static auto host() { return &k_fwd_tma<T, LOSS, NCW>; }
+template <typename T, int LOSS>
+struct TmaKernel<T, LOSS, kPassFwd> {
+  static auto host() { return &k_fwd_tma<T, LOSS>; }
 };
-template <typename T, int LOSS, int NCW>
-struct TmaKernel<T, LOSS, NCW, kPassBwd> {
-  static auto host() { return &k_bwd_tma<T, LOSS, NCW, kBackward>; }
-  MAFED_TAIL_LAUNCH(k_bwd_tma<T, LOSS, NCW, kBackward>)
+template <typename T, int LOSS>
+struct TmaKernel<T, LOSS, kPassBwd> {
+  static auto host() { return &k_bwd_tma<T, LOSS, kBackward>; }
+  MAFED_TAIL_LAUNCH(k_bwd_tma<T, LOSS, kBackward>)
 };
-template <typename T, int LOSS, int NCW>
-struct TmaKernel<T, LOSS, NCW, kPassFused> {
-  static auto host() { return &k_bwd_tma<T, LOSS, NCW, kFused>; }
+template <typename T, int LOSS>
+struct TmaKernel<T, LOSS, kPassFused> {
+  static auto host() { return &k_bwd_tma<T, LOSS, kFused>; }
 };
 
 template <typename T, int LOSS>
@@ -213,35 +208,32 @@ struct GenericBwdKernel {
 };
 
 template <typename T, int CPL, int RPI, int LOSS, int PASS, typename Launcher>
-int launch_ldg(const mafed_shape_t& sh, const PathParams& p, const Launcher& go) {
+int launch_ldg(const PathParams& p, const Launcher& go) {
   static_assert(LOSS != kLossL2Norm || PASS == kPassFwd, "the token-norm reduction has no backward");
   using Kernel = LdgKernel<T, CPL, RPI, LOSS, PASS>;
   static int occ[kMaxDevices] = {};   // per kernel and per device
   const DeviceInfo& dv = device_info();
   if (occ[dv.index] == 0) occ[dv.index] = blocks_per_sm(Kernel::host(), kLdgThreads, 0);
-  int per_sm = occ[dv.index];
-  const int cap = tune(sh, kTuneLdgBlocksPerSm);
-  if (cap > 0 && cap < per_sm) per_sm = cap;
   const long long rows_per_iter = (long long)kLdgWarps * RPI;
   const long long total = ((p.n_rows + rows_per_iter - 1) / rows_per_iter) * p.n_layers;
-  const unsigned grid = (unsigned)clamp_grid((long long)dv.sm_count * per_sm, total);
+  const unsigned grid = (unsigned)clamp_grid((long long)dv.sm_count * occ[dv.index], total);
   go.template run<Kernel>(grid, kLdgThreads, 0, p);
   return (int)cudaPeekAtLastError();
 }
 
 template <typename T, int LOSS, int PASS, typename Launcher>
-int dispatch_ldg(const mafed_shape_t& sh, const PathParams& p, const Launcher& go) {
+int dispatch_ldg(const PathParams& p, const Launcher& go) {
   const int cpl = (p.n_chunks + 31) / 32;
   // rows per warp per iteration: more independent loads in flight for short rows; the cosine gradient keeps the row
   // statistics and two coefficients per row as well, so it takes half as many rows at a time (with 4 / 2 it spilled
   // 150-250 bytes per thread under the 128-register cap)
   constexpr bool kHeavy = LOSS == MAFED_LOSS_COSINE && PASS != kPassFwd;
-  if (cpl <= 1) return launch_ldg<T, 1, kHeavy ? 2 : 4, LOSS, PASS>(sh, p, go);
-  if (cpl <= 2) return launch_ldg<T, 2, kHeavy ? 2 : 4, LOSS, PASS>(sh, p, go);
-  if (cpl <= 3) return launch_ldg<T, 3, kHeavy ? 1 : 2, LOSS, PASS>(sh, p, go);
-  if (cpl <= 4) return launch_ldg<T, 4, kHeavy ? 1 : 2, LOSS, PASS>(sh, p, go);
-  if (cpl <= 6) return launch_ldg<T, 6, 1, LOSS, PASS>(sh, p, go);
-  return launch_ldg<T, 8, 1, LOSS, PASS>(sh, p, go);  // multi-pass for rows longer than 4 KB
+  if (cpl <= 1) return launch_ldg<T, 1, kHeavy ? 2 : 4, LOSS, PASS>(p, go);
+  if (cpl <= 2) return launch_ldg<T, 2, kHeavy ? 2 : 4, LOSS, PASS>(p, go);
+  if (cpl <= 3) return launch_ldg<T, 3, kHeavy ? 1 : 2, LOSS, PASS>(p, go);
+  if (cpl <= 4) return launch_ldg<T, 4, kHeavy ? 1 : 2, LOSS, PASS>(p, go);
+  if (cpl <= 6) return launch_ldg<T, 6, 1, LOSS, PASS>(p, go);
+  return launch_ldg<T, 8, 1, LOSS, PASS>(p, go);  // multi-pass for rows longer than 4 KB
 }
 
 // Any D / any alignment: element-wise kernels.  The fused pass is simply forward then backward.
@@ -261,61 +253,49 @@ inline bool tma_geometry(const mafed_shape_t& sh, const PathParams& p, int pass,
   const long long row_bytes = (long long)p.n_chunks * 16;
   if (row_bytes > 32768) return false;
   const long long budget = (long long)dv.smem_optin - 16 * 1024;  // static smem + slack
-  int rows = tune(sh, kTuneTmaRows + pass);
-  const bool rows_default = rows <= 0, stages_default = tune(sh, kTuneTmaStages + pass) <= 0;
-  bool cosine_fine = false, fused_fine = false, wide = false;
-  if (rows <= 0) {
-    // Measured on B200 (profiles/r02l_geometry_sweep.txt: one-pass step, 13 shapes x 13 rings; r02q_geometry_sweep_
-    // {fwd,bwd}.txt: the two passes; all after the producer stopped paying 64-bit divisions and the mask round trip
-    // per tile).  What the memory system is sensitive to is the number of bytes in flight per SM:
-    //  * forward pass (reads only): 2 stages x 96 KB -- best or within 2 % for every shape; ragged long text +13 %
-    //    and cosine +5 % over 2 x 72 KB.
-    //  * passes that also write the gradient (backward, one-pass step): 3 stages x 32 KB (96 KB in flight) is the best
-    //    or within 2.5 % of it for every shape of 256 visual + ~32 text rows (base / 410M / 1B, bf16 and fp32, 16..256
-    //    samples), 5-12 % ahead of 2 x 64 KB; 64 KB in flight is latency-bound (+20 %), 128 KB and more queue up in
-    //    the memory system (+5-13 %).
-    //  * the cosine gradient needs two sweeps over a row with a warp reduction in between, so a stage drains more
-    //    slowly: 4 stages x 32 KB keep more rows in different phases at once.
-    //  * text-heavy batches (more than a quarter of the rows behind the attention mask, where ragged masks make
-    //    whole tiles zero-fill only) keep the coarse ring, 2 x 64-72 KB: fewer, larger tiles amortise the per-tile
-    //    cost of the padded ones (3 x 32 KB is 4-16 % behind there).
-    const bool text_heavy = (long long)(sh.T - sh.n_vis) * 4 > (long long)sh.T;
-    wide = pass == kPassFwd;
-    cosine_fine = !wide && loss == MAFED_LOSS_COSINE;
-    fused_fine = !wide && !cosine_fine && !text_heavy;
-    const long long stage_target = wide ? 96 * 1024 : ((cosine_fine || fused_fine) ? 32 * 1024 : 72 * 1024);
-    rows = (int)(stage_target / (2 * row_bytes));
-    if (rows >= 8 && !wide && !cosine_fine && !fused_fine) rows &= ~7;
-  }
+  // Measured on B200 (profiles/r02l_geometry_sweep.txt: one-pass step, 13 shapes x 13 rings; r02q_geometry_sweep_
+  // {fwd,bwd}.txt: the two passes; all after the producer stopped paying 64-bit divisions and the mask round trip
+  // per tile).  What the memory system is sensitive to is the number of bytes in flight per SM:
+  //  * forward pass (reads only): 2 stages x 96 KB -- best or within 2 % for every shape; ragged long text +13 %
+  //    and cosine +5 % over 2 x 72 KB.
+  //  * passes that also write the gradient (backward, one-pass step): 3 stages x 32 KB (96 KB in flight) is the best
+  //    or within 2.5 % of it for every shape of 256 visual + ~32 text rows (base / 410M / 1B, bf16 and fp32, 16..256
+  //    samples), 5-12 % ahead of 2 x 64 KB; 64 KB in flight is latency-bound (+20 %), 128 KB and more queue up in
+  //    the memory system (+5-13 %).
+  //  * the cosine gradient needs two sweeps over a row with a warp reduction in between, so a stage drains more
+  //    slowly: 4 stages x 32 KB keep more rows in different phases at once.
+  //  * text-heavy batches (more than a quarter of the rows behind the attention mask, where ragged masks make
+  //    whole tiles zero-fill only) keep the coarse ring, 2 x 64-72 KB: fewer, larger tiles amortise the per-tile
+  //    cost of the padded ones (3 x 32 KB is 4-16 % behind there).
+  const bool text_heavy = (long long)(sh.T - sh.n_vis) * 4 > (long long)sh.T;
+  const bool wide = pass == kPassFwd;
+  const bool cosine_fine = !wide && loss == MAFED_LOSS_COSINE;
+  const bool fused_fine = !wide && !cosine_fine && !text_heavy;
+  const long long stage_target = wide ? 96 * 1024 : ((cosine_fine || fused_fine) ? 32 * 1024 : 72 * 1024);
+  int rows = (int)(stage_target / (2 * row_bytes));
+  if (rows >= 8 && !wide && !cosine_fine && !fused_fine) rows &= ~7;
   if (rows > kTmaMaxRows) rows = kTmaMaxRows;
   if (rows < 1) rows = 1;
   if (2 * rows * row_bytes > budget) rows = (int)(budget / (2 * row_bytes));
   if (rows < 1) return false;
   geo.rows = rows;
   geo.stage_bytes = (int)(2 * rows * row_bytes);
-  int stages = tune(sh, kTuneTmaStages + pass);
-  if (stages <= 0) stages = cosine_fine ? 4 : (fused_fine ? 3 : ((wide || 2 * geo.stage_bytes >= 96 * 1024) ? 2 : 3));
+  int stages = cosine_fine ? 4 : (fused_fine ? 3 : ((wide || 2 * geo.stage_bytes >= 96 * 1024) ? 2 : 3));
   if (stages > kTmaMaxStages) stages = kTmaMaxStages;
   while (stages > 1 && (long long)stages * geo.stage_bytes > budget) --stages;
   geo.stages = stages;
   // Refill pacing (profiles/r02n_pace_sweep.txt).  The coarse ring of a text-heavy one-pass step, every row live:
   // 0.96 ms refilled at once, 0.90 ms with ~0.5 us between a free slot and its refill (in-flight bytes per SM are
   // what the memory system is sensitive to); with a ragged mask the same pause costs 4 %, so the producer drops it
-  // at the first padded row it meets.  kTunePaceNs: > 0 explicit (unconditional), < 0 off.
-  const int pace = tune(sh, kTunePaceNs);
-  geo.pace_ns = pace > 0 ? pace : 0;
-  geo.pace_dense = 0;
-  if (pace == 0 && pass != kPassFwd && !fused_fine && !cosine_fine && rows_default && stages_default) {
-    geo.pace_ns = 500;
-    geo.pace_dense = 1;
-  }
+  // at the first padded row it meets.
+  geo.pace = pass != kPassFwd && !fused_fine && !cosine_fine;
   return true;
 }
 
-template <typename T, int LOSS, int NCW, int PASS, typename Launcher>
-int launch_tma(const mafed_shape_t& sh, const PathParams& p, const TmaGeom& geo, const Launcher& go) {
+template <typename T, int LOSS, int PASS, typename Launcher>
+int launch_tma(const PathParams& p, const TmaGeom& geo, const Launcher& go) {
   static_assert(LOSS != kLossL2Norm || PASS == kPassFwd, "the token-norm reduction has no backward");
-  using Kernel = TmaKernel<T, LOSS, NCW, PASS>;
+  using Kernel = TmaKernel<T, LOSS, PASS>;
   // the opt-in shared-memory size is a per-device function attribute: remember it per kernel and device
   static bool attr_set[kMaxDevices] = {};
   const DeviceInfo& dv = device_info();
@@ -326,10 +306,8 @@ int launch_tma(const mafed_shape_t& sh, const PathParams& p, const TmaGeom& geo,
     attr_set[dv.index] = true;
   }
   const long long total = ((p.n_rows + geo.rows - 1) / geo.rows) * p.n_layers;
-  int mul = tune(sh, kTuneGridMul);
-  if (mul <= 0) mul = 1;
-  const unsigned grid = (unsigned)clamp_grid((long long)dv.sm_count * mul, total);
-  go.template run<Kernel>(grid, (NCW + 1) * 32, dyn, p, geo);
+  const unsigned grid = (unsigned)clamp_grid((long long)dv.sm_count, total);   // one persistent CTA per SM
+  go.template run<Kernel>(grid, kTmaConsumerThreads + 32, dyn, p, geo);   // + the producer warp
   return (int)cudaPeekAtLastError();
 }
 
@@ -342,25 +320,19 @@ inline bool vector_path(const mafed_shape_t& sh, const PathParams& p, int pass) 
   return ok;
 }
 
-inline int chosen_variant(const mafed_shape_t& sh, int pass) {
-  int variant = tune(sh, kTuneVariant + pass);
-  if (variant == 0) variant = tune(sh, kTuneVariantAll);
+inline int chosen_variant(const mafed_shape_t& sh) {
+  const int variant = tune(sh, MAFED_TUNE_VARIANT_ALL);
   return variant == 0 ? 2 : variant;   // 1 ldg, 2 tma (default)
 }
 
 template <typename T, int LOSS, int PASS, typename Launcher>
 int dispatch_typed(const mafed_shape_t& sh, PathParams& p, bool vector_ok, const Launcher& go) {
   if (!vector_ok) return launch_generic<T, LOSS, PASS>(sh, p, go);
-  if (chosen_variant(sh, PASS) == 2) {
+  if (chosen_variant(sh) == 2) {
     TmaGeom geo;
-    if (tma_geometry(sh, p, PASS, geo, LOSS)) {
-      // 16 consumer warps: two stages are drained concurrently when a stage holds <= 8 rows (+2.6 % on the
-      // 1B shape, neutral elsewhere; profiles/r01_call4_sweep_extra.json)
-      if (tune(sh, kTuneTmaWarps) == 8) return launch_tma<T, LOSS, 8, PASS>(sh, p, geo, go);
-      return launch_tma<T, LOSS, 16, PASS>(sh, p, geo, go);
-    }
+    if (tma_geometry(sh, p, PASS, geo, LOSS)) return launch_tma<T, LOSS, PASS>(p, geo, go);
   }
-  return dispatch_ldg<T, LOSS, PASS>(sh, p, go);
+  return dispatch_ldg<T, LOSS, PASS>(p, go);
 }
 
 template <typename T, int PASS, typename Launcher>
@@ -376,8 +348,6 @@ template <int PASS, typename Launcher>
 int dispatch(const mafed_shape_t& sh, PathParams& p, const Launcher& go, int loss_override = -1) {
   const bool vector_ok = vector_path(sh, p, PASS);
   p.n_chunks = vector_ok ? (int)((size_t)sh.D * elem_size(sh.dtype) / 16) : 0;
-  p.load_policy = tune(sh, kTuneLoadPolicy);
-  p.store_policy = tune(sh, kTuneStorePolicy);
   const int loss = loss_override >= 0 ? loss_override : sh.loss_kind;
   switch (sh.dtype) {
     case MAFED_F32: return dispatch_loss<float, PASS>(sh, p, loss, vector_ok, go);
@@ -388,7 +358,7 @@ int dispatch(const mafed_shape_t& sh, PathParams& p, const Launcher& go, int los
 
 // Will `dispatch` take the TMA-ring kernels for this call?  (Same decision, made ahead of the launch.)
 inline bool uses_tma(const mafed_shape_t& sh, const PathParams& p, int pass) {
-  if (!vector_path(sh, p, pass) || chosen_variant(sh, pass) != 2) return false;
+  if (!vector_path(sh, p, pass) || chosen_variant(sh) != 2) return false;
   PathParams q = p;
   q.n_chunks = (int)((size_t)sh.D * elem_size(sh.dtype) / 16);
   TmaGeom geo;

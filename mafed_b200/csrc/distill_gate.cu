@@ -115,8 +115,7 @@ int gated_backward(const mafed_shape_t* shape, const void* const* student_ptrs, 
   p.bwd_scale = bwd_scale;
   p.grad_out = grad_out;       // the started kernel reads the upstream gradient itself
   p.gout_scale = grad_out_scale;
-  p.reverse = tune(*shape, kTuneBwdForward) ? 0 : 1;
-  const bool pdl = tune(*shape, kTuneNoPdl) == 0 && !consume_gate_mark(stream);   // (a gate right behind a gate)
+  const bool pdl = !consume_gate_mark(stream);   // (a gate right behind a gate)
   GateLaunch go{(cudaStream_t)stream, pdl, GateArgs{grad_out, grad_out_scale, assumed, grad_out_seen, 0, 0, 0}};
   rc = dispatch<kPassBwd>(*shape, p, go);
   note_gate_launch(stream);

@@ -28,7 +28,6 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocks) k_fwd_ldg(const __
   const long long total = groups_per_layer * p.n_layers;
   const int n_pass = (CPL == 8) ? (p.n_chunks + 32 * CPL - 1) / (32 * CPL) : 1;
   const long long row_bytes = p.row_stride * (long long)sizeof(T);
-  const uint64_t lpol = make_policy(p.load_policy);
 
   float acc_text = 0.f, acc_vis = 0.f;
   int cur = -1;
@@ -65,8 +64,8 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocks) k_fwd_ldg(const __
           const int c = pass * 32 * CPL + lane + 32 * i;
           tv[r][i] = make_uint4(0, 0, 0, 0);
           if (w[r] != 0.f && c < p.n_chunks) {
-            sv[r][i] = ldg_stream(sb + off + (long long)c * 16, p.load_policy, lpol);
-            if (LOSS != kLossL2Norm) tv[r][i] = ldg_stream(tb + off + (long long)c * 16, p.load_policy, lpol);
+            sv[r][i] = ldg_stream(sb + off + (long long)c * 16);
+            if (LOSS != kLossL2Norm) tv[r][i] = ldg_stream(tb + off + (long long)c * 16);
           } else {
             sv[r][i] = make_uint4(0, 0, 0, 0);
           }
@@ -124,15 +123,15 @@ __device__ __forceinline__ bool upstream_grad(const PathParams& p, float& gout) 
   return !(p.skip_if_gout_equals && gout == p.fixed_gout);
 }
 
-// MODE = kBackward: gradients only (2 reads + 1 write).  MODE = kFused: the same pass also
-// accumulates the forward's [layer][modality] loss sums, so student and teacher are read once per step.
+// MODE = kBackward: gradients only (2 reads + 1 write), work items walked last-to-first so that the pass starts on
+// the rows the forward left in L2.  MODE = kFused: the same pass also accumulates the forward's [layer][modality]
+// loss sums, so student and teacher are read once per step.
 template <typename T, int CPL, int RPI, int LOSS, int MODE>
 __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const __grid_constant__ PathParams p) {
   constexpr int NE = Pack<T>::kPer16;
   constexpr bool FUSED = MODE == kFused;
   __shared__ CtaSums<FUSED ? kLdgWarps : 1> sums;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint64_t spol = make_policy(p.store_policy), lpol = make_policy(p.load_policy);
   pdl_launch_dependents();
   pdl_wait();
   float gout;
@@ -149,8 +148,11 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
 
   float acc_text = 0.f, acc_vis = 0.f;
   int cur = -1;
-  for (long long g0 = blockIdx.x; g0 < total; g0 += gridDim.x) {
-    const long long g = p.reverse ? (total - 1 - g0) : g0;
+  // (the backward steps g itself down: mirroring an ascending index instead costs up to 15 registers per thread and,
+  // at short rows, a CTA per SM)
+  constexpr bool kReverse = MODE == kBackward;
+  const long long step = kReverse ? -(long long)gridDim.x : (long long)gridDim.x;
+  for (long long g = kReverse ? total - 1 - blockIdx.x : blockIdx.x; g >= 0 && g < total; g += step) {
     const int l = (int)(g / groups_per_layer);
     const long long gi = g - (long long)l * groups_per_layer;
     char* gb = reinterpret_cast<char*>(p.g[l]);
@@ -209,8 +211,8 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
         for (int i = 0; i < CPL; ++i) {
           const int c = pass * 32 * CPL + lane + 32 * i;
           if (wraw[r] != 0.f && c < p.n_chunks) {
-            sv[r][i] = ldg_stream(sb + off + (long long)c * 16, p.load_policy, lpol);
-            tv[r][i] = ldg_stream(tb + off + (long long)c * 16, p.load_policy, lpol);
+            sv[r][i] = ldg_stream(sb + off + (long long)c * 16);
+            tv[r][i] = ldg_stream(tb + off + (long long)c * 16);
           } else {
             sv[r][i] = make_uint4(0, 0, 0, 0);
             tv[r][i] = make_uint4(0, 0, 0, 0);
@@ -256,7 +258,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
           } else {
             grad_elems<LOSS, NE>(a, b, w[r], ch[r], cp[r], o);
           }
-          if (gb != nullptr) stg_128(gb + off + (long long)c * 16, Pack<T>::pack(o), p.store_policy, spol);
+          if (gb != nullptr) stg_128(gb + off + (long long)c * 16, Pack<T>::pack(o));
         }
       }
     }

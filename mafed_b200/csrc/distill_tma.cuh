@@ -11,13 +11,18 @@ namespace MAFED_NS {
 
 constexpr int kTmaMaxStages = 8;
 constexpr int kTmaMaxRows = 32;  // rows per stage (one per producer lane)
+// 16 consumer warps: two stages are drained concurrently when a stage holds <= 8 rows (+2.6 % on the 1B shape over
+// 8 warps, neutral elsewhere; profiles/r01_call4_sweep_extra.json)
+constexpr int kTmaConsumerWarps = 16;
+constexpr int kTmaConsumerThreads = kTmaConsumerWarps * 32;
+constexpr unsigned kTmaPaceNs = 500;  // refill pause of a paced ring (see tma_geometry)
 
 struct TmaGeom {
   int stages;
   int rows;         // rows per stage
   int stage_bytes;  // 2 * rows * row_bytes
-  int pace_ns;      // producer: pause between a slot becoming free and its refill (0: none)
-  int pace_dense;   // 1: only while this CTA has met no padded row yet (the batch looks dense)
+  int pace;         // 1: the producer pauses kTmaPaceNs between a slot becoming free and its refill, as long as this
+                    // CTA has met no padded row (the batch looks dense)
 };
 
 struct TmaStageMeta {
@@ -54,15 +59,9 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   } while (!ok);
 }
 // 1-D bulk async copy global -> shared, completion signalled on an mbarrier (bytes % 16 == 0).
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, int kind,
-                                         uint64_t pol) {
-  if (kind == kPolicyNone) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-  } else {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-                 :: "r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(pol) : "memory");
-  }
+__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               :: "r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
 __device__ __forceinline__ uint4 lds_128(uint32_t addr) {
   uint4 r;
@@ -74,7 +73,8 @@ __device__ __forceinline__ void named_bar_sync(int id, int n_threads) {
 }
 
 // ---------------------------------------------------------------- producer
-// All 32 lanes of the producer warp run this; lane r owns row r of every stage.
+// All 32 lanes of the producer warp run this; lane r owns row r of every stage.  The backward walks its tiles
+// last-to-first, so that it starts on the rows the forward left in L2.
 template <typename T>
 __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom& geo, unsigned char* data,
                                              uint64_t* full, uint64_t* empty, TmaStageMeta* meta, int lane,
@@ -84,7 +84,6 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
   const uint32_t row_bytes = (uint32_t)p.n_chunks * 16u;
   const long long row_pitch = p.row_stride * (long long)sizeof(T);
   const bool contiguous = row_pitch == (long long)row_bytes;
-  const uint64_t lpol = make_policy(p.load_policy);
   int stage = 0;
   uint32_t phase = 0;
   // The row weights of a tile come from the attention mask (an L2 round trip).  They are fetched one tile ahead, so
@@ -98,8 +97,8 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
   long long f_til = (long long)blockIdx.x - (long long)f_l * tiles_per_layer;
   auto fetch = [&]() {
     Tile x;
-    x.l = p.reverse ? (p.n_layers - 1 - f_l) : f_l;
-    x.row0 = (p.reverse ? (tiles_per_layer - 1 - f_til) : f_til) * geo.rows;
+    x.l = for_backward ? (p.n_layers - 1 - f_l) : f_l;
+    x.row0 = (for_backward ? (tiles_per_layer - 1 - f_til) : f_til) * geo.rows;
     x.n_rows = (int)min((long long)geo.rows, p.n_rows - x.row0);
     x.m = 1;
     x.w = 0.f;
@@ -134,7 +133,7 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
     // the critical path and must not be held back.
     if (lane < n_rows && w == 0.f) seen_padded = true;
     seen_padded = __any_sync(0xffffffffu, seen_padded);
-    if (geo.pace_ns > 0 && !(geo.pace_dense && seen_padded)) __nanosleep((unsigned)geo.pace_ns);
+    if (geo.pace && !seen_padded) __nanosleep(kTmaPaceNs);
 
     const unsigned valid = __ballot_sync(0xffffffffu, w != 0.f);
     TmaStageMeta& mt = meta[stage];
@@ -153,13 +152,12 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
     const unsigned all = (n_rows >= 32) ? 0xffffffffu : ((1u << n_rows) - 1u);
     if (contiguous && valid == all) {
       // whole tile live: one bulk copy per tensor
-      if (lane == 0) bulk_g2s(s_dst, sb, (uint32_t)n_rows * row_bytes, bar, p.load_policy, lpol);
-      if (lane == 1 && both) bulk_g2s(t_dst, tb, (uint32_t)n_rows * row_bytes, bar, p.load_policy, lpol);
+      if (lane == 0) bulk_g2s(s_dst, sb, (uint32_t)n_rows * row_bytes, bar);
+      if (lane == 1 && both) bulk_g2s(t_dst, tb, (uint32_t)n_rows * row_bytes, bar);
     } else if (w != 0.f) {
       // ragged tile: only live rows are fetched (padded text rows cost no bandwidth)
-      bulk_g2s(s_dst + (uint32_t)lane * row_bytes, sb + (long long)lane * row_pitch, row_bytes, bar, p.load_policy, lpol);
-      if (both)
-        bulk_g2s(t_dst + (uint32_t)lane * row_bytes, tb + (long long)lane * row_pitch, row_bytes, bar, p.load_policy, lpol);
+      bulk_g2s(s_dst + (uint32_t)lane * row_bytes, sb + (long long)lane * row_pitch, row_bytes, bar);
+      if (both) bulk_g2s(t_dst + (uint32_t)lane * row_bytes, tb + (long long)lane * row_pitch, row_bytes, bar);
     }
     if (++stage == geo.stages) { stage = 0; phase ^= 1u; }
   }
@@ -171,12 +169,11 @@ struct TmaSmem {
   TmaStageMeta meta[kTmaMaxStages];
 };
 
-template <int NCW>
 __device__ __forceinline__ void tma_prologue(TmaSmem& sm, const TmaGeom& geo) {
   if (threadIdx.x == 0) {
     for (int i = 0; i < geo.stages; ++i) {
       mbar_init(smem_u32(&sm.full[i]), 1);      // producer's arrive.expect_tx
-      mbar_init(smem_u32(&sm.empty[i]), NCW);   // one arrive per consumer warp
+      mbar_init(smem_u32(&sm.empty[i]), kTmaConsumerWarps);   // one arrive per consumer warp
     }
     mbar_fence_init();
   }
@@ -237,18 +234,18 @@ __device__ __forceinline__ void tma_tail(const PathParams& p, const double* coun
 }
 
 // ---------------------------------------------------------------- forward
-template <typename T, int LOSS, int NCW>
-__global__ void __launch_bounds__((NCW + 1) * 32, 1)
+template <typename T, int LOSS>
+__global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
 k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo) {
   constexpr int NE = Pack<T>::kPer16;
   extern __shared__ __align__(128) unsigned char dyn_smem[];
   __shared__ TmaSmem sm;
-  __shared__ CtaSums<NCW> sums;
+  __shared__ CtaSums<kTmaConsumerWarps> sums;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   cta_sums_zero(sums, p.n_layers);
-  tma_prologue<NCW>(sm, geo);
+  tma_prologue(sm, geo);
 
-  if (warp == NCW) {
+  if (warp == kTmaConsumerWarps) {
     tma_producer<T>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, false);
     return;
   }
@@ -271,8 +268,9 @@ k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     const uint32_t s_base = smem_u32(dyn_smem + (size_t)stage * geo.stage_bytes);
     const uint32_t t_base = s_base + (uint32_t)geo.rows * row_bytes;
     // rotate the row->warp map with the iteration so short tiles still use every warp over time
-    const int first = (int)((warp + NCW - (int)((it * geo.rows) % NCW)) % NCW);
-    for (int r = first; r < mt.n_rows; r += NCW) {
+    const int first =
+        (int)((warp + kTmaConsumerWarps - (int)((it * geo.rows) % kTmaConsumerWarps)) % kTmaConsumerWarps);
+    for (int r = first; r < mt.n_rows; r += kTmaConsumerWarps) {
       const float w = mt.w[r];
       if (w == 0.f) continue;
       const uint32_t sa = s_base + (uint32_t)r * row_bytes, ta = t_base + (uint32_t)r * row_bytes;
@@ -315,9 +313,9 @@ k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     if (++stage == geo.stages) { stage = 0; phase ^= 1u; }
   }
   cta_sums_flush(sums, warp, lane, cur, acc_text, acc_vis);
-  named_bar_sync(1, NCW * 32);
-  cta_sums_store(sums, p.ws, p.n_layers, 0, NCW * 32);
-  if (p.tail_done != nullptr) tma_tail<NCW * 32>(p, nullptr);
+  named_bar_sync(1, kTmaConsumerThreads);
+  cta_sums_store(sums, p.ws, p.n_layers, 0, kTmaConsumerThreads);
+  if (p.tail_done != nullptr) tma_tail<kTmaConsumerThreads>(p, nullptr);
 }
 
 // ---------------------------------------------------------------- backward
@@ -411,18 +409,17 @@ __device__ __forceinline__ float cosine_row_unrolled(uint32_t sa, uint32_t ta, i
 
 // MODE = kBackward: gradients only.  MODE = kFused: the consumers also accumulate the forward's loss
 // sums from the rows they already hold in shared memory (one pass over student and teacher per step).
-template <typename T, int LOSS, int NCW, int MODE>
-__global__ void __launch_bounds__((NCW + 1) * 32, 1)
+template <typename T, int LOSS, int MODE>
+__global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
 k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo) {
   constexpr int NE = Pack<T>::kPer16;
   constexpr bool FUSED = MODE == kFused;
   extern __shared__ __align__(128) unsigned char dyn_smem[];
   __shared__ TmaSmem sm;
-  __shared__ CtaSums<FUSED ? NCW : 1> sums;
+  __shared__ CtaSums<FUSED ? kTmaConsumerWarps : 1> sums;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint64_t spol = make_policy(p.store_policy);
   if (FUSED) cta_sums_zero(sums, p.n_layers);
-  tma_prologue<NCW>(sm, geo);
+  tma_prologue(sm, geo);
   float gout;
   if (FUSED) {
     gout = p.fixed_gout;
@@ -430,7 +427,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     gout = (p.grad_out ? __ldg(p.grad_out) : 1.f) * p.gout_scale;
     if (p.skip_if_gout_equals && gout == p.fixed_gout) return;  // fix-up launch with nothing to fix
   }
-  if (warp == NCW) {
+  if (warp == kTmaConsumerWarps) {
     tma_producer<T>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, !FUSED);
     return;
   }
@@ -443,7 +440,8 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
   if (FUSED && p.lang_mask_out != nullptr) {
     // the masks the reference leaves in `batch` (distillation.py:134-144): a few hundred KB spread over all CTAs
     const long long n = p.n_rows;
-    for (long long i = (long long)blockIdx.x * (NCW * 32) + threadIdx.x; i < n; i += (long long)gridDim.x * (NCW * 32)) {
+    for (long long i = (long long)blockIdx.x * kTmaConsumerThreads + threadIdx.x; i < n;
+         i += (long long)gridDim.x * kTmaConsumerThreads) {
       const long long b = i / p.T;
       const int t = (int)(i - b * p.T);
       const bool vis = t < p.n_vis;
@@ -452,7 +450,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     }
   }
   if (FUSED && p.inline_scale) {
-    __shared__ long long s_cnt[NCW];
+    __shared__ long long s_cnt[kTmaConsumerWarps];
     __shared__ double s_peer[kCommMaxRanks][2];
     const CommDev& c = p.comm;
     const bool sharded = c.world > 1 && p.comm_counts;
@@ -470,7 +468,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
           s_peer[r][k] = ll_wait(ll_count_slot(c.ll[c.rank], (int)(e % kCommCountSlots), r, k), ll_tag(e), c.status,
                                  c.timeout_cycles);
         }
-        named_bar_sync(1, NCW * 32);
+        named_bar_sync(1, kTmaConsumerThreads);
         if (blockIdx.x == 0 && threadIdx.x == 0) c.trace[0] += (unsigned long long)(clock64() - t_x0);
         n_text = 0.0;
         n_vis_rows = 0.0;
@@ -484,14 +482,14 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
       }
     } else {
       long long cnt = 0;
-      for (long long i = threadIdx.x; i < p.n_mask; i += NCW * 32) cnt += p.mask[i];
+      for (long long i = threadIdx.x; i < p.n_mask; i += kTmaConsumerThreads) cnt += p.mask[i];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
       if (lane == 0) s_cnt[warp] = cnt;
-      named_bar_sync(1, NCW * 32);
+      named_bar_sync(1, kTmaConsumerThreads);
       long long n_text_local = 0;
 #pragma unroll
-      for (int i = 0; i < NCW; ++i) n_text_local += s_cnt[i];
+      for (int i = 0; i < kTmaConsumerWarps; ++i) n_text_local += s_cnt[i];
       n_text = (double)n_text_local;
       n_vis_rows = p.n_vis_rows;
       if (sharded) {
@@ -515,7 +513,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
           const int r = threadIdx.x >> 1, k = threadIdx.x & 1;
           s_peer[r][k] = ll_wait(ll_slot(c.ll[c.rank], par, r, k), tag, c.status, c.timeout_cycles);
         }
-        named_bar_sync(1, NCW * 32);
+        named_bar_sync(1, kTmaConsumerThreads);
         if (blockIdx.x == 0 && threadIdx.x == 0) c.trace[0] += (unsigned long long)(clock64() - t_x0);
         n_text = 0.0;
         n_vis_rows = 0.0;
@@ -537,9 +535,9 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
       }
     }
   } else {
-    for (int i = threadIdx.x; i < 2 * p.n_layers; i += NCW * 32) s_scale[i] = __ldg(p.bwd_scale + i);
+    for (int i = threadIdx.x; i < 2 * p.n_layers; i += kTmaConsumerThreads) s_scale[i] = __ldg(p.bwd_scale + i);
   }
-  named_bar_sync(1, NCW * 32);
+  named_bar_sync(1, kTmaConsumerThreads);
 
   const long long tiles_per_layer = (p.n_rows + geo.rows - 1) / geo.rows;
   const long long total = tiles_per_layer * p.n_layers;
@@ -562,9 +560,10 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     char* gb = reinterpret_cast<char*>(p.g[l]);
     const uint32_t s_base = smem_u32(dyn_smem + (size_t)stage * geo.stage_bytes);
     const uint32_t t_base = s_base + (uint32_t)geo.rows * row_bytes;
-    const int first = (int)((warp + NCW - (int)((it * geo.rows) % NCW)) % NCW);
+    const int first =
+        (int)((warp + kTmaConsumerWarps - (int)((it * geo.rows) % kTmaConsumerWarps)) % kTmaConsumerWarps);
     if (FUSED || gb != nullptr) {
-      for (int r = first; r < mt.n_rows; r += NCW) {
+      for (int r = first; r < mt.n_rows; r += kTmaConsumerWarps) {
         char* grow = gb + (mt.row0 + r) * row_pitch;
         const float w = mt.w[r] * (gout * s_scale[2 * l + mt.mod[r]]);
         if (mt.w[r] == 0.f) {  // padded text row: nothing was fetched; grad = 0 * scale (zero, or NaN if scale is)
@@ -573,65 +572,18 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
           for (int i = 0; i < NE; ++i) o[i] = w;
           const uint4 fill = Pack<T>::pack(o);
           if (gb != nullptr)
-            for (int c = lane; c < p.n_chunks; c += 32) stg_128(grow + (long long)c * 16, fill, p.store_policy, spol);
+            for (int c = lane; c < p.n_chunks; c += 32) stg_128(grow + (long long)c * 16, fill);
           continue;
         }
         const uint32_t sa = s_base + (uint32_t)r * row_bytes, ta = t_base + (uint32_t)r * row_bytes;
         float ch = 0.f, cp = 0.f, rowval = 0.f;
-        if (LOSS == MAFED_LOSS_COSINE && NCW == 16 && (p.n_chunks == 96 || p.n_chunks == 128 || p.n_chunks == 192)) {
+        if (LOSS == MAFED_LOSS_COSINE && (p.n_chunks == 96 || p.n_chunks == 128 || p.n_chunks == 192)) {
           // short rows (1.5 / 2 / 3 KB: base and 410M hidden sizes in bf16, base in fp32): fully unrolled forms
           float val;
           if (p.n_chunks == 96) val = cosine_row_unrolled<T, 3, true>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
           else if (p.n_chunks == 128) val = cosine_row_unrolled<T, 4, false>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
           else val = cosine_row_unrolled<T, 6, false>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
           if (FUSED && lane == 0) {
-            if (mt.mod[r] == 0) acc_text = fmaf(mt.w[r], val, acc_text);
-            else acc_vis = fmaf(mt.w[r], val, acc_vis);
-          }
-          continue;
-        }
-        if (LOSS == MAFED_LOSS_COSINE && NCW == 8 && p.n_chunks <= 256) {
-          // cosine, rows up to 4 KB, 8-warp build only (the 16-warp default has no register room for it and
-          // hides the latency of the two-pass form better, profiles/): the lane's share of the row pair lives in
-          // registers between the statistics pass and the gradient pass
-          uint4 sv[8], tv[8];
-          float x = 0.f, y = 0.f, z = 0.f;
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int c = lane + 32 * u;
-            if (c < p.n_chunks) {
-              sv[u] = lds_128(sa + (uint32_t)c * 16u);
-              tv[u] = lds_128(ta + (uint32_t)c * 16u);
-            } else {
-              sv[u] = make_uint4(0, 0, 0, 0);
-              tv[u] = make_uint4(0, 0, 0, 0);
-            }
-          }
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            float a[NE], b[NE];
-            Pack<T>::unpack(sv[u], a);
-            Pack<T>::unpack(tv[u], b);
-            accumulate<LOSS, NE>(a, b, x, y, z);
-          }
-          x = warp_sum(x); y = warp_sum(y); z = warp_sum(z);
-          const float aa = y + kCosEps, den = sqrtf(aa * (z + kCosEps));
-          ch = w * (x / den) / aa;
-          cp = w / den;
-          if (gb != nullptr) {
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-              const int c = lane + 32 * u;
-              if (c >= p.n_chunks) continue;
-              float a[NE], b[NE], o[NE];
-              Pack<T>::unpack(sv[u], a);
-              Pack<T>::unpack(tv[u], b);
-              grad_elems_tma<LOSS, NE>(a, b, w, ch, cp, o);
-              stg_128(grow + (long long)c * 16, Pack<T>::pack(o), p.store_policy, spol);
-            }
-          }
-          if (FUSED && lane == 0) {
-            const float val = 1.f - x / den;
             if (mt.mod[r] == 0) acc_text = fmaf(mt.w[r], val, acc_text);
             else acc_vis = fmaf(mt.w[r], val, acc_vis);
           }
@@ -669,7 +621,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
               accumulate<LOSS, NE>(a, b, rowval, y, z);
             }
             grad_elems_tma<LOSS, NE>(a, b, w, ch, cp, o);
-            if (gb != nullptr) stg_128(grow + (long long)(c + 32 * u) * 16, Pack<T>::pack(o), p.store_policy, spol);
+            if (gb != nullptr) stg_128(grow + (long long)(c + 32 * u) * 16, Pack<T>::pack(o));
           }
         }
         for (; c < p.n_chunks; c += 32) {
@@ -681,7 +633,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
             accumulate<LOSS, NE>(a, b, rowval, y, z);
           }
           grad_elems_tma<LOSS, NE>(a, b, w, ch, cp, o);
-          if (gb != nullptr) stg_128(grow + (long long)c * 16, Pack<T>::pack(o), p.store_policy, spol);
+          if (gb != nullptr) stg_128(grow + (long long)c * 16, Pack<T>::pack(o));
         }
         if (FUSED) {
           if (mt.mod[r] == 0) acc_text = fmaf(mt.w[r], rowval, acc_text);
@@ -695,9 +647,9 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
   }
   if (FUSED) {
     cta_sums_flush(sums, warp, lane, cur, acc_text, acc_vis);
-    named_bar_sync(1, NCW * 32);
-    cta_sums_store(sums, p.ws, p.n_layers, 0, NCW * 32);
-    if (p.tail_done != nullptr) tma_tail<NCW * 32>(p, p.inline_scale ? s_counts : p.tail_counts_in, counts_epoch);
+    named_bar_sync(1, kTmaConsumerThreads);
+    cta_sums_store(sums, p.ws, p.n_layers, 0, kTmaConsumerThreads);
+    if (p.tail_done != nullptr) tma_tail<kTmaConsumerThreads>(p, p.inline_scale ? s_counts : p.tail_counts_in, counts_epoch);
   }
 }
 

@@ -51,6 +51,13 @@ def test_no_process_global_knobs():
             assert inner.v[cabi.TUNE_NO_TAIL] == 1 and inner.v[cabi.TUNE_NO_GATE] == 1
     assert cabi.active_tuning_address() == 0
     assert not cabi.make_shape(1, 1, 4, 2, 8, cabi.F32, cabi.LOSS_MSE).tuning
+    # only the three keys the library reads are accepted; a retired or misspelt one is an error, not a silent no-op
+    import pytest
+    for bad in ({"TUNE_TMA_WARPS": 8}, {"F32": 1}, {"raw": {9: 8}}):
+        with pytest.raises(TypeError, match="unknown tuning key"):
+            with cabi.tuning(**bad):
+                pass
+    assert cabi.active_tuning_address() == 0
 
 
 def test_torch_extension_builds_and_binds():
@@ -98,6 +105,10 @@ def test_argument_errors_without_a_gpu():
     assert lib.mafed_distill_step(ctypes.byref(ok), None, None, None, None, ctypes.byref(w), one, None, 8, None, None,
                                   8, None, None, None, None) == -1
     assert lib.mafed_distill_bwd(ctypes.byref(ok), None, None, None, None, None, None, one, None, None, None) == -1
+    # a NULL shape is an argument error on the gate path too (grad table, scale table and skip_if_equals given)
+    scale = (ctypes.c_float * 2)()
+    assert lib.mafed_distill_bwd(None, None, None, cabi.ptr_array([8]), None, scale, None, one, ctypes.byref(one), None,
+                                 None) == -1
     assert lib.mafed_distill_prefetch_counts(ctypes.byref(ok), None, None, None, None) == -1
     assert lib.mafed_distill_scalar_stage(ctypes.byref(ok), None, cabi.STAGE_LOSSES, None, None, None, None, None, None, 0,
                                           None) == -1

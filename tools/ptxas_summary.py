@@ -45,7 +45,7 @@ def main():
     for k, v in fam.items():
         regs = [r["regs"] for r in v]
         print(f"  {k}: {len(v)}, {min(regs)}-{max(regs)}, {sum(1 for r in v if r['st'] or r['ld'])}")
-    print("\nTMA-ring kernels <dtype, loss (0 mse, 1 cosine, 2 L2 norm), consumer warps[, pass (1 backward, 2 one-pass step)]>:")
+    print("\nTMA-ring kernels <dtype, loss (0 mse, 1 cosine, 2 L2 norm)[, pass (1 backward, 2 one-pass step)]>:")
     for r in rows:
         if "_tma" in r["name"]:
             print(f"  {r['name']}: {r['regs']} registers, stack {r['stack']} B, spill stores / loads {r['st']} / {r['ld']} B")

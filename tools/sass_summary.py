@@ -43,12 +43,12 @@ def main():
             if re.search(pat, line):
                 counts[cur][key] += 1
     names = demangle(order)
-    want = [("fused step, bf16 mse (headline)", "mafed::k_bwd_tma<__nv_bfloat16, 0, 16, 2>"),
-            ("fused step, bf16 cosine", "mafed::k_bwd_tma<__nv_bfloat16, 1, 16, 2>"),
-            ("fused step, fp32 mse", "mafed::k_bwd_tma<float, 0, 16, 2>"),
-            ("forward, bf16 mse", "mafed::k_fwd_tma<__nv_bfloat16, 0, 16>"),
-            ("backward, bf16 mse", "mafed::k_bwd_tma<__nv_bfloat16, 0, 16, 1>"),
-            ("backward started by the gate, bf16 mse (rdc unit)", "mafed_gate::k_bwd_tma<__nv_bfloat16, 0, 16, 1>"),
+    want = [("fused step, bf16 mse (headline)", "mafed::k_bwd_tma<__nv_bfloat16, 0, 2>"),
+            ("fused step, bf16 cosine", "mafed::k_bwd_tma<__nv_bfloat16, 1, 2>"),
+            ("fused step, fp32 mse", "mafed::k_bwd_tma<float, 0, 2>"),
+            ("forward, bf16 mse", "mafed::k_fwd_tma<__nv_bfloat16, 0>"),
+            ("backward, bf16 mse", "mafed::k_bwd_tma<__nv_bfloat16, 0, 1>"),
+            ("backward started by the gate, bf16 mse (rdc unit)", "mafed_gate::k_bwd_tma<__nv_bfloat16, 0, 1>"),
             ("register-staged fused step, bf16 mse, 4 KB rows", "mafed::k_bwd_ldg<__nv_bfloat16, 8, 1, 0, 2>"),
             ("scalar stage", "mafed::k_epilogue"), ("count prefetch", "mafed::k_prefetch_counts")]
     print(f"library: {os.path.relpath(LIB, ROOT)}   target(s): {', '.join(sorted(arch))}   kernels: {len(order)}")

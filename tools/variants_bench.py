@@ -2,7 +2,7 @@
 """Kernel-level step time for the non-headline variants: cosine loss, fp32 / fp16 hidden states, 'equal'
 weights, at the 1B and base shapes (one-pass and two-pass), both kernel families.
 
-    python tools/variants_bench.py [--only cosine_base] [--warps 8|16] [--out gpurun_out/variants_bench.json]
+    python tools/variants_bench.py [--only cosine_base] [--out FILE]
 
 ``--only cosine_base`` runs just the cosine one-pass step at the base shape (the case to profile under ncu).
 """
@@ -37,7 +37,6 @@ def time_ms(fn, iters=50, warm=8):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=None)
-    ap.add_argument("--warps", type=int, default=0)
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "variants_bench.json"))
     args = ap.parse_args()
     cabi.load()
@@ -63,7 +62,7 @@ def main():
             plan = DistillPlan(layers=list(range(L)), layer_coeffs=[1.0 / L] * L, modality_kind=cabi.MODW_EQUAL,
                                loss_kind=loss)
             for variant in variants:
-                with cabi.tuning(variant=variant, raw={cabi.TUNE_TMA_WARPS: args.warps}):
+                with cabi.tuning(variant=variant):
                     def one():
                         o, s, l = distill_fused(st, te, grads, am, plan, group=False)
                         distill_backward(l, grads, s, gout, skip_if_equals=1.0)
@@ -75,7 +74,7 @@ def main():
                     m1 = time_ms(one, iters=iters, warm=3 if args.only else 8)
                     m2 = time_ms(two, iters=iters) if not args.only else None
                 rec = dict(shape=name, loss="mse" if loss == 0 else "cosine", variant="tma" if variant == 2 else "ldg",
-                           warps=args.warps or 16, one_ms=m1, one_gbs=3 * D * esize * units / m1 / 1e6)
+                           one_ms=m1, one_gbs=3 * D * esize * units / m1 / 1e6)
                 if m2 is not None:
                     rec.update(two_ms=m2, two_gbs=5 * D * esize * units / m2 / 1e6)
                 out.append(rec)
