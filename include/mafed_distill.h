@@ -48,6 +48,14 @@ extern "C" {
 #define MAFED_MAX_LAYERS 64
 
 enum { MAFED_F32 = 0, MAFED_BF16 = 1, MAFED_F16 = 2 };
+/* mafed_shape_t::dtype of a call whose teacher has another type than the student: bits 0-7 hold the student's (and the
+ * gradient's) type, bits 8-15 the teacher's type + 1; 0 there means "the student's type", so a plain MAFED_F32 /
+ * MAFED_BF16 / MAFED_F16 keeps its meaning.  Supported pairs: MAFED_DTYPE_PAIR(MAFED_F32, MAFED_BF16) and
+ * MAFED_DTYPE_PAIR(MAFED_F32, MAFED_F16) -- an fp32 student distilled against a half-precision teacher, read as such
+ * by the kernels (no up-cast copy).  Every other pair is MAFED_E_DTYPE, as is any pair given to
+ * mafed_distill_token_norm_sums (one input) and to the host-buffer step (mafed_host_step_device_bytes returns 0).
+ * (A library built before the encoding rejects every pair with MAFED_E_DTYPE.) */
+#define MAFED_DTYPE_PAIR(student, teacher) ((student) | (((teacher) + 1) << 8))
 enum { MAFED_LOSS_MSE = 0, MAFED_LOSS_COSINE = 1 };
 /* modality weighting (distillation_loss_weights.py:71-79):
  *   EQUAL: w_text = n_text/(n_text+n_vis) from the mask counts (:148-155);
@@ -85,7 +93,7 @@ typedef struct mafed_shape {
   int32_t T;          /* n_vis + text positions */
   int32_t n_vis;      /* 256 in the reference (distillation.py:73) */
   int32_t D;          /* hidden size */
-  int32_t dtype;      /* MAFED_F32 | MAFED_BF16 | MAFED_F16 (student, teacher and gradient) */
+  int32_t dtype;      /* MAFED_F32 | MAFED_BF16 | MAFED_F16 (student, teacher and gradient), or a MAFED_DTYPE_PAIR */
   int32_t loss_kind;  /* MAFED_LOSS_MSE (distillation.py:237-249) | MAFED_LOSS_COSINE (:226-235) */
   int32_t cls;        /* 1: CLS distillation (distillation.py:126-132,251-257) */
   const mafed_tuning_t* tuning;   /* NULL: defaults */

@@ -11,6 +11,16 @@ import threading
 
 MAX_LAYERS = 64
 F32, BF16, F16 = 0, 1, 2
+# mafed_shape_t::dtype of a call whose teacher has another type (MAFED_DTYPE_PAIR of the header): the student's type in
+# the low byte, the teacher's type + 1 in the next one.  Supported: an F32 student with a BF16 or F16 teacher.
+DTYPE_PAIR_SHIFT = 8
+
+
+def dtype_pair(student: int, teacher: int) -> int:
+    """MAFED_DTYPE_PAIR(student, teacher)."""
+    return student | ((teacher + 1) << DTYPE_PAIR_SHIFT)
+
+
 LOSS_MSE, LOSS_COSINE = 0, 1
 MODW_EQUAL, MODW_TABLE, MODW_CLS, MODW_TEXT_ONLY = 0, 1, 2, 3
 VARIANT_DEFAULT, VARIANT_LDG, VARIANT_TMA = 0, 1, 2
@@ -193,9 +203,11 @@ def ptr_array(ptrs):
     return (ctypes.c_void_p * len(ptrs))(*ptrs)
 
 
-def make_shape(n_layers, B, T, n_vis, D, dtype, loss_kind, cls=False):
-    """mafed_shape_t of one call; carries the Tuning installed by `tuning(...)`, if any (kept alive by the shape)."""
-    sh = Shape(n_layers, B, T, n_vis, D, dtype, loss_kind, 1 if cls else 0, None)
+def make_shape(n_layers, B, T, n_vis, D, dtype, loss_kind, cls=False, teacher_dtype=None):
+    """mafed_shape_t of one call; carries the Tuning installed by `tuning(...)`, if any (kept alive by the shape).
+    ``teacher_dtype``: the teacher's type when it differs from ``dtype`` (the student's), else None."""
+    code = dtype if teacher_dtype is None or teacher_dtype == dtype else dtype_pair(dtype, teacher_dtype)
+    sh = Shape(n_layers, B, T, n_vis, D, code, loss_kind, 1 if cls else 0, None)
     if _active_tuning is not None:
         sh.tuning = ctypes.pointer(_active_tuning)
     return sh

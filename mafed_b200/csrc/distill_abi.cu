@@ -223,8 +223,11 @@ int mafed_distill_fwd(const mafed_shape_t* shape, const void* const* student_ptr
 
 int mafed_distill_token_norm_sums(const mafed_shape_t* shape, const void* const* tensor_ptrs, const int64_t* attn_mask,
                                   void* ws, void* stream) {
+  int rc = check_shape(shape);
+  if (rc) return rc;
+  if (mixed_pair(*shape)) return MAFED_E_DTYPE;   // one input: a teacher type means nothing here
   PathParams p;
-  int rc = fill_params(shape, tensor_ptrs, tensor_ptrs, nullptr, attn_mask, p);
+  rc = fill_params(shape, tensor_ptrs, tensor_ptrs, nullptr, attn_mask, p);
   if (rc) return rc;
   if (!ws) return MAFED_E_ARG;
   p.ws = reinterpret_cast<float*>(ws);
@@ -473,9 +476,10 @@ int mafed_distill_modality_masks(const mafed_shape_t* shape, const int64_t* attn
 }
 
 // ---------------------------------------------------------------- host-buffer step
+// The host-buffer step stages student, teacher and gradient in equal slots: it takes no student / teacher pair.
 size_t mafed_host_step_device_bytes(const mafed_shape_t* shape) {
-  if (check_shape(shape)) return 0;
-  const size_t layer = (size_t)shape->B * shape->T * shape->D * elem_size(shape->dtype);
+  if (check_shape(shape) || mixed_pair(*shape)) return 0;
+  const size_t layer = (size_t)shape->B * shape->T * shape->D * student_size(*shape);
   const size_t mask = needs_mask(*shape) ? (size_t)shape->B * (shape->T - shape->n_vis) * sizeof(int64_t) : 0;
   return 3 * layer * shape->n_layers + mask + (size_t)shape->n_layers * (mafed_distill_ws_bytes(1) + 128) + 4096;
 }
@@ -483,12 +487,13 @@ size_t mafed_host_step_device_bytes(const mafed_shape_t* shape) {
 int mafed_host_step_create(const mafed_shape_t* shape, mafed_host_step_t** out) {
   int rc = check_shape(shape);
   if (rc) return rc;
+  if (mixed_pair(*shape)) return MAFED_E_DTYPE;
   if (!out || shape->cls) return MAFED_E_ARG;
   if (!device_info().ok) return MAFED_E_NODEVICE;
   mafed_host_step* h = new mafed_host_step();
   h->shape = *shape;
   const int L = shape->n_layers;
-  h->layer_bytes = (((size_t)shape->B * shape->T * shape->D * elem_size(shape->dtype)) + 255) & ~(size_t)255;
+  h->layer_bytes = (((size_t)shape->B * shape->T * shape->D * student_size(*shape)) + 255) & ~(size_t)255;
   h->mask_bytes = ((needs_mask(*shape) ? (size_t)shape->B * (shape->T - shape->n_vis) * sizeof(int64_t) : 0) + 255) & ~(size_t)255;
   h->ws_bytes = (mafed_distill_ws_bytes(1) + 255) & ~(size_t)255;
   const size_t total = 3 * h->layer_bytes * L + h->mask_bytes + (size_t)L * h->ws_bytes + (size_t)L * 6 * sizeof(float) +
@@ -531,7 +536,7 @@ int mafed_host_step_run(mafed_host_step_t* h, const mafed_weights_t* weights, co
   const mafed_shape_t& sh = h->shape;
   const int L = sh.n_layers;
   if (needs_mask(sh) && !h_mask) return MAFED_E_ARG;
-  const size_t layer = (size_t)sh.B * sh.T * sh.D * elem_size(sh.dtype);
+  const size_t layer = (size_t)sh.B * sh.T * sh.D * student_size(sh);
   const size_t mask = needs_mask(sh) ? (size_t)sh.B * (sh.T - sh.n_vis) * sizeof(int64_t) : 0;
   cudaError_t e = cudaSuccess;
   if (mask) e = cudaMemcpyAsync(h->d_mask, h_mask, mask, cudaMemcpyHostToDevice, h->s_in);

@@ -183,6 +183,41 @@ __device__ __forceinline__ void stg_128(void* p, const uint4& v) {
   asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};"
                :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
+__device__ __forceinline__ uint2 ldg_stream_64(const void* p) {
+  uint2 r;
+  asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
+  return r;
+}
+
+// ---------------------------------------------------------------- the teacher's share of a work unit
+// The unit of the vector kernels is one 16-byte chunk of the student row (and of the gradient row).  The teacher
+// values of the same elements are, with the student's dtype, a 16-byte chunk as well; with an fp32 student and a
+// bf16 / fp16 teacher they are 4 half-precision values, 8 bytes.  Widening them to fp32 is exact, so every
+// per-element expression sees the same operands as it would on the teacher up-cast to fp32.
+template <typename TS, typename TT>
+struct TeacherChunk {
+  using Vec = uint4;
+  static constexpr int kBytes = 16;
+  static constexpr int kShift = 0;   // teacher row bytes = student row bytes >> kShift
+  __device__ __forceinline__ static uint4 ldg(const void* p) { return ldg_stream(p); }
+  __device__ __forceinline__ static void unpack(const uint4& v, float (&f)[Pack<TS>::kPer16]) { Pack<TT>::unpack(v, f); }
+};
+
+template <typename TT>
+struct HalfTeacherChunk {
+  using Vec = uint2;
+  static constexpr int kBytes = 8;
+  static constexpr int kShift = 1;
+  __device__ __forceinline__ static uint2 ldg(const void* p) { return ldg_stream_64(p); }
+  __device__ __forceinline__ static void unpack(const uint2& v, float (&f)[4]) {
+    float lo[2], hi[2];
+    Pack<TT>::unpack_word(v.x, lo);
+    Pack<TT>::unpack_word(v.y, hi);
+    f[0] = lo[0]; f[1] = lo[1]; f[2] = hi[0]; f[3] = hi[1];
+  }
+};
+template <> struct TeacherChunk<float, __nv_bfloat16> : HalfTeacherChunk<__nv_bfloat16> {};
+template <> struct TeacherChunk<float, __half> : HalfTeacherChunk<__half> {};
 
 // ---------------------------------------------------------------- programmatic dependent launch
 // Every kernel of the path is launched with programmaticStreamSerialization: it may become resident

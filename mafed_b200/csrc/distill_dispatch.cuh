@@ -9,6 +9,7 @@
 // occupancy / opt-in shared memory are per kernel and per device.
 #pragma once
 #include <cstring>
+#include <type_traits>
 
 #include "distill_common.cuh"
 #include "distill_ldg.cuh"
@@ -74,16 +75,30 @@ inline const DeviceInfo& device_info() {
   return d;
 }
 
+// mafed_shape_t::dtype: bits 0-7 the student / gradient type, bits 8-15 the teacher type + 1 (0: the student's)
+inline int student_dtype(const mafed_shape_t& sh) { return sh.dtype & 0xff; }
+inline int teacher_dtype(const mafed_shape_t& sh) {
+  const int t = (sh.dtype >> 8) & 0xff;
+  return t == 0 ? student_dtype(sh) : t - 1;
+}
+inline bool mixed_pair(const mafed_shape_t& sh) { return teacher_dtype(sh) != student_dtype(sh); }
+
 inline int check_shape(const mafed_shape_t* sh) {
   if (sh == nullptr) return MAFED_E_ARG;
   if (sh->n_layers < 1 || sh->n_layers > kMaxLayers) return MAFED_E_ARG;
   if (sh->B < 1 || sh->T < 1 || sh->D < 1 || sh->n_vis < 0 || sh->n_vis > sh->T) return MAFED_E_ARG;
-  if (sh->dtype < MAFED_F32 || sh->dtype > MAFED_F16) return MAFED_E_DTYPE;
+  if (sh->dtype < 0 || (sh->dtype >> 16) != 0) return MAFED_E_DTYPE;
+  const int s = student_dtype(*sh), t = teacher_dtype(*sh);
+  if (s > MAFED_F16 || t > MAFED_F16) return MAFED_E_DTYPE;
+  // the pairs with kernels of their own: an fp32 student with a bf16 or fp16 teacher
+  if (s != t && !(s == MAFED_F32 && (t == MAFED_BF16 || t == MAFED_F16))) return MAFED_E_DTYPE;
   if (sh->loss_kind != MAFED_LOSS_MSE && sh->loss_kind != MAFED_LOSS_COSINE) return MAFED_E_DTYPE;
   return 0;
 }
 
 inline size_t elem_size(int dtype) { return dtype == MAFED_F32 ? 4 : 2; }
+inline size_t student_size(const mafed_shape_t& sh) { return elem_size(student_dtype(sh)); }
+inline size_t teacher_size(const mafed_shape_t& sh) { return elem_size(teacher_dtype(sh)); }
 
 // Fill the geometry part of PathParams.  CLS mode (distillation.py:251-257) is the same path over
 // B rows (position 0 of every sample), all of them "visual", T*D elements apart.
@@ -122,10 +137,10 @@ inline int fill_params(const mafed_shape_t* shape, const void* const* student_pt
   memset(&p, 0, sizeof(p));
   fill_geometry(*shape, p);
   p.gout_scale = 1.f;
-  const size_t es = elem_size(shape->dtype);
+  const size_t es = student_size(*shape), et = teacher_size(*shape);
   for (int l = 0; l < shape->n_layers; ++l) {
     if (!student_ptrs[l] || !teacher_ptrs[l]) return MAFED_E_ARG;
-    if (!aligned_to(student_ptrs[l], es) || !aligned_to(teacher_ptrs[l], es)) return MAFED_E_ALIGN;
+    if (!aligned_to(student_ptrs[l], es) || !aligned_to(teacher_ptrs[l], et)) return MAFED_E_ALIGN;
     p.s[l] = student_ptrs[l];
     p.t[l] = teacher_ptrs[l];
     if (grad_ptrs) {
@@ -165,52 +180,53 @@ inline long long clamp_grid(long long grid, long long total) {
 #define MAFED_TAIL_LAUNCH(...)
 #endif
 
-template <typename T, int CPL, int RPI, int LOSS, int PASS>
+// TT (last parameter everywhere below): the teacher's element type, the student's unless the call passes a pair
+template <typename T, int CPL, int RPI, int LOSS, int PASS, typename TT>
 struct LdgKernel;
-template <typename T, int CPL, int RPI, int LOSS>
-struct LdgKernel<T, CPL, RPI, LOSS, kPassFwd> {
-  static auto host() { return &k_fwd_ldg<T, CPL, RPI, LOSS>; }
+template <typename T, int CPL, int RPI, int LOSS, typename TT>
+struct LdgKernel<T, CPL, RPI, LOSS, kPassFwd, TT> {
+  static auto host() { return &k_fwd_ldg<T, CPL, RPI, LOSS, TT>; }
 };
-template <typename T, int CPL, int RPI, int LOSS>
-struct LdgKernel<T, CPL, RPI, LOSS, kPassBwd> {
-  static auto host() { return &k_bwd_ldg<T, CPL, RPI, LOSS, kBackward>; }
-  MAFED_TAIL_LAUNCH(k_bwd_ldg<T, CPL, RPI, LOSS, kBackward>)
+template <typename T, int CPL, int RPI, int LOSS, typename TT>
+struct LdgKernel<T, CPL, RPI, LOSS, kPassBwd, TT> {
+  static auto host() { return &k_bwd_ldg<T, CPL, RPI, LOSS, kBackward, TT>; }
+  MAFED_TAIL_LAUNCH(k_bwd_ldg<T, CPL, RPI, LOSS, kBackward, TT>)
 };
-template <typename T, int CPL, int RPI, int LOSS>
-struct LdgKernel<T, CPL, RPI, LOSS, kPassFused> {
-  static auto host() { return &k_bwd_ldg<T, CPL, RPI, LOSS, kFused>; }
+template <typename T, int CPL, int RPI, int LOSS, typename TT>
+struct LdgKernel<T, CPL, RPI, LOSS, kPassFused, TT> {
+  static auto host() { return &k_bwd_ldg<T, CPL, RPI, LOSS, kFused, TT>; }
 };
 
-template <typename T, int LOSS, int PASS>
+template <typename T, int LOSS, int PASS, typename TT>
 struct TmaKernel;
-template <typename T, int LOSS>
-struct TmaKernel<T, LOSS, kPassFwd> {
-  static auto host() { return &k_fwd_tma<T, LOSS>; }
+template <typename T, int LOSS, typename TT>
+struct TmaKernel<T, LOSS, kPassFwd, TT> {
+  static auto host() { return &k_fwd_tma<T, LOSS, TT>; }
 };
-template <typename T, int LOSS>
-struct TmaKernel<T, LOSS, kPassBwd> {
-  static auto host() { return &k_bwd_tma<T, LOSS, kBackward>; }
-  MAFED_TAIL_LAUNCH(k_bwd_tma<T, LOSS, kBackward>)
+template <typename T, int LOSS, typename TT>
+struct TmaKernel<T, LOSS, kPassBwd, TT> {
+  static auto host() { return &k_bwd_tma<T, LOSS, kBackward, TT>; }
+  MAFED_TAIL_LAUNCH(k_bwd_tma<T, LOSS, kBackward, TT>)
 };
-template <typename T, int LOSS>
-struct TmaKernel<T, LOSS, kPassFused> {
-  static auto host() { return &k_bwd_tma<T, LOSS, kFused>; }
+template <typename T, int LOSS, typename TT>
+struct TmaKernel<T, LOSS, kPassFused, TT> {
+  static auto host() { return &k_bwd_tma<T, LOSS, kFused, TT>; }
 };
 
-template <typename T, int LOSS>
+template <typename T, int LOSS, typename TT>
 struct GenericFwdKernel {
-  static auto host() { return &k_fwd_generic<T, LOSS>; }
+  static auto host() { return &k_fwd_generic<T, LOSS, TT>; }
 };
-template <typename T, int LOSS>
+template <typename T, int LOSS, typename TT>
 struct GenericBwdKernel {
-  static auto host() { return &k_bwd_generic<T, LOSS>; }
-  MAFED_TAIL_LAUNCH(k_bwd_generic<T, LOSS>)
+  static auto host() { return &k_bwd_generic<T, LOSS, TT>; }
+  MAFED_TAIL_LAUNCH(k_bwd_generic<T, LOSS, TT>)
 };
 
-template <typename T, int CPL, int RPI, int LOSS, int PASS, typename Launcher>
+template <typename T, int CPL, int RPI, int LOSS, int PASS, typename TT, typename Launcher>
 int launch_ldg(const PathParams& p, const Launcher& go) {
   static_assert(LOSS != kLossL2Norm || PASS == kPassFwd, "the token-norm reduction has no backward");
-  using Kernel = LdgKernel<T, CPL, RPI, LOSS, PASS>;
+  using Kernel = LdgKernel<T, CPL, RPI, LOSS, PASS, TT>;
   static int occ[kMaxDevices] = {};   // per kernel and per device
   const DeviceInfo& dv = device_info();
   if (occ[dv.index] == 0) occ[dv.index] = blocks_per_sm(Kernel::host(), kLdgThreads, 0);
@@ -221,30 +237,35 @@ int launch_ldg(const PathParams& p, const Launcher& go) {
   return (int)cudaPeekAtLastError();
 }
 
-template <typename T, int LOSS, int PASS, typename Launcher>
+template <typename T, int LOSS, int PASS, typename TT, typename Launcher>
 int dispatch_ldg(const PathParams& p, const Launcher& go) {
-  const int cpl = (p.n_chunks + 31) / 32;
-  // rows per warp per iteration: more independent loads in flight for short rows; the cosine gradient keeps the row
-  // statistics and two coefficients per row as well, so it takes half as many rows at a time (with 4 / 2 it spilled
-  // 150-250 bytes per thread under the 128-register cap)
-  constexpr bool kHeavy = LOSS == MAFED_LOSS_COSINE && PASS != kPassFwd;
-  if (cpl <= 1) return launch_ldg<T, 1, kHeavy ? 2 : 4, LOSS, PASS>(p, go);
-  if (cpl <= 2) return launch_ldg<T, 2, kHeavy ? 2 : 4, LOSS, PASS>(p, go);
-  if (cpl <= 3) return launch_ldg<T, 3, kHeavy ? 1 : 2, LOSS, PASS>(p, go);
-  if (cpl <= 4) return launch_ldg<T, 4, kHeavy ? 1 : 2, LOSS, PASS>(p, go);
-  if (cpl <= 6) return launch_ldg<T, 6, 1, LOSS, PASS>(p, go);
-  return launch_ldg<T, 8, 1, LOSS, PASS>(p, go);  // multi-pass for rows longer than 4 KB
+  // a half-precision teacher under an fp32 student: the multi-pass class only (its guards cover any row length)
+  if constexpr (!std::is_same<T, TT>::value) {
+    return launch_ldg<T, 8, 1, LOSS, PASS, TT>(p, go);
+  } else {
+    const int cpl = (p.n_chunks + 31) / 32;
+    // rows per warp per iteration: more independent loads in flight for short rows; the cosine gradient keeps the
+    // row statistics and two coefficients per row as well, so it takes half as many rows at a time (with 4 / 2 it
+    // spilled 150-250 bytes per thread under the 128-register cap)
+    constexpr bool kHeavy = LOSS == MAFED_LOSS_COSINE && PASS != kPassFwd;
+    if (cpl <= 1) return launch_ldg<T, 1, kHeavy ? 2 : 4, LOSS, PASS, TT>(p, go);
+    if (cpl <= 2) return launch_ldg<T, 2, kHeavy ? 2 : 4, LOSS, PASS, TT>(p, go);
+    if (cpl <= 3) return launch_ldg<T, 3, kHeavy ? 1 : 2, LOSS, PASS, TT>(p, go);
+    if (cpl <= 4) return launch_ldg<T, 4, kHeavy ? 1 : 2, LOSS, PASS, TT>(p, go);
+    if (cpl <= 6) return launch_ldg<T, 6, 1, LOSS, PASS, TT>(p, go);
+    return launch_ldg<T, 8, 1, LOSS, PASS, TT>(p, go);  // multi-pass for rows longer than 4 KB
+  }
 }
 
 // Any D / any alignment: element-wise kernels.  The fused pass is simply forward then backward.
-template <typename T, int LOSS, int PASS, typename Launcher>
+template <typename T, int LOSS, int PASS, typename TT, typename Launcher>
 int launch_generic(const mafed_shape_t& sh, const PathParams& p, const Launcher& go) {
   const DeviceInfo& dv = device_info();
   const long long total = ((p.n_rows + kLdgWarps - 1) / kLdgWarps) * p.n_layers;
   const unsigned grid = (unsigned)clamp_grid((long long)dv.sm_count * 4, total);
-  if constexpr (PASS == kPassFwd || PASS == kPassFused) go.template run<GenericFwdKernel<T, LOSS>>(grid, kLdgThreads, 0, p);
+  if constexpr (PASS == kPassFwd || PASS == kPassFused) go.template run<GenericFwdKernel<T, LOSS, TT>>(grid, kLdgThreads, 0, p);
   if constexpr (LOSS != kLossL2Norm && (PASS == kPassBwd || PASS == kPassFused))
-    go.template run<GenericBwdKernel<T, LOSS>>(grid, kLdgThreads, 0, p, PASS == kPassFused ? 1 : 0);
+    go.template run<GenericBwdKernel<T, LOSS, TT>>(grid, kLdgThreads, 0, p, PASS == kPassFused ? 1 : 0);
   return (int)cudaPeekAtLastError();
 }
 
@@ -252,6 +273,16 @@ inline bool tma_geometry(const mafed_shape_t& sh, const PathParams& p, int pass,
   const DeviceInfo& dv = device_info();
   const long long row_bytes = (long long)p.n_chunks * 16;
   if (row_bytes > 32768) return false;
+  // bytes of one row of student and teacher together: what a stage holds per row
+  long long pair_bytes = 2 * row_bytes;
+  if (mixed_pair(sh)) {
+    // cp.async.bulk moves multiples of 16 bytes between 16-byte aligned addresses: the half-precision teacher rows
+    // (2 * D bytes) must be whole 16-byte chunks too
+    if (sh.D % 8 != 0 || (p.row_stride * 2) % 16 != 0) return false;
+    for (int l = 0; l < sh.n_layers; ++l)
+      if (!aligned_to(p.t[l], 16)) return false;
+    pair_bytes = row_bytes + row_bytes / 2;
+  }
   const long long budget = (long long)dv.smem_optin - 16 * 1024;  // static smem + slack
   // Measured on B200 (profiles/r02l_geometry_sweep.txt: one-pass step, 13 shapes x 13 rings; r02q_geometry_sweep_
   // {fwd,bwd}.txt: the two passes; all after the producer stopped paying 64-bit divisions and the mask round trip
@@ -272,14 +303,14 @@ inline bool tma_geometry(const mafed_shape_t& sh, const PathParams& p, int pass,
   const bool cosine_fine = !wide && loss == MAFED_LOSS_COSINE;
   const bool fused_fine = !wide && !cosine_fine && !text_heavy;
   const long long stage_target = wide ? 96 * 1024 : ((cosine_fine || fused_fine) ? 32 * 1024 : 72 * 1024);
-  int rows = (int)(stage_target / (2 * row_bytes));
+  int rows = (int)(stage_target / pair_bytes);
   if (rows >= 8 && !wide && !cosine_fine && !fused_fine) rows &= ~7;
   if (rows > kTmaMaxRows) rows = kTmaMaxRows;
   if (rows < 1) rows = 1;
-  if (2 * rows * row_bytes > budget) rows = (int)(budget / (2 * row_bytes));
+  if (rows * pair_bytes > budget) rows = (int)(budget / pair_bytes);
   if (rows < 1) return false;
   geo.rows = rows;
-  geo.stage_bytes = (int)(2 * rows * row_bytes);
+  geo.stage_bytes = (int)(rows * pair_bytes);
   int stages = cosine_fine ? 4 : (fused_fine ? 3 : ((wide || 2 * geo.stage_bytes >= 96 * 1024) ? 2 : 3));
   if (stages > kTmaMaxStages) stages = kTmaMaxStages;
   while (stages > 1 && (long long)stages * geo.stage_bytes > budget) --stages;
@@ -292,10 +323,10 @@ inline bool tma_geometry(const mafed_shape_t& sh, const PathParams& p, int pass,
   return true;
 }
 
-template <typename T, int LOSS, int PASS, typename Launcher>
+template <typename T, int LOSS, int PASS, typename TT, typename Launcher>
 int launch_tma(const PathParams& p, const TmaGeom& geo, const Launcher& go) {
   static_assert(LOSS != kLossL2Norm || PASS == kPassFwd, "the token-norm reduction has no backward");
-  using Kernel = TmaKernel<T, LOSS, PASS>;
+  using Kernel = TmaKernel<T, LOSS, PASS, TT>;
   // the opt-in shared-memory size is a per-device function attribute: remember it per kernel and device
   static bool attr_set[kMaxDevices] = {};
   const DeviceInfo& dv = device_info();
@@ -312,11 +343,13 @@ int launch_tma(const PathParams& p, const TmaGeom& geo, const Launcher& go) {
 }
 
 inline bool vector_path(const mafed_shape_t& sh, const PathParams& p, int pass) {
-  // vector kernels: rows are whole, 16-byte aligned chunks
-  const size_t es = elem_size(sh.dtype);
+  // vector kernels: student (and gradient) rows are whole, 16-byte aligned chunks; the teacher's matching share of a
+  // chunk (16 bytes, or 8 for a half-precision teacher under an fp32 student) is aligned to its size
+  const size_t es = student_size(sh);
+  const size_t t_align = 16 * teacher_size(sh) / es;
   bool ok = ((size_t)sh.D * es) % 16 == 0 && ((size_t)p.row_stride * es) % 16 == 0;
   for (int l = 0; l < sh.n_layers && ok; ++l)
-    ok = aligned_to(p.s[l], 16) && aligned_to(p.t[l], 16) && (pass == kPassFwd || aligned_to(p.g[l], 16));
+    ok = aligned_to(p.s[l], 16) && aligned_to(p.t[l], t_align) && (pass == kPassFwd || aligned_to(p.g[l], 16));
   return ok;
 }
 
@@ -325,34 +358,38 @@ inline int chosen_variant(const mafed_shape_t& sh) {
   return variant == 0 ? 2 : variant;   // 1 ldg, 2 tma (default)
 }
 
-template <typename T, int LOSS, int PASS, typename Launcher>
+template <typename T, int LOSS, int PASS, typename TT, typename Launcher>
 int dispatch_typed(const mafed_shape_t& sh, PathParams& p, bool vector_ok, const Launcher& go) {
-  if (!vector_ok) return launch_generic<T, LOSS, PASS>(sh, p, go);
+  if (!vector_ok) return launch_generic<T, LOSS, PASS, TT>(sh, p, go);
   if (chosen_variant(sh) == 2) {
     TmaGeom geo;
-    if (tma_geometry(sh, p, PASS, geo, LOSS)) return launch_tma<T, LOSS, PASS>(p, geo, go);
+    if (tma_geometry(sh, p, PASS, geo, LOSS)) return launch_tma<T, LOSS, PASS, TT>(p, geo, go);
   }
-  return dispatch_ldg<T, LOSS, PASS>(p, go);
+  return dispatch_ldg<T, LOSS, PASS, TT>(p, go);
 }
 
-template <typename T, int PASS, typename Launcher>
+template <typename T, int PASS, typename TT, typename Launcher>
 int dispatch_loss(const mafed_shape_t& sh, PathParams& p, int loss, bool vector_ok, const Launcher& go) {
-  if (loss == MAFED_LOSS_MSE) return dispatch_typed<T, MAFED_LOSS_MSE, PASS>(sh, p, vector_ok, go);
-  if constexpr (PASS == kPassFwd) {
-    if (loss == kLossL2Norm) return dispatch_typed<T, kLossL2Norm, PASS>(sh, p, vector_ok, go);
+  if (loss == MAFED_LOSS_MSE) return dispatch_typed<T, MAFED_LOSS_MSE, PASS, TT>(sh, p, vector_ok, go);
+  if constexpr (PASS == kPassFwd && std::is_same<T, TT>::value) {   // (single input: never a pair)
+    if (loss == kLossL2Norm) return dispatch_typed<T, kLossL2Norm, PASS, TT>(sh, p, vector_ok, go);
   }
-  return dispatch_typed<T, MAFED_LOSS_COSINE, PASS>(sh, p, vector_ok, go);
+  return dispatch_typed<T, MAFED_LOSS_COSINE, PASS, TT>(sh, p, vector_ok, go);
 }
 
 template <int PASS, typename Launcher>
 int dispatch(const mafed_shape_t& sh, PathParams& p, const Launcher& go, int loss_override = -1) {
   const bool vector_ok = vector_path(sh, p, PASS);
-  p.n_chunks = vector_ok ? (int)((size_t)sh.D * elem_size(sh.dtype) / 16) : 0;
+  p.n_chunks = vector_ok ? (int)((size_t)sh.D * student_size(sh) / 16) : 0;
   const int loss = loss_override >= 0 ? loss_override : sh.loss_kind;
-  switch (sh.dtype) {
-    case MAFED_F32: return dispatch_loss<float, PASS>(sh, p, loss, vector_ok, go);
-    case MAFED_BF16: return dispatch_loss<__nv_bfloat16, PASS>(sh, p, loss, vector_ok, go);
-    default: return dispatch_loss<__half, PASS>(sh, p, loss, vector_ok, go);
+  if (mixed_pair(sh)) {   // check_shape admits only an fp32 student with a bf16 or fp16 teacher
+    if (teacher_dtype(sh) == MAFED_BF16) return dispatch_loss<float, PASS, __nv_bfloat16>(sh, p, loss, vector_ok, go);
+    return dispatch_loss<float, PASS, __half>(sh, p, loss, vector_ok, go);
+  }
+  switch (student_dtype(sh)) {
+    case MAFED_F32: return dispatch_loss<float, PASS, float>(sh, p, loss, vector_ok, go);
+    case MAFED_BF16: return dispatch_loss<__nv_bfloat16, PASS, __nv_bfloat16>(sh, p, loss, vector_ok, go);
+    default: return dispatch_loss<__half, PASS, __half>(sh, p, loss, vector_ok, go);
   }
 }
 
@@ -360,7 +397,7 @@ int dispatch(const mafed_shape_t& sh, PathParams& p, const Launcher& go, int los
 inline bool uses_tma(const mafed_shape_t& sh, const PathParams& p, int pass) {
   if (!vector_path(sh, p, pass) || chosen_variant(sh) != 2) return false;
   PathParams q = p;
-  q.n_chunks = (int)((size_t)sh.D * elem_size(sh.dtype) / 16);
+  q.n_chunks = (int)((size_t)sh.D * student_size(sh) / 16);
   TmaGeom geo;
   return tma_geometry(sh, q, pass, geo, MAFED_LOSS_MSE);   // eligibility does not depend on the loss kind
 }

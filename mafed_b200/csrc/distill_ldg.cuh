@@ -13,9 +13,12 @@ constexpr int kLdgMinBlocksBwd = 2;   // backward keeps a whole row pair in regi
 
 // CPL : 16-byte chunks per lane per pass (a pass covers 32*CPL chunks of a row)
 // RPI : rows per warp per iteration (more independent loads in flight for short rows)
-template <typename T, int CPL, int RPI, int LOSS>
+// TT: the teacher's element type (TeacherChunk: the teacher's share of a 16-byte student chunk)
+template <typename T, int CPL, int RPI, int LOSS, typename TT = T>
 __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocks) k_fwd_ldg(const __grid_constant__ PathParams p) {
   constexpr int NE = Pack<T>::kPer16;
+  using Tch = TeacherChunk<T, TT>;
+  using TV = typename Tch::Vec;
   __shared__ CtaSums<kLdgWarps> sums;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   cta_sums_zero(sums, p.n_layers);
@@ -28,6 +31,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocks) k_fwd_ldg(const __
   const long long total = groups_per_layer * p.n_layers;
   const int n_pass = (CPL == 8) ? (p.n_chunks + 32 * CPL - 1) / (32 * CPL) : 1;
   const long long row_bytes = p.row_stride * (long long)sizeof(T);
+  const long long t_row_bytes = p.row_stride * (long long)sizeof(TT);
 
   float acc_text = 0.f, acc_vis = 0.f;
   int cur = -1;
@@ -55,17 +59,19 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocks) k_fwd_ldg(const __
     for (int r = 0; r < RPI; ++r) x[r] = y[r] = z[r] = 0.f;
 
     for (int pass = 0; pass < n_pass; ++pass) {
-      uint4 sv[RPI][CPL], tv[RPI][CPL];
+      uint4 sv[RPI][CPL];
+      TV tv[RPI][CPL];
 #pragma unroll
       for (int r = 0; r < RPI; ++r) {
         const long long off = (row0 + r) * row_bytes;
+        const long long t_off = (row0 + r) * t_row_bytes;
 #pragma unroll
         for (int i = 0; i < CPL; ++i) {
           const int c = pass * 32 * CPL + lane + 32 * i;
-          tv[r][i] = make_uint4(0, 0, 0, 0);
+          tv[r][i] = TV{};
           if (w[r] != 0.f && c < p.n_chunks) {
             sv[r][i] = ldg_stream(sb + off + (long long)c * 16);
-            if (LOSS != kLossL2Norm) tv[r][i] = ldg_stream(tb + off + (long long)c * 16);
+            if (LOSS != kLossL2Norm) tv[r][i] = Tch::ldg(tb + t_off + (long long)c * Tch::kBytes);
           } else {
             sv[r][i] = make_uint4(0, 0, 0, 0);
           }
@@ -77,7 +83,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocks) k_fwd_ldg(const __
         for (int i = 0; i < CPL; ++i) {
           float a[NE], b[NE];
           Pack<T>::unpack(sv[r][i], a);
-          Pack<T>::unpack(tv[r][i], b);
+          Tch::unpack(tv[r][i], b);
           accumulate<LOSS, NE>(a, b, x[r], y[r], z[r]);
         }
       }
@@ -126,9 +132,11 @@ __device__ __forceinline__ bool upstream_grad(const PathParams& p, float& gout) 
 // MODE = kBackward: gradients only (2 reads + 1 write), work items walked last-to-first so that the pass starts on
 // the rows the forward left in L2.  MODE = kFused: the same pass also accumulates the forward's [layer][modality]
 // loss sums, so student and teacher are read once per step.
-template <typename T, int CPL, int RPI, int LOSS, int MODE>
+template <typename T, int CPL, int RPI, int LOSS, int MODE, typename TT = T>
 __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const __grid_constant__ PathParams p) {
   constexpr int NE = Pack<T>::kPer16;
+  using Tch = TeacherChunk<T, TT>;
+  using TV = typename Tch::Vec;
   constexpr bool FUSED = MODE == kFused;
   __shared__ CtaSums<FUSED ? kLdgWarps : 1> sums;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -145,6 +153,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
   const long long total = groups_per_layer * p.n_layers;
   const int n_pass = (CPL == 8) ? (p.n_chunks + 32 * CPL - 1) / (32 * CPL) : 1;
   const long long row_bytes = p.row_stride * (long long)sizeof(T);
+  const long long t_row_bytes = p.row_stride * (long long)sizeof(TT);
 
   float acc_text = 0.f, acc_vis = 0.f;
   int cur = -1;
@@ -188,10 +197,11 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
         if (wraw[r] == 0.f) continue;
         float x = 0.f, y = 0.f, z = 0.f;
         const long long off = (row0 + r) * row_bytes;
+        const long long t_off = (row0 + r) * t_row_bytes;
         for (int c = lane; c < p.n_chunks; c += 32) {
           float a[NE], b[NE];
           Pack<T>::unpack(ldg_stream(sb + off + (long long)c * 16), a);
-          Pack<T>::unpack(ldg_stream(tb + off + (long long)c * 16), b);
+          Tch::unpack(Tch::ldg(tb + t_off + (long long)c * Tch::kBytes), b);
           accumulate<LOSS, NE>(a, b, x, y, z);
         }
         x = warp_sum(x); y = warp_sum(y); z = warp_sum(z);
@@ -203,19 +213,21 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
     }
 
     for (int pass = 0; pass < n_pass; ++pass) {
-      uint4 sv[RPI][CPL], tv[RPI][CPL];
+      uint4 sv[RPI][CPL];
+      TV tv[RPI][CPL];
 #pragma unroll
       for (int r = 0; r < RPI; ++r) {
         const long long off = (row0 + r) * row_bytes;
+        const long long t_off = (row0 + r) * t_row_bytes;
 #pragma unroll
         for (int i = 0; i < CPL; ++i) {
           const int c = pass * 32 * CPL + lane + 32 * i;
           if (wraw[r] != 0.f && c < p.n_chunks) {
             sv[r][i] = ldg_stream(sb + off + (long long)c * 16);
-            tv[r][i] = ldg_stream(tb + off + (long long)c * 16);
+            tv[r][i] = Tch::ldg(tb + t_off + (long long)c * Tch::kBytes);
           } else {
             sv[r][i] = make_uint4(0, 0, 0, 0);
-            tv[r][i] = make_uint4(0, 0, 0, 0);
+            tv[r][i] = TV{};
           }
         }
       }
@@ -227,7 +239,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
           for (int i = 0; i < CPL; ++i) {
             float a[NE], b[NE];
             Pack<T>::unpack(sv[r][i], a);
-            Pack<T>::unpack(tv[r][i], b);
+            Tch::unpack(tv[r][i], b);
             accumulate<LOSS, NE>(a, b, x, y, z);
           }
           x = warp_sum(x); y = warp_sum(y); z = warp_sum(z);
@@ -247,7 +259,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
           if (c >= p.n_chunks) continue;
           float a[NE], b[NE], o[NE];
           Pack<T>::unpack(sv[r][i], a);
-          Pack<T>::unpack(tv[r][i], b);
+          Tch::unpack(tv[r][i], b);
           if (FUSED && LOSS == MAFED_LOSS_MSE) {
             float y = 0.f, z = 0.f;
             accumulate<LOSS, NE>(a, b, rowval[r], y, z);  // lane-partial sum of (h-p)^2
@@ -280,7 +292,7 @@ __global__ void __launch_bounds__(kLdgThreads, kLdgMinBlocksBwd) k_bwd_ldg(const
 
 // ---------------------------------------------------------------- generic fallback (any D, any alignment)
 // Element-wise loads; used only when a row is not a whole number of aligned 16-byte chunks.
-template <typename T, int LOSS>
+template <typename T, int LOSS, typename TT = T>
 __global__ void __launch_bounds__(kLdgThreads) k_fwd_generic(const __grid_constant__ PathParams p) {
   __shared__ CtaSums<kLdgWarps> sums;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -307,7 +319,7 @@ __global__ void __launch_bounds__(kLdgThreads) k_fwd_generic(const __grid_consta
     float x = 0.f, y = 0.f, z = 0.f;
     for (int d = lane; d < p.D; d += 32) {
       float a[1] = {Pack<T>::load1(p.s[l], row * p.row_stride + d)};
-      float b[1] = {Pack<T>::load1(p.t[l], row * p.row_stride + d)};
+      float b[1] = {Pack<TT>::load1(p.t[l], row * p.row_stride + d)};
       accumulate<LOSS, 1>(a, b, x, y, z);
     }
     x = warp_sum(x); y = warp_sum(y); z = warp_sum(z);
@@ -320,7 +332,7 @@ __global__ void __launch_bounds__(kLdgThreads) k_fwd_generic(const __grid_consta
   cta_sums_store(sums, p.ws, p.n_layers, 0, kLdgThreads);
 }
 
-template <typename T, int LOSS>
+template <typename T, int LOSS, typename TT = T>
 __global__ void __launch_bounds__(kLdgThreads) k_bwd_generic(const __grid_constant__ PathParams p, int use_fixed_gout) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long groups_per_layer = (p.n_rows + kLdgWarps - 1) / kLdgWarps;
@@ -342,7 +354,7 @@ __global__ void __launch_bounds__(kLdgThreads) k_bwd_generic(const __grid_consta
       float x = 0.f, y = 0.f, z = 0.f;
       for (int d = lane; d < p.D; d += 32) {
         float a[1] = {Pack<T>::load1(p.s[l], row * p.row_stride + d)};
-        float b[1] = {Pack<T>::load1(p.t[l], row * p.row_stride + d)};
+        float b[1] = {Pack<TT>::load1(p.t[l], row * p.row_stride + d)};
         accumulate<LOSS, 1>(a, b, x, y, z);
       }
       x = warp_sum(x); y = warp_sum(y); z = warp_sum(z);
@@ -354,7 +366,7 @@ __global__ void __launch_bounds__(kLdgThreads) k_bwd_generic(const __grid_consta
       float o[1] = {w};
       if (wraw != 0.f) {
         float a[1] = {Pack<T>::load1(p.s[l], row * p.row_stride + d)};
-        float b[1] = {Pack<T>::load1(p.t[l], row * p.row_stride + d)};
+        float b[1] = {Pack<TT>::load1(p.t[l], row * p.row_stride + d)};
         grad_elems<LOSS, 1>(a, b, w, ch, cp, o);
       }
       Pack<T>::store1(p.g[l], row * p.row_stride + d, o[0]);

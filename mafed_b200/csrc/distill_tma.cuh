@@ -3,6 +3,8 @@
 // read the staged rows with conflict-free 128-bit shared loads.  One persistent CTA per SM; the ring
 // keeps up to ~190 KB per SM in flight without spending registers on it.
 #pragma once
+#include <type_traits>
+
 #include "distill_comm.cuh"
 #include "distill_common.cuh"
 #include "distill_epilogue.cuh"
@@ -20,7 +22,7 @@ constexpr unsigned kTmaPaceNs = 500;  // refill pause of a paced ring (see tma_g
 struct TmaGeom {
   int stages;
   int rows;         // rows per stage
-  int stage_bytes;  // 2 * rows * row_bytes
+  int stage_bytes;  // rows * (student row bytes + teacher row bytes)
   int pace;         // 1: the producer pauses kTmaPaceNs between a slot becoming free and its refill, as long as this
                     // CTA has met no padded row (the batch looks dense)
 };
@@ -68,21 +70,33 @@ __device__ __forceinline__ uint4 lds_128(uint32_t addr) {
   asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
   return r;
 }
+__device__ __forceinline__ uint2 lds_64(uint32_t addr) {
+  uint2 r;
+  asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(r.x), "=r"(r.y) : "r"(addr));
+  return r;
+}
+// the teacher's share of a staged chunk (TeacherChunk::Vec): LDS.128, or LDS.64 for a half-precision teacher
+template <typename V> __device__ __forceinline__ V lds_vec(uint32_t addr);
+template <> __device__ __forceinline__ uint4 lds_vec<uint4>(uint32_t addr) { return lds_128(addr); }
+template <> __device__ __forceinline__ uint2 lds_vec<uint2>(uint32_t addr) { return lds_64(addr); }
 __device__ __forceinline__ void named_bar_sync(int id, int n_threads) {
   asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(n_threads) : "memory");
 }
 
 // ---------------------------------------------------------------- producer
 // All 32 lanes of the producer warp run this; lane r owns row r of every stage.  The backward walks its tiles
-// last-to-first, so that it starts on the rows the forward left in L2.
-template <typename T>
+// last-to-first, so that it starts on the rows the forward left in L2.  A stage holds its rows' student bytes, then
+// their teacher bytes (TT: the teacher's element type; its rows are row_bytes >> TeacherChunk::kShift long).
+template <typename T, typename TT>
 __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom& geo, unsigned char* data,
                                              uint64_t* full, uint64_t* empty, TmaStageMeta* meta, int lane,
                                              bool for_backward) {
   const long long tiles_per_layer = (p.n_rows + geo.rows - 1) / geo.rows;
   const long long total = tiles_per_layer * p.n_layers;
   const uint32_t row_bytes = (uint32_t)p.n_chunks * 16u;
+  const uint32_t t_row_bytes = row_bytes >> TeacherChunk<T, TT>::kShift;
   const long long row_pitch = p.row_stride * (long long)sizeof(T);
+  const long long t_row_pitch = p.row_stride * (long long)sizeof(TT);
   const bool contiguous = row_pitch == (long long)row_bytes;
   int stage = 0;
   uint32_t phase = 0;
@@ -143,21 +157,25 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
     __syncwarp();
     const uint32_t bar = smem_u32(&full[stage]);
     const bool both = !p.single_input;
-    if (lane == 0) mbar_arrive_expect_tx(bar, (uint32_t)__popc(valid) * (both ? 2u : 1u) * row_bytes);
+    if (lane == 0) {
+      const uint32_t live_bytes = std::is_same<T, TT>::value ? (both ? 2u : 1u) * row_bytes
+                                                             : row_bytes + (both ? t_row_bytes : 0u);
+      mbar_arrive_expect_tx(bar, (uint32_t)__popc(valid) * live_bytes);
+    }
     __syncwarp();
     const uint32_t s_dst = smem_u32(data + (size_t)stage * geo.stage_bytes);
     const uint32_t t_dst = s_dst + (uint32_t)geo.rows * row_bytes;
     const char* sb = reinterpret_cast<const char*>(p.s[l]) + row0 * row_pitch;
-    const char* tb = reinterpret_cast<const char*>(p.t[l]) + row0 * row_pitch;
+    const char* tb = reinterpret_cast<const char*>(p.t[l]) + row0 * t_row_pitch;
     const unsigned all = (n_rows >= 32) ? 0xffffffffu : ((1u << n_rows) - 1u);
     if (contiguous && valid == all) {
       // whole tile live: one bulk copy per tensor
       if (lane == 0) bulk_g2s(s_dst, sb, (uint32_t)n_rows * row_bytes, bar);
-      if (lane == 1 && both) bulk_g2s(t_dst, tb, (uint32_t)n_rows * row_bytes, bar);
+      if (lane == 1 && both) bulk_g2s(t_dst, tb, (uint32_t)n_rows * t_row_bytes, bar);
     } else if (w != 0.f) {
       // ragged tile: only live rows are fetched (padded text rows cost no bandwidth)
       bulk_g2s(s_dst + (uint32_t)lane * row_bytes, sb + (long long)lane * row_pitch, row_bytes, bar);
-      if (both) bulk_g2s(t_dst + (uint32_t)lane * row_bytes, tb + (long long)lane * row_pitch, row_bytes, bar);
+      if (both) bulk_g2s(t_dst + (uint32_t)lane * t_row_bytes, tb + (long long)lane * t_row_pitch, t_row_bytes, bar);
     }
     if (++stage == geo.stages) { stage = 0; phase ^= 1u; }
   }
@@ -234,10 +252,12 @@ __device__ __forceinline__ void tma_tail(const PathParams& p, const double* coun
 }
 
 // ---------------------------------------------------------------- forward
-template <typename T, int LOSS>
+template <typename T, int LOSS, typename TT = T>
 __global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
 k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo) {
   constexpr int NE = Pack<T>::kPer16;
+  using Tch = TeacherChunk<T, TT>;
+  using TV = typename Tch::Vec;
   extern __shared__ __align__(128) unsigned char dyn_smem[];
   __shared__ TmaSmem sm;
   __shared__ CtaSums<kTmaConsumerWarps> sums;
@@ -246,12 +266,13 @@ k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
   tma_prologue(sm, geo);
 
   if (warp == kTmaConsumerWarps) {
-    tma_producer<T>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, false);
+    tma_producer<T, TT>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, false);
     return;
   }
   const long long tiles_per_layer = (p.n_rows + geo.rows - 1) / geo.rows;
   const long long total = tiles_per_layer * p.n_layers;
   const uint32_t row_bytes = (uint32_t)p.n_chunks * 16u;
+  const uint32_t t_row_bytes = row_bytes >> Tch::kShift;
   float acc_text = 0.f, acc_vis = 0.f;
   int cur = -1, stage = 0;
   uint32_t phase = 0;
@@ -273,21 +294,23 @@ k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     for (int r = first; r < mt.n_rows; r += kTmaConsumerWarps) {
       const float w = mt.w[r];
       if (w == 0.f) continue;
-      const uint32_t sa = s_base + (uint32_t)r * row_bytes, ta = t_base + (uint32_t)r * row_bytes;
+      const uint32_t sa = s_base + (uint32_t)r * row_bytes, ta = t_base + (uint32_t)r * t_row_bytes;
       float x = 0.f, y = 0.f, z = 0.f;
       int c = lane;
       for (; c + 96 < p.n_chunks; c += 128) {
-        uint4 sv[4], tv[4];
+        uint4 sv[4];
+        TV tv[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
           sv[u] = lds_128(sa + (uint32_t)(c + 32 * u) * 16u);
-          tv[u] = (LOSS == kLossL2Norm) ? sv[u] : lds_128(ta + (uint32_t)(c + 32 * u) * 16u);
+          if constexpr (LOSS == kLossL2Norm) tv[u] = sv[u];
+          else tv[u] = lds_vec<TV>(ta + (uint32_t)(c + 32 * u) * (uint32_t)Tch::kBytes);
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
           float a[NE], b[NE];
           Pack<T>::unpack(sv[u], a);
-          Pack<T>::unpack(tv[u], b);
+          Tch::unpack(tv[u], b);
           accumulate<LOSS, NE>(a, b, x, y, z);
         }
       }
@@ -295,7 +318,8 @@ k_fwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
         float a[NE], b[NE];
         const uint4 sv1 = lds_128(sa + (uint32_t)c * 16u);
         Pack<T>::unpack(sv1, a);
-        Pack<T>::unpack((LOSS == kLossL2Norm) ? sv1 : lds_128(ta + (uint32_t)c * 16u), b);
+        if constexpr (LOSS == kLossL2Norm) Tch::unpack(sv1, b);
+        else Tch::unpack(lds_vec<TV>(ta + (uint32_t)c * (uint32_t)Tch::kBytes), b);
         accumulate<LOSS, NE>(a, b, x, y, z);
       }
       float val;
@@ -409,11 +433,15 @@ __device__ __forceinline__ float cosine_row_unrolled(uint32_t sa, uint32_t ta, i
 
 // MODE = kBackward: gradients only.  MODE = kFused: the consumers also accumulate the forward's loss
 // sums from the rows they already hold in shared memory (one pass over student and teacher per step).
-template <typename T, int LOSS, int MODE>
+template <typename T, int LOSS, int MODE, typename TT = T>
 __global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
 k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo) {
   constexpr int NE = Pack<T>::kPer16;
   constexpr bool FUSED = MODE == kFused;
+  // a half-precision teacher under an fp32 student: no unrolled short-row cosine forms (general two-sweep loop)
+  constexpr bool kSameType = std::is_same<T, TT>::value;
+  using Tch = TeacherChunk<T, TT>;
+  using TV = typename Tch::Vec;
   extern __shared__ __align__(128) unsigned char dyn_smem[];
   __shared__ TmaSmem sm;
   __shared__ CtaSums<FUSED ? kTmaConsumerWarps : 1> sums;
@@ -428,7 +456,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     if (p.skip_if_gout_equals && gout == p.fixed_gout) return;  // fix-up launch with nothing to fix
   }
   if (warp == kTmaConsumerWarps) {
-    tma_producer<T>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, !FUSED);
+    tma_producer<T, TT>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, !FUSED);
     return;
   }
   // Scale table in shared memory.  One-pass step with the prologue folded in: while the producer's first
@@ -542,6 +570,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
   const long long tiles_per_layer = (p.n_rows + geo.rows - 1) / geo.rows;
   const long long total = tiles_per_layer * p.n_layers;
   const uint32_t row_bytes = (uint32_t)p.n_chunks * 16u;
+  const uint32_t t_row_bytes = row_bytes >> Tch::kShift;
   const long long row_pitch = p.row_stride * (long long)sizeof(T);
   float acc_text = 0.f, acc_vis = 0.f;
   int cur = -1;
@@ -575,26 +604,28 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
             for (int c = lane; c < p.n_chunks; c += 32) stg_128(grow + (long long)c * 16, fill);
           continue;
         }
-        const uint32_t sa = s_base + (uint32_t)r * row_bytes, ta = t_base + (uint32_t)r * row_bytes;
+        const uint32_t sa = s_base + (uint32_t)r * row_bytes, ta = t_base + (uint32_t)r * t_row_bytes;
         float ch = 0.f, cp = 0.f, rowval = 0.f;
-        if (LOSS == MAFED_LOSS_COSINE && (p.n_chunks == 96 || p.n_chunks == 128 || p.n_chunks == 192)) {
-          // short rows (1.5 / 2 / 3 KB: base and 410M hidden sizes in bf16, base in fp32): fully unrolled forms
-          float val;
-          if (p.n_chunks == 96) val = cosine_row_unrolled<T, 3, true>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
-          else if (p.n_chunks == 128) val = cosine_row_unrolled<T, 4, false>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
-          else val = cosine_row_unrolled<T, 6, false>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
-          if (FUSED && lane == 0) {
-            if (mt.mod[r] == 0) acc_text = fmaf(mt.w[r], val, acc_text);
-            else acc_vis = fmaf(mt.w[r], val, acc_vis);
+        if constexpr (kSameType) {
+          if (LOSS == MAFED_LOSS_COSINE && (p.n_chunks == 96 || p.n_chunks == 128 || p.n_chunks == 192)) {
+            // short rows (1.5 / 2 / 3 KB: base and 410M hidden sizes in bf16, base in fp32): fully unrolled forms
+            float val;
+            if (p.n_chunks == 96) val = cosine_row_unrolled<T, 3, true>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
+            else if (p.n_chunks == 128) val = cosine_row_unrolled<T, 4, false>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
+            else val = cosine_row_unrolled<T, 6, false>(sa, ta, lane, w, gb != nullptr ? grow : nullptr);
+            if (FUSED && lane == 0) {
+              if (mt.mod[r] == 0) acc_text = fmaf(mt.w[r], val, acc_text);
+              else acc_vis = fmaf(mt.w[r], val, acc_vis);
+            }
+            continue;
           }
-          continue;
         }
         if (LOSS == MAFED_LOSS_COSINE) {
           float x = 0.f, y = 0.f, z = 0.f;
           for (int c = lane; c < p.n_chunks; c += 32) {
             float a[NE], b[NE];
             Pack<T>::unpack(lds_128(sa + (uint32_t)c * 16u), a);
-            Pack<T>::unpack(lds_128(ta + (uint32_t)c * 16u), b);
+            Tch::unpack(lds_vec<TV>(ta + (uint32_t)c * (uint32_t)Tch::kBytes), b);
             accumulate<LOSS, NE>(a, b, x, y, z);
           }
           x = warp_sum(x); y = warp_sum(y); z = warp_sum(z);
@@ -605,17 +636,18 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
         }
         int c = lane;
         for (; c + 96 < p.n_chunks; c += 128) {
-          uint4 sv[4], tv[4];
+          uint4 sv[4];
+          TV tv[4];
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             sv[u] = lds_128(sa + (uint32_t)(c + 32 * u) * 16u);
-            tv[u] = lds_128(ta + (uint32_t)(c + 32 * u) * 16u);
+            tv[u] = lds_vec<TV>(ta + (uint32_t)(c + 32 * u) * (uint32_t)Tch::kBytes);
           }
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             float a[NE], b[NE], o[NE];
             Pack<T>::unpack(sv[u], a);
-            Pack<T>::unpack(tv[u], b);
+            Tch::unpack(tv[u], b);
             if (FUSED && LOSS == MAFED_LOSS_MSE) {
               float y = 0.f, z = 0.f;
               accumulate<LOSS, NE>(a, b, rowval, y, z);
@@ -627,7 +659,7 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
         for (; c < p.n_chunks; c += 32) {
           float a[NE], b[NE], o[NE];
           Pack<T>::unpack(lds_128(sa + (uint32_t)c * 16u), a);
-          Pack<T>::unpack(lds_128(ta + (uint32_t)c * 16u), b);
+          Tch::unpack(lds_vec<TV>(ta + (uint32_t)c * (uint32_t)Tch::kBytes), b);
           if (FUSED && LOSS == MAFED_LOSS_MSE) {
             float y = 0.f, z = 0.f;
             accumulate<LOSS, NE>(a, b, rowval, y, z);

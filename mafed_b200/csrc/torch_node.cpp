@@ -237,7 +237,8 @@ struct DistillBackward : public Node {
 };
 
 // ---------------------------------------------------------------- forward
-// students / teachers: the selected [B, T, D] hidden states (same dtype, shape, device).  attn_mask: int64 [B, T - n_vis]
+// students / teachers: the selected [B, T, D] hidden states (same shape and device; one dtype, or fp32 students with
+// bf16 / fp16 teachers -- other mixes are up-cast to fp32).  attn_mask: int64 [B, T - n_vis]
 // (ignored in cls mode).  masks_out: None, an int64 [2, B, T] tensor, or True to have one allocated here; it receives
 // (lang_masks, image_masks).  comm: a mafed_comm_t* (0: single rank).  ticket: optional int64[4] from
 // prefetch_counts.  seen: optional pinned float[1].
@@ -251,12 +252,17 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
   const int L = plan->n_layers;
   TORCH_CHECK((int)students.size() == L && (int)teachers.size() == L, "students / teachers / plan length mismatch");
   {
-    // layers of different dtypes: up-cast both sides to fp32, which is what the reference's autocast region does to
-    // the inputs of its loss functions (distillation.py:90,244); the casts are ordinary autograd ops
-    bool mixed = false;
-    for (int i = 0; i < L && !mixed; ++i)
-      mixed = students[i].scalar_type() != students[0].scalar_type() || teachers[i].scalar_type() != students[0].scalar_type();
-    if (mixed)
+    // One dtype everywhere, or fp32 students with teachers of one half-precision dtype: the kernels read the tensors
+    // as they are (a teacher pair, MAFED_DTYPE_PAIR).  Any other mix -- layers of different dtypes, a student narrower
+    // than its teacher -- is up-cast to fp32 on both sides, which is what the reference's autocast region does to
+    // the inputs of its loss functions (distillation.py:90,244); the casts are ordinary autograd ops.
+    const at::ScalarType s_type = students[0].scalar_type(), t_type = teachers[0].scalar_type();
+    bool uniform = true;
+    for (int i = 0; i < L && uniform; ++i)
+      uniform = students[i].scalar_type() == s_type && teachers[i].scalar_type() == t_type;
+    const bool native = uniform && (s_type == t_type || (s_type == at::kFloat && (t_type == at::kBFloat16 ||
+                                                                                  t_type == at::kHalf)));
+    if (!native)
       for (int i = 0; i < L; ++i) {
         students[i] = students[i].to(at::kFloat);
         teachers[i] = teachers[i].to(at::kFloat);
@@ -267,6 +273,7 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
               ": the distillation path runs only as sm_100a CUDA kernels (there is no CPU fallback)");
   TORCH_CHECK_VALUE(s0.dim() == 3, "hidden states must be [B, T, D]");
   const int code = dtype_code(s0.scalar_type());
+  const int t_code = dtype_code(teachers[0].scalar_type());
   const auto device = s0.device();
   const bool grad_mode = at::GradMode::is_enabled();
   std::vector<bool> needs(L, false);
@@ -276,7 +283,7 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
     at::Tensor& t = teachers[i];
     TORCH_CHECK_VALUE(s.sizes() == s0.sizes() && t.sizes() == s0.sizes(),
                       "all selected hidden states must share one [B, T, D] shape");
-    TORCH_CHECK_VALUE(s.scalar_type() == s0.scalar_type() && t.scalar_type() == s0.scalar_type() &&
+    TORCH_CHECK_VALUE(s.scalar_type() == s0.scalar_type() && t.scalar_type() == teachers[0].scalar_type() &&
                           s.device() == device && t.device() == device,
                       "student / teacher dtype or device mismatch");
     needs[i] = grad_mode && s.requires_grad();
@@ -299,7 +306,7 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
   shape.T = (int32_t)T;
   shape.n_vis = plan->cls ? (int32_t)std::min<int64_t>(plan->n_vis, T) : plan->n_vis;
   shape.D = (int32_t)D;
-  shape.dtype = code;
+  shape.dtype = t_code == code ? code : MAFED_DTYPE_PAIR(code, t_code);
   shape.loss_kind = plan->loss_kind;
   shape.cls = plan->cls ? 1 : 0;
   shape.tuning = reinterpret_cast<const mafed_tuning_t*>(tuning_addr);

@@ -37,6 +37,18 @@ from . import cabi, node
 from .comm import get_peer_comm
 
 _DTYPES = {torch.float32: cabi.F32, torch.bfloat16: cabi.BF16, torch.float16: cabi.F16}
+# (student, teacher) dtype pairs the kernels read as they are besides one dtype on both sides
+_TEACHER_PAIRS = {(torch.float32, torch.bfloat16), (torch.float32, torch.float16)}
+
+
+def _native_dtypes(students, teachers) -> bool:
+    """True when the kernels take these layers without an up-cast: one dtype everywhere, or fp32 students with
+    teachers of one half-precision dtype."""
+    s_types, t_types = {t.dtype for t in students}, {t.dtype for t in teachers}
+    if len(s_types) != 1 or len(t_types) != 1:
+        return False
+    pair = (next(iter(s_types)), next(iter(t_types)))
+    return pair[0] == pair[1] or pair in _TEACHER_PAIRS
 
 
 @dataclass
@@ -139,12 +151,16 @@ class _Launch:
         if s0.dim() != 3:
             raise ValueError("hidden states must be [B, T, D]")
         shape, dtype, device = s0.shape, s0.dtype, s0.device
+        t_dtype = teachers[0].dtype
+        if t_dtype != dtype and (dtype, t_dtype) not in _TEACHER_PAIRS:
+            raise ValueError(f"student / teacher dtype mismatch ({dtype} / {t_dtype}): the kernels take one dtype, "
+                             "or float32 students with bfloat16 or float16 teachers")
         self.B, self.T, self.D = shape
-        for group in (students, teachers):
+        for group, want in ((students, dtype), (teachers, t_dtype)):
             for t in group:
                 if t.shape != shape:
                     raise ValueError("all selected hidden states must share one [B, T, D] shape")
-                if t.dtype != dtype or t.device != device:
+                if t.dtype != want or t.device != device:
                     raise ValueError("student / teacher dtype or device mismatch")
         self.device = device
         self.dtype = dtype
@@ -163,7 +179,7 @@ class _Launch:
             self.mask = attn_mask.contiguous()
         self.n_layers = len(students)
         self.shape = cabi.make_shape(self.n_layers, self.B, self.T, n_vis if not plan.cls else min(n_vis, self.T),
-                                     self.D, _DTYPES[self.dtype], plan.loss_kind, plan.cls)
+                                     self.D, _DTYPES[self.dtype], plan.loss_kind, plan.cls, _DTYPES[t_dtype])
         self.shape_ref = ctypes.byref(self.shape)
         self.students = students
         self.teachers = teachers
@@ -459,7 +475,7 @@ def _step(plan: DistillPlan, attn_mask, group, teachers, mask_out, students, tic
             mask_out = torch.empty((2, attn_mask.shape[0], plan.n_vis + attn_mask.shape[1]), dtype=torch.int64,
                                    device=attn_mask.device)
         both = (mask_out[0], mask_out[1]) if mask_out is not None else None
-        if len({t.dtype for t in students} | {t.dtype for t in teachers}) > 1:
+        if not _native_dtypes(students, teachers):
             students, teachers = [s.float() for s in students], [t.float() for t in teachers]
         total, aux = _DistillFunction.apply(plan, attn_mask, group, tuple(_prepare(teachers)), both, *students)
         return total, aux, mask_out
@@ -486,8 +502,8 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
         teachers = [t.detach() for t in teachers]
     if len(students) != len(teachers) or len(students) != len(plan.layers):
         raise ValueError("students / teachers / plan.layers length mismatch")
-    # (layers of different dtypes: the node up-casts both sides to fp32, as the reference does under autocast,
-    # distillation.py:90,244)
+    # (fp32 students with bf16 / fp16 teachers run as they are; other mixes of dtypes are up-cast to fp32 on both
+    # sides, as the reference does under autocast, distillation.py:90,244)
     n = len(students)
     if n <= cabi.MAX_LAYERS:
         total, aux, both = _step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)

@@ -16,6 +16,7 @@ autograd node (``mafed_b200.node``).
 """
 from __future__ import annotations
 
+import contextlib
 from collections import deque
 from copy import deepcopy
 from typing import Dict, List, Optional
@@ -25,7 +26,7 @@ import torch
 
 from mafed_b200 import cabi
 from mafed_b200 import comm as _comm
-from mafed_b200.capture import HiddenStateCapture
+from mafed_b200.capture import HiddenStateCapture, HiddenStateTuple
 from mafed_b200.distill_op import DistillPlan, distill_loss, modality_masks, resolve_group, seen_slot
 from mafed_b200.methods.base import CLStrategy
 from mafed_b200.methods.distillation_loss_weights import DistillationWeights
@@ -123,6 +124,13 @@ class FeatureDistillation(CLStrategy):
         self.selective_capture = bool(kwargs.get("selective_capture", False))
         # walk one memory-loader iterator instead of spawning a fresh one per replay step
         self.persistent_memory_iterator = bool(kwargs.get("persistent_memory_iterator", False))
+        # hold the frozen teacher snapshot in bf16 / fp16 (None: the model's own dtype, as the reference does).  Its
+        # forward runs under an autocast of that dtype and every teacher hidden state is handed over in it (see
+        # _teacher_forward), so the step reads them as they are next to fp32 student states; the teacher's weights and
+        # states are rounded to it, so the numbers differ from the reference's
+        self.teacher_dtype = kwargs.get("teacher_dtype")
+        if self.teacher_dtype not in (None, torch.bfloat16, torch.float16):
+            raise ValueError(f"teacher_dtype must be None, torch.bfloat16 or torch.float16, not {self.teacher_dtype!r}")
         self._mem_iter = self._mem_iter_source = None
         self._mem_epoch = 0
         self._plan_cache = None
@@ -347,10 +355,25 @@ class FeatureDistillation(CLStrategy):
             batch["lang_masks"], batch["image_masks"] = masks
         return total, aux
 
+    def _teacher_forward(self, batch):
+        """Autocast region of the teacher forward.  A snapshot held in ``teacher_dtype`` runs under an autocast of that
+        dtype: inside replay's bf16 region an fp16 snapshot would otherwise get bf16 out of its linears next to fp16 out
+        of its embeddings, and its hidden states would come out in mixed dtypes."""
+        if self.teacher_dtype is None:
+            return contextlib.nullcontext()
+        am = batch.get("attention_mask")
+        return torch.autocast(am.device.type if torch.is_tensor(am) else "cuda", dtype=self.teacher_dtype)
+
+    def _as_teacher_dtype(self, h):
+        """A teacher hidden state in ``teacher_dtype`` (if set).  Autocast leaves some of them in fp32 (the output of the
+        final layer norm: layer_norm is an fp32 op under autocast); rounding that one too keeps every distilled teacher
+        state in one dtype, so the step reads them natively instead of up-casting every layer."""
+        return h if self.teacher_dtype is None or h.dtype == self.teacher_dtype else h.to(self.teacher_dtype)
+
     def _past_states(self, batch, layers):
         """Teacher hidden states of the distilled layers only (same forward and side effects as
         ``_get_past_hidden_states``)."""
-        with torch.no_grad():
+        with torch.no_grad(), self._teacher_forward(batch):
             batch.pop("labels", None)
             if self.selective_capture:
                 with HiddenStateCapture(self.past_model, layers, detach=True) as cap:
@@ -360,18 +383,21 @@ class FeatureDistillation(CLStrategy):
                 states = self.past_model(**batch, output_hidden_states=True, return_dict=True).hidden_states
         # no per-tensor `.detach()` (distillation.py:223): these come out of a no_grad forward, and the node never builds
         # a graph edge to a teacher tensor whatever its flags are
-        return [states[l] for l in layers]
+        return [self._as_teacher_dtype(states[l]) for l in layers]
 
     def _get_past_hidden_states(self, batch):
-        with torch.no_grad():
+        with torch.no_grad(), self._teacher_forward(batch):
             batch.pop("labels", None)
             if self.selective_capture:
                 layers = self.loss_weights.get_distillation_layers()
                 with HiddenStateCapture(self.past_model, layers, detach=True) as cap:
                     self.past_model(**batch, output_hidden_states=False, return_dict=True)
-                return cap.hidden_states
+                hs = cap.hidden_states
+                if self.teacher_dtype is None:
+                    return hs
+                return HiddenStateTuple(len(hs), {l: self._as_teacher_dtype(hs[l]) for l in layers})
             states = self.past_model(**batch, output_hidden_states=True, return_dict=True).hidden_states
-        return [h.detach() for h in states]
+        return [self._as_teacher_dtype(h.detach()) for h in states]
 
     # ---- single-tensor token losses, kept for API compatibility (distillation.py:226-257)
     def _masked_token_loss(self, hidden_states, past_hidden_states, mask, loss_kind):
@@ -496,8 +522,10 @@ class FeatureDistillation(CLStrategy):
 
     # ------------------------------------------------------------------ between tasks
     def _update_model(self, model):
-        """Freeze a copy of the just-trained model as the next task's teacher."""
+        """Freeze a copy of the just-trained model as the next task's teacher (in ``teacher_dtype`` if set)."""
         self.past_model = deepcopy(model)
+        if self.teacher_dtype is not None:
+            self.past_model.to(self.teacher_dtype)
         self.past_model.eval()
 
     def _update_memory(self, dataset):

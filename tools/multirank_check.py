@@ -6,7 +6,11 @@
 
 Every rank holds a contiguous slice of the batch; the sharded loss and the concatenation of the
 per-rank gradients must equal the single-device CPU oracle on the full batch (SURVEY.md 8e).
+
+``--teacher-dtype {bf16,fp16}``: instead, fp32 student states against a teacher in that dtype (read as it is by the
+kernels); every rank's loss and gradient slice must equal the same step run on one GPU over the concatenated batch.
 """
+import argparse
 import os
 import sys
 
@@ -19,10 +23,17 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--teacher-dtype", choices=["bf16", "fp16"], default=None,
+                    help="fp32 students against a teacher in this dtype (default: today's same-dtype cases)")
+    args = ap.parse_args()
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
     torch.cuda.set_device(local)
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    if args.teacher_dtype is not None:
+        ok = mixed_teacher_check(rank, world, {"bf16": torch.bfloat16, "fp16": torch.float16}[args.teacher_dtype])
+        finish(ok)
     from gpu_util import Out, make_method, rel_err
     from golden_util import oracle_cfg
     from oracle import distill_oracle as O
@@ -68,11 +79,62 @@ def main():
     if os.environ.get("MAFED_B200_DIST", "peer") == "peer":
         ok &= peer is not None          # on one NVLink box the mailboxes must map
     print(f"rank {rank}: exchange path = {mode}", flush=True)
+    finish(ok)
+
+
+def finish(ok):
+    """Exit 0 when every rank passed."""
     flag = torch.tensor([1 if ok else 0], device="cuda")
     dist.all_reduce(flag, op=dist.ReduceOp.MIN)
     dist.barrier()
     dist.destroy_process_group()
     sys.exit(0 if int(flag) == 1 else 1)
+
+
+def mixed_teacher_check(rank, world, teacher_dtype):
+    """fp32 student states, half-precision teacher, batch-sharded one-pass and two-pass steps: the loss equals the
+    one-GPU step on the concatenated batch to 1e-6 (the sums are added in another order) and every rank's gradient
+    slice equals it bit for bit (mse) or to 1e-6 (cosine: the row statistics of another tile geometry)."""
+    from gpu_util import Out, make_method, rel_err
+    from mafed_b200.comm import get_peer_comm
+    from oracle import distill_oracle as O
+    # MAFED_B200_DIST=nccl: no communicator, the sharded steps run the NCCL sequence of ctypes calls (_DistillFunction)
+    mode = "nccl" if get_peer_comm(None) is None else "peer-memory"
+    ok = True
+    for loss, single_pass in [("mse", True), ("cosine", True), ("mse", False), ("cosine", False)]:
+        B = 4 * world + 2
+        st, te, am = O.make_inputs(4, B, 9, 768, n_vis=256, seed=37, mask="ragged", teacher="independent")
+        te = [t.to(teacher_dtype) for t in te]
+        meta = dict(modality="equal", layer_strategy="discounted", loss=loss, gamma=0.5, num_hidden_layers=3,
+                    layer=None, n_vis=256, coeff=1.0, cls=False, lang_coeff=None)
+        lo = rank * 4
+        hi = B if rank == world - 1 else lo + 4
+
+        def run(a, b, group):
+            fd = make_method(meta, single_pass=single_pass)
+            fd.grad_multiplier = 1.0
+            fd.process_group = group
+            leaves = [s[a:b].cuda().contiguous().requires_grad_(True) for s in st]
+            teach = [t[a:b].cuda().contiguous() for t in te]
+            fd.past_model = lambda **kw: Out(tuple(teach))
+            loss_v = fd.distill(Out(tuple(leaves)), {"attention_mask": am[a:b].cuda()})
+            (loss_v * 0.5).backward()
+            torch.cuda.synchronize()
+            return loss_v.detach(), [l.grad for l in leaves]
+
+        loss_s, g_s = run(lo, hi, None)
+        loss_f, g_f = run(0, B, False)
+        e_loss = abs(float(loss_s) - float(loss_f)) / abs(float(loss_f))
+        pairs = [(a, b[lo:hi]) for a, b in zip(g_s, g_f) if b is not None]
+        if loss == "mse":
+            same = all(torch.equal(a, b) for a, b in pairs)
+        else:
+            same = max(rel_err(a.cpu(), b.cpu()) for a, b in pairs) < 1e-6
+        good = e_loss < 1e-6 and same and len(pairs) == 3
+        ok &= good
+        print(f"rank {rank}/{world} ({mode}) fp32 student, {teacher_dtype} teacher, {loss} single_pass={single_pass}: "
+              f"loss err {e_loss:.2e} gradients {'equal' if same else 'DIFFER'} {'OK' if good else 'FAIL'}", flush=True)
+    return ok
 
 
 def graph_replay_check(rank, world):
