@@ -66,6 +66,7 @@ class Shape(ctypes.Structure):
 # Overrides travel with each call (mafed_shape_t::tuning); the library itself keeps no mutable state.
 # Benchmarks and tests install a Tuning for the calls made inside a `with cabi.tuning(...)` block of THIS process.
 _active_tuning = None
+_active_tuning_address = 0      # its address as a plain int (what a compiled step reads, and guards on)
 
 
 def active_tuning_address() -> int:
@@ -77,7 +78,7 @@ def active_tuning_address() -> int:
 def tuning(variant: int = 0, **keys):
     """``with cabi.tuning(variant=cabi.VARIANT_LDG, TUNE_NO_TAIL=1): ...`` -- overrides for the calls inside the block.
     Keys are the names of TUNE_KEYS; any other keyword raises TypeError."""
-    global _active_tuning
+    global _active_tuning, _active_tuning_address
     unknown = sorted(set(keys) - set(TUNE_KEYS))
     if unknown:
         raise TypeError(f"unknown tuning key(s) {unknown}; the library reads {sorted(TUNE_KEYS)}")
@@ -89,10 +90,12 @@ def tuning(variant: int = 0, **keys):
     for name, value in keys.items():
         t.v[TUNE_KEYS[name]] = int(value)
     prev, _active_tuning = _active_tuning, t
+    _active_tuning_address = ctypes.addressof(t)
     try:
         yield t
     finally:
         _active_tuning = prev
+        _active_tuning_address = ctypes.addressof(prev) if prev is not None else 0
 
 
 class Weights(ctypes.Structure):

@@ -20,6 +20,9 @@ import torch.distributed as dist
 from . import cabi
 
 _cache: Dict[tuple, Optional["PeerComm"]] = {}
+# Bumped whenever the communicators are torn down: a compiled step reads it (Dynamo guards on its value), so a graph
+# traced against a communicator is retraced instead of replaying a stale handle.
+_generation = 0
 
 
 class PeerComm:
@@ -106,6 +109,8 @@ def peek_peer_comm(group=None) -> Optional[PeerComm]:
 
 
 def reset():
+    global _generation
+    _generation += 1
     for c in _cache.values():
         if c is not None:
             c.close()

@@ -156,6 +156,134 @@ std::vector<at::Tensor> layer_views(const at::Tensor& buf, int64_t n) {
   return out;
 }
 
+// ---------------------------------------------------------------- shared by the node and the torch.library ops
+// Pointer tables of one launch.
+struct Tables {
+  const void* s[MAFED_MAX_LAYERS];
+  const void* t[MAFED_MAX_LAYERS];
+  void* g[MAFED_MAX_LAYERS];
+};
+
+void fill_tables(const std::vector<at::Tensor>& students, const std::vector<at::Tensor>& teachers, Tables& tb) {
+  for (size_t i = 0; i < students.size(); ++i) {
+    tb.s[i] = students[i].data_ptr();
+    tb.t[i] = teachers[i].data_ptr();
+    tb.g[i] = nullptr;
+  }
+}
+
+// Gradient pointers into one [n_need, B, T, D] buffer: layer i gets the next slice if it needs a gradient.
+void fill_grad_ptrs(const at::Tensor& buf, const std::vector<bool>& needs, Tables& tb) {
+  char* g0 = reinterpret_cast<char*>(buf.data_ptr());
+  const size_t layer_bytes = buf.size(0) == 0 ? 0 : (size_t)(buf.numel() / buf.size(0)) * buf.element_size();
+  for (size_t i = 0, j = 0; i < needs.size(); ++i) tb.g[i] = needs[i] ? g0 + (j++) * layer_bytes : nullptr;
+}
+
+int64_t count_needs(const std::vector<bool>& needs) {
+  int64_t n = 0;
+  for (bool b : needs) n += b ? 1 : 0;
+  return n;
+}
+
+// The gradient buffer of the needed layers; cls: only row 0 of each sample is written by the kernels.
+at::Tensor alloc_grads(int64_t n_need, const at::Tensor& s0, bool cls) {
+  std::vector<int64_t> sz = {n_need, s0.size(0), s0.size(1), s0.size(2)};
+  const auto opts = s0.options().requires_grad(false);
+  return cls ? at::zeros(sz, opts) : at::empty(sz, opts);
+}
+
+mafed_shape_t make_shape(const at::Tensor& s0, const at::Tensor& t0, int L, int loss_kind, bool cls, int n_vis,
+                         int64_t tuning_addr) {
+  const int code = dtype_code(s0.scalar_type());
+  const int t_code = dtype_code(t0.scalar_type());
+  const int64_t T = s0.size(1);
+  mafed_shape_t shape;
+  std::memset(&shape, 0, sizeof(shape));
+  shape.n_layers = L;
+  shape.B = (int32_t)s0.size(0);
+  shape.T = (int32_t)T;
+  shape.n_vis = cls ? (int32_t)std::min<int64_t>(n_vis, T) : n_vis;
+  shape.D = (int32_t)s0.size(2);
+  shape.dtype = t_code == code ? code : MAFED_DTYPE_PAIR(code, t_code);
+  shape.loss_kind = loss_kind;
+  shape.cls = cls ? 1 : 0;
+  shape.tuning = reinterpret_cast<const mafed_tuning_t*>(tuning_addr);
+  return shape;
+}
+
+// int64 [B, T - n_vis] contiguous attention mask on the device (undefined in cls mode, where it is not read).
+at::Tensor prepare_mask(const c10::optional<at::Tensor>& attn_mask, bool cls, int n_vis, int64_t B, int64_t T) {
+  at::Tensor mask;
+  if (cls) return mask;
+  TORCH_CHECK_VALUE(attn_mask.has_value() && attn_mask->defined(), "attention_mask is required");
+  mask = *attn_mask;
+  TORCH_CHECK(mask.is_cuda(), "attention_mask is on ", mask.device(),
+              ": the distillation path runs only as sm_100a CUDA kernels (there is no CPU fallback)");
+  if (mask.scalar_type() != at::kLong) mask = mask.to(at::kLong);
+  TORCH_CHECK_VALUE(mask.dim() == 2 && mask.size(0) == B && mask.size(1) == T - n_vis, "attention_mask shape ",
+                    mask.sizes(), " != (B, T - n_vis) = (", B, ", ", T - n_vis, ")");
+  if (!mask.is_contiguous()) mask = mask.contiguous();
+  return mask;
+}
+
+// One scratch allocation: the partial-sum workspace, then [the scale table,] then [the sharded fp64 sums].
+struct Scratch {
+  at::Tensor buf;
+  char* ws = nullptr;
+  float* bwd_scale = nullptr;
+  double* sums = nullptr;
+};
+
+Scratch alloc_scratch(int L, c10::Device device, bool with_scale, bool sharded) {
+  const size_t ws_bytes = (api().ws_bytes(L) + 255) & ~(size_t)255;
+  const size_t scale_bytes = with_scale ? ((size_t)8 * L + 255) & ~(size_t)255 : 0;
+  const size_t sums_bytes = sharded ? (size_t)8 * (2 * L + 2) : 0;
+  Scratch sc;
+  sc.buf = at::empty({(int64_t)(ws_bytes + scale_bytes + sums_bytes)},
+                     at::TensorOptions().dtype(at::kByte).device(device));
+  sc.ws = reinterpret_cast<char*>(sc.buf.data_ptr());
+  if (with_scale) sc.bwd_scale = reinterpret_cast<float*>(sc.ws + ws_bytes);
+  if (sharded) sc.sums = reinterpret_cast<double*>(sc.ws + ws_bytes + scale_bytes);
+  return sc;
+}
+
+at::Tensor alloc_out(int L, c10::Device device) {
+  return at::empty({1 + 3 * (int64_t)L}, at::TensorOptions().dtype(at::kFloat).device(device));
+}
+
+void launch_step(const mafed_shape_t& shape, const Tables& tb, const at::Tensor& mask, const mafed_weights_t& w,
+                 float fixed, const Scratch& sc, float* out, float* bwd_scale, int64_t* lang, int64_t* image,
+                 int64_t comm, const int64_t* ticket, cudaStream_t stream) {
+  check_rc(api().step(&shape, tb.s, tb.t, tb.g, mask.defined() ? mask.data_ptr<int64_t>() : nullptr, &w, fixed, sc.ws,
+                      out, bwd_scale, sc.sums, lang, image, reinterpret_cast<mafed_comm_t*>(comm), ticket, stream),
+           "mafed_distill_step");
+}
+
+void launch_fwd_step(const mafed_shape_t& shape, const Tables& tb, const at::Tensor& mask, const mafed_weights_t& w,
+                     const Scratch& sc, float* out, float* bwd_scale, int64_t* lang, int64_t* image, int64_t comm,
+                     cudaStream_t stream) {
+  const int64_t* mask_ptr = mask.defined() ? mask.data_ptr<int64_t>() : nullptr;
+  check_rc(api().fwd_step(&shape, tb.s, tb.t, mask_ptr, &w, sc.ws, out, bwd_scale, sc.sums,
+                          reinterpret_cast<mafed_comm_t*>(comm), stream),
+           "mafed_distill_fwd_step");
+  if (lang != nullptr) check_rc(api().modality_masks(&shape, mask_ptr, lang, image, stream), "mafed_distill_modality_masks");
+}
+
+// The gate (skip != nullptr) or the full backward into the pointers of `tb.g`.  g: the device fp32 upstream gradient.
+void launch_bwd(const mafed_shape_t& shape, const Tables& tb, const at::Tensor& mask, const float* bwd_scale,
+                const at::Tensor& g, float grad_out_scale, const float* skip, float* seen, cudaStream_t stream) {
+  check_rc(api().bwd(&shape, tb.s, tb.t, tb.g, mask.defined() ? mask.data_ptr<int64_t>() : nullptr, bwd_scale,
+                     g.data_ptr<float>(), grad_out_scale, skip, seen, stream),
+           "mafed_distill_bwd");
+}
+
+// The upstream gradient as the kernels read it: fp32, contiguous, on `device`.
+at::Tensor upstream(at::Tensor g, c10::Device device) {
+  if (g.scalar_type() != at::kFloat || g.device() != device) g = g.to(device, at::kFloat);
+  if (!g.is_contiguous()) g = g.contiguous();
+  return g;
+}
+
 // ---------------------------------------------------------------- the backward node
 struct DistillBackward : public Node {
   std::shared_ptr<Plan> plan;
@@ -190,47 +318,33 @@ struct DistillBackward : public Node {
     if (grads_in.empty() || !grads_in[0].defined()) return out;
     TORCH_CHECK(!released, "Trying to backward through the distillation step a second time (its saved tensors have "
                            "been freed); pass retain_graph=True to the first backward");
-    const Api& a = api();
     auto self = shared_from_this();
     std::vector<at::Tensor> s(n), t(n);
-    const void* s_ptrs[MAFED_MAX_LAYERS];
-    const void* t_ptrs[MAFED_MAX_LAYERS];
-    void* g_ptrs[MAFED_MAX_LAYERS];
     for (size_t i = 0; i < n; ++i) {
       s[i] = students[i].unpack(self);
       t[i] = teachers[i].unpack(self);
-      s_ptrs[i] = s[i].data_ptr();
-      t_ptrs[i] = t[i].data_ptr();
     }
+    Tables tb;
+    fill_tables(s, t, tb);
     at::Tensor m;
     if (has_mask) m = mask.unpack(self);
     const auto device = s[0].device();
     c10::cuda::CUDAGuard guard(device);
     const cudaStream_t stream = c10::cuda::getCurrentCUDAStream(device.index()).stream();
     at::AutoDispatchBelowADInplaceOrView below;
-    at::Tensor g = grads_in[0];
-    if (g.scalar_type() != at::kFloat || g.device() != device) g = g.to(device, at::kFloat);
-    if (!g.is_contiguous()) g = g.contiguous();
+    const at::Tensor g = upstream(grads_in[0], device);
     shape.tuning = has_tuning ? &tuning : nullptr;
 
-    int64_t n_need = 0;
-    for (bool b : needs) n_need += b ? 1 : 0;
+    const int64_t n_need = count_needs(needs);
     const bool gate = grad_buf.defined();   // one-pass step: gradients exist, fix them up only if g differs
-    at::Tensor buf = grad_buf;
-    if (!gate) {
-      std::vector<int64_t> sz = {n_need, shape.B, shape.T, shape.D};
-      buf = plan->cls ? at::zeros(sz, s[0].options()) : at::empty(sz, s[0].options());
-    }
+    const at::Tensor buf = gate ? grad_buf : alloc_grads(n_need, s[0], plan->cls);
+    fill_grad_ptrs(buf, needs, tb);
     auto views = layer_views(buf, n_need);
-    for (size_t i = 0, j = 0; i < n; ++i) {
-      g_ptrs[i] = needs[i] ? views[j].data_ptr() : nullptr;
+    for (size_t i = 0, j = 0; i < n; ++i)
       if (needs[i]) out[i] = std::move(views[j++]);
-    }
     const float fixed = plan->fixed();
-    check_rc(a.bwd(&shape, s_ptrs, t_ptrs, g_ptrs, has_mask ? m.data_ptr<int64_t>() : nullptr, bwd_scale,
-                   g.data_ptr<float>(), (float)plan->grad_multiplier, gate ? &fixed : nullptr, gate ? seen : nullptr,
-                   stream),
-             "mafed_distill_bwd");
+    launch_bwd(shape, tb, m, bwd_scale, g, (float)plan->grad_multiplier, gate ? &fixed : nullptr, gate ? seen : nullptr,
+               stream);
     grad_buf.reset();   // handed to autograd: a second backward (retain_graph) recomputes into a fresh buffer
     return out;
   }
@@ -248,7 +362,6 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
     const std::shared_ptr<Plan>& plan, std::vector<at::Tensor> students, std::vector<at::Tensor> teachers,
     const c10::optional<at::Tensor>& attn_mask, const py::object& masks_out, int64_t comm,
     const std::shared_ptr<CountsTicket>& ticket, const c10::optional<at::Tensor>& seen, int64_t tuning_addr) {
-  const Api& a = api();
   const int L = plan->n_layers;
   TORCH_CHECK((int)students.size() == L && (int)teachers.size() == L, "students / teachers / plan length mismatch");
   {
@@ -272,8 +385,6 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
   TORCH_CHECK(s0.is_cuda(), "hidden_states is on ", s0.device(),
               ": the distillation path runs only as sm_100a CUDA kernels (there is no CPU fallback)");
   TORCH_CHECK_VALUE(s0.dim() == 3, "hidden states must be [B, T, D]");
-  const int code = dtype_code(s0.scalar_type());
-  const int t_code = dtype_code(teachers[0].scalar_type());
   const auto device = s0.device();
   const bool grad_mode = at::GradMode::is_enabled();
   std::vector<bool> needs(L, false);
@@ -298,52 +409,18 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
     if (!students[i].is_contiguous()) students[i] = students[i].contiguous();
     if (!teachers[i].is_contiguous()) teachers[i] = teachers[i].contiguous();
   }
-  const int64_t B = s0.size(0), T = s0.size(1), D = s0.size(2);
-  mafed_shape_t shape;
-  std::memset(&shape, 0, sizeof(shape));
-  shape.n_layers = L;
-  shape.B = (int32_t)B;
-  shape.T = (int32_t)T;
-  shape.n_vis = plan->cls ? (int32_t)std::min<int64_t>(plan->n_vis, T) : plan->n_vis;
-  shape.D = (int32_t)D;
-  shape.dtype = t_code == code ? code : MAFED_DTYPE_PAIR(code, t_code);
-  shape.loss_kind = plan->loss_kind;
-  shape.cls = plan->cls ? 1 : 0;
-  shape.tuning = reinterpret_cast<const mafed_tuning_t*>(tuning_addr);
-
-  at::Tensor mask;
-  if (!plan->cls) {
-    TORCH_CHECK_VALUE(attn_mask.has_value() && attn_mask->defined(), "attention_mask is required");
-    mask = *attn_mask;
-    TORCH_CHECK(mask.is_cuda(), "attention_mask is on ", mask.device(),
-                ": the distillation path runs only as sm_100a CUDA kernels (there is no CPU fallback)");
-    if (mask.scalar_type() != at::kLong) mask = mask.to(at::kLong);
-    TORCH_CHECK_VALUE(mask.dim() == 2 && mask.size(0) == B && mask.size(1) == T - plan->n_vis, "attention_mask shape ",
-                      mask.sizes(), " != (B, T - n_vis) = (", B, ", ", T - plan->n_vis, ")");
-    if (!mask.is_contiguous()) mask = mask.contiguous();
-  }
+  const int64_t B = s0.size(0), T = s0.size(1);
+  const mafed_shape_t shape = make_shape(s0, teachers[0], L, plan->loss_kind, plan->cls, plan->n_vis, tuning_addr);
+  const at::Tensor mask = prepare_mask(attn_mask, plan->cls, plan->n_vis, B, T);
 
   c10::cuda::CUDAGuard guard(device);
   const cudaStream_t stream = c10::cuda::getCurrentCUDAStream(device.index()).stream();
-  const size_t ws_bytes = (a.ws_bytes(L) + 255) & ~(size_t)255;
-  const size_t scale_bytes = ((size_t)8 * L + 255) & ~(size_t)255;
-  const bool sharded = comm != 0;
-  const size_t sums_bytes = sharded ? (size_t)8 * (2 * L + 2) : 0;
-  const auto byte_opts = at::TensorOptions().dtype(at::kByte).device(device);
-  at::Tensor scratch = at::empty({(int64_t)(ws_bytes + scale_bytes + sums_bytes)}, byte_opts);
-  at::Tensor out = at::empty({1 + 3 * (int64_t)L}, at::TensorOptions().dtype(at::kFloat).device(device));
-  char* base = reinterpret_cast<char*>(scratch.data_ptr());
-  float* bwd_scale = reinterpret_cast<float*>(base + ws_bytes);
-  double* sums = sharded ? reinterpret_cast<double*>(base + ws_bytes + scale_bytes) : nullptr;
-
-  const void* s_ptrs[MAFED_MAX_LAYERS];
-  const void* t_ptrs[MAFED_MAX_LAYERS];
-  void* g_ptrs[MAFED_MAX_LAYERS];
-  for (int i = 0; i < L; ++i) {
-    s_ptrs[i] = students[i].data_ptr();
-    t_ptrs[i] = teachers[i].data_ptr();
-    g_ptrs[i] = nullptr;
-  }
+  const Scratch sc = alloc_scratch(L, device, /*with_scale=*/true, /*sharded=*/comm != 0);
+  const at::Tensor scratch = sc.buf;
+  float* bwd_scale = sc.bwd_scale;
+  at::Tensor out = alloc_out(L, device);
+  Tables tb;
+  fill_tables(students, teachers, tb);
   int64_t* lang = nullptr;
   int64_t* image = nullptr;
   c10::optional<at::Tensor> masks;
@@ -362,7 +439,6 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
       image = lang + B * T;
     }
   }
-  const int64_t* mask_ptr = mask.defined() ? mask.data_ptr<int64_t>() : nullptr;
   const int64_t* ticket_ptr = nullptr;
   if (ticket != nullptr) {
     ticket->wait();     // this stream behind the prefetch launch (a no-op wait: it finished a forward pass ago)
@@ -371,23 +447,12 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
 
   at::Tensor grad_buf;
   if (plan->single_pass && any_need) {
-    int64_t n_need = 0;
-    for (bool b : needs) n_need += b ? 1 : 0;
-    std::vector<int64_t> sz = {n_need, B, T, D};
-    // cls: only row 0 of each sample is written by the kernel
-    grad_buf = plan->cls ? at::zeros(sz, s0.options().requires_grad(false)) : at::empty(sz, s0.options().requires_grad(false));
-    char* g0 = reinterpret_cast<char*>(grad_buf.data_ptr());
-    const size_t layer_bytes = (size_t)B * T * D * grad_buf.element_size();
-    for (int i = 0, j = 0; i < L; ++i)
-      if (needs[i]) g_ptrs[i] = g0 + (size_t)(j++) * layer_bytes;
-    check_rc(a.step(&shape, s_ptrs, t_ptrs, g_ptrs, mask_ptr, &plan->w, plan->fixed(), base, out.data_ptr<float>(),
-                    bwd_scale, sums, lang, image, reinterpret_cast<mafed_comm_t*>(comm), ticket_ptr, stream),
-             "mafed_distill_step");
+    grad_buf = alloc_grads(count_needs(needs), s0, plan->cls);
+    fill_grad_ptrs(grad_buf, needs, tb);
+    launch_step(shape, tb, mask, plan->w, plan->fixed(), sc, out.data_ptr<float>(), bwd_scale, lang, image, comm,
+                ticket_ptr, stream);
   } else {
-    check_rc(a.fwd_step(&shape, s_ptrs, t_ptrs, mask_ptr, &plan->w, base, out.data_ptr<float>(), bwd_scale, sums,
-                        reinterpret_cast<mafed_comm_t*>(comm), stream),
-             "mafed_distill_fwd_step");
-    if (lang != nullptr) check_rc(a.modality_masks(&shape, mask_ptr, lang, image, stream), "mafed_distill_modality_masks");
+    launch_fwd_step(shape, tb, mask, plan->w, sc, out.data_ptr<float>(), bwd_scale, lang, image, comm, stream);
   }
 
   at::Tensor total = out.select(0, 0);
@@ -461,6 +526,143 @@ std::shared_ptr<CountsTicket> prefetch_counts(const at::Tensor& attn_mask, int64
   return ticket;
 }
 
+// ---------------------------------------------------------------- the step as torch.library ops
+// `mafed::step`, `mafed::fwd_step` and `mafed::bwd` are the three C-ABI calls of a step as dispatcher ops, so that
+// torch.compile can trace a step into the caller's graph (the pybind `distill` above builds its own autograd node,
+// which Dynamo cannot trace).  Their fake implementations and the autograd formula live in mafed_b200/ops.py.  The
+// plan arrives as plain values; the workspace is scratch from the caching allocator, as in `distill`.  The ops take
+// one dtype everywhere, or fp32 students with bf16 / fp16 teachers: other mixes are up-cast by the caller.
+
+struct OpInputs {
+  std::vector<at::Tensor> students, teachers;
+  at::Tensor mask;
+  mafed_shape_t shape;
+  Tables tb;
+};
+
+OpInputs op_inputs(const at::TensorList students, const at::TensorList teachers, const c10::optional<at::Tensor>& mask,
+                   int64_t loss_kind, bool cls, int64_t n_vis, int64_t tuning) {
+  const int64_t L = (int64_t)students.size();
+  TORCH_CHECK(L >= 1 && L <= MAFED_MAX_LAYERS, "1..", MAFED_MAX_LAYERS, " layers per call");
+  TORCH_CHECK((int64_t)teachers.size() == L, "students / teachers length mismatch");
+  OpInputs in;
+  const at::Tensor& s0 = students[0];
+  const at::Tensor& t0 = teachers[0];
+  TORCH_CHECK_VALUE(s0.dim() == 3, "hidden states must be [B, T, D]");
+  const bool native = s0.scalar_type() == t0.scalar_type() ||
+                      (s0.scalar_type() == at::kFloat && (t0.scalar_type() == at::kBFloat16 || t0.scalar_type() == at::kHalf));
+  TORCH_CHECK_TYPE(native, "student / teacher dtypes ", s0.scalar_type(), " / ", t0.scalar_type(),
+                   ": one dtype, or float32 students with bfloat16 or float16 teachers");
+  for (int64_t i = 0; i < L; ++i) {
+    TORCH_CHECK_VALUE(students[i].sizes() == s0.sizes() && teachers[i].sizes() == s0.sizes(),
+                      "all selected hidden states must share one [B, T, D] shape");
+    TORCH_CHECK_VALUE(students[i].scalar_type() == s0.scalar_type() && teachers[i].scalar_type() == t0.scalar_type() &&
+                          students[i].device() == s0.device() && teachers[i].device() == s0.device(),
+                      "student / teacher dtype or device mismatch");
+    in.students.push_back(students[i].contiguous());
+    in.teachers.push_back(teachers[i].contiguous());
+  }
+  in.shape = make_shape(s0, t0, (int)L, (int)loss_kind, cls, (int)n_vis, tuning);
+  in.mask = prepare_mask(mask, cls, (int)n_vis, s0.size(0), s0.size(1));
+  fill_tables(in.students, in.teachers, in.tb);
+  return in;
+}
+
+mafed_weights_t op_weights(int64_t L, at::ArrayRef<double> layer_coeffs, const c10::optional<at::ArrayRef<double>>& lang_weights,
+                           int64_t modality_kind, double distill_coeff) {
+  TORCH_CHECK((int64_t)layer_coeffs.size() == L, "layer_coeffs / students length mismatch");
+  c10::optional<std::vector<double>> lw;
+  if (lang_weights.has_value()) lw = lang_weights->vec();
+  return Plan((int)modality_kind, distill_coeff, layer_coeffs.vec(), lw, MAFED_LOSS_MSE, false, 0, 1.0, true, 1.0).w;
+}
+
+std::vector<bool> op_needs(c10::List<bool> needs, int64_t L) {
+  TORCH_CHECK((int64_t)needs.size() == L, "needs / students length mismatch");
+  std::vector<bool> v(needs.begin(), needs.end());
+  return v;
+}
+
+at::Tensor op_masks(bool want, bool cls, const at::Tensor& s0) {
+  const auto opts = at::TensorOptions().dtype(at::kLong).device(s0.device());
+  return want && !cls ? at::empty({2, s0.size(0), s0.size(1)}, opts) : at::empty({0}, opts);
+}
+
+// -> (out [1 + 3L]: total, then aux; grads [n_need, B, T, D]; bwd_scale [2L]; masks [2, B, T] or [0])
+std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> op_step(
+    at::TensorList students, at::TensorList teachers, const c10::optional<at::Tensor>& mask,
+    at::ArrayRef<double> layer_coeffs, c10::optional<at::ArrayRef<double>> lang_weights, int64_t modality_kind,
+    double distill_coeff, int64_t loss_kind, bool cls, int64_t n_vis, double assumed_grad_out, double grad_multiplier,
+    c10::List<bool> needs, int64_t comm, bool want_masks, int64_t tuning) {
+  const int64_t L = (int64_t)students.size();
+  OpInputs in = op_inputs(students, teachers, mask, loss_kind, cls, n_vis, tuning);
+  const mafed_weights_t w = op_weights(L, layer_coeffs, lang_weights, modality_kind, distill_coeff);
+  const std::vector<bool> nd = op_needs(needs, L);
+  const at::Tensor& s0 = in.students[0];
+  const auto device = s0.device();
+  c10::cuda::CUDAGuard guard(device);
+  const cudaStream_t stream = c10::cuda::getCurrentCUDAStream(device.index()).stream();
+  const Scratch sc = alloc_scratch((int)L, device, /*with_scale=*/false, /*sharded=*/comm != 0);
+  at::Tensor out = alloc_out((int)L, device);
+  at::Tensor bwd_scale = at::empty({2 * L}, at::TensorOptions().dtype(at::kFloat).device(device));
+  at::Tensor grads = alloc_grads(count_needs(nd), s0, cls);
+  at::Tensor masks = op_masks(want_masks, cls, s0);
+  int64_t* lang = masks.numel() ? masks.data_ptr<int64_t>() : nullptr;
+  fill_grad_ptrs(grads, nd, in.tb);
+  launch_step(in.shape, in.tb, in.mask, w, (float)(assumed_grad_out * grad_multiplier), sc, out.data_ptr<float>(),
+              bwd_scale.data_ptr<float>(), lang, lang ? lang + s0.size(0) * s0.size(1) : nullptr, comm, nullptr, stream);
+  return std::make_tuple(out, grads, bwd_scale, masks);
+}
+
+// -> (out [1 + 3L]: total, then aux; bwd_scale [2L]; masks [2, B, T] or [0])
+std::tuple<at::Tensor, at::Tensor, at::Tensor> op_fwd_step(
+    at::TensorList students, at::TensorList teachers, const c10::optional<at::Tensor>& mask,
+    at::ArrayRef<double> layer_coeffs, c10::optional<at::ArrayRef<double>> lang_weights, int64_t modality_kind,
+    double distill_coeff, int64_t loss_kind, bool cls, int64_t n_vis, double grad_multiplier, c10::List<bool> needs,
+    int64_t comm, bool want_masks, int64_t tuning) {
+  // grad_multiplier and needs are read by the autograd formula (its backward), not by the launch
+  const int64_t L = (int64_t)students.size();
+  op_needs(needs, L);
+  OpInputs in = op_inputs(students, teachers, mask, loss_kind, cls, n_vis, tuning);
+  const mafed_weights_t w = op_weights(L, layer_coeffs, lang_weights, modality_kind, distill_coeff);
+  const at::Tensor& s0 = in.students[0];
+  const auto device = s0.device();
+  c10::cuda::CUDAGuard guard(device);
+  const cudaStream_t stream = c10::cuda::getCurrentCUDAStream(device.index()).stream();
+  const Scratch sc = alloc_scratch((int)L, device, /*with_scale=*/false, /*sharded=*/comm != 0);
+  at::Tensor out = alloc_out((int)L, device);
+  at::Tensor bwd_scale = at::empty({2 * L}, at::TensorOptions().dtype(at::kFloat).device(device));
+  at::Tensor masks = op_masks(want_masks, cls, s0);
+  int64_t* lang = masks.numel() ? masks.data_ptr<int64_t>() : nullptr;
+  launch_fwd_step(in.shape, in.tb, in.mask, w, sc, out.data_ptr<float>(), bwd_scale.data_ptr<float>(), lang,
+                  lang ? lang + s0.size(0) * s0.size(1) : nullptr, comm, stream);
+  return std::make_tuple(out, bwd_scale, masks);
+}
+
+// The backward into `grads` ([n_need, B, T, D], mutated).  With `skip_if_equals` it is the one-pass step's 1-CTA gate:
+// nothing happens when grad_out * grad_out_scale equals it, otherwise the exact backward overwrites `grads`.
+void op_bwd(at::TensorList students, at::TensorList teachers, const c10::optional<at::Tensor>& mask,
+            const at::Tensor& grads, const at::Tensor& bwd_scale, const at::Tensor& grad_out, double grad_out_scale,
+            c10::optional<double> skip_if_equals, c10::List<bool> needs, int64_t loss_kind, bool cls, int64_t n_vis,
+            int64_t tuning) {
+  const int64_t L = (int64_t)students.size();
+  OpInputs in = op_inputs(students, teachers, mask, loss_kind, cls, n_vis, tuning);
+  const std::vector<bool> nd = op_needs(needs, L);
+  const at::Tensor& s0 = in.students[0];
+  TORCH_CHECK_VALUE(grads.is_contiguous() && grads.scalar_type() == s0.scalar_type() && grads.dim() == 4 &&
+                        grads.size(0) == count_needs(nd) && grads.sizes().slice(1) == s0.sizes(),
+                    "grads must be a contiguous [n_need, B, T, D] tensor of the student dtype");
+  TORCH_CHECK_VALUE(bwd_scale.is_contiguous() && bwd_scale.scalar_type() == at::kFloat && bwd_scale.numel() == 2 * L,
+                    "bwd_scale must be a contiguous float32 [2L] tensor");
+  const auto device = s0.device();
+  c10::cuda::CUDAGuard guard(device);
+  const cudaStream_t stream = c10::cuda::getCurrentCUDAStream(device.index()).stream();
+  const at::Tensor g = upstream(grad_out, device);
+  fill_grad_ptrs(grads, nd, in.tb);
+  const float skip = skip_if_equals.has_value() ? (float)*skip_if_equals : 0.f;
+  launch_bwd(in.shape, in.tb, in.mask, bwd_scale.data_ptr<float>(), g, (float)grad_out_scale,
+             skip_if_equals.has_value() ? &skip : nullptr, nullptr, stream);
+}
+
 }  // namespace
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
@@ -484,4 +686,21 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("distill", &distill, py::arg("plan"), py::arg("students"), py::arg("teachers"), py::arg("attn_mask"),
         py::arg("masks_out"), py::arg("comm"), py::arg("ticket"), py::arg("seen"), py::arg("tuning"));
   m.def("prefetch_counts", &prefetch_counts, py::arg("attn_mask"), py::arg("n_vis"), py::arg("comm"), py::arg("tuning"));
+}
+
+TORCH_LIBRARY(mafed, m) {
+  m.def("step(Tensor[] students, Tensor[] teachers, Tensor? mask, float[] layer_coeffs, float[]? lang_weights, "
+        "int modality_kind, float distill_coeff, int loss_kind, bool cls, int n_vis, float assumed_grad_out, "
+        "float grad_multiplier, bool[] needs, int comm, bool want_masks, int tuning) -> (Tensor, Tensor, Tensor, Tensor)");
+  m.def("fwd_step(Tensor[] students, Tensor[] teachers, Tensor? mask, float[] layer_coeffs, float[]? lang_weights, "
+        "int modality_kind, float distill_coeff, int loss_kind, bool cls, int n_vis, float grad_multiplier, bool[] needs, "
+        "int comm, bool want_masks, int tuning) -> (Tensor, Tensor, Tensor)");
+  m.def("bwd(Tensor[] students, Tensor[] teachers, Tensor? mask, Tensor(a!) grads, Tensor bwd_scale, Tensor grad_out, "
+        "float grad_out_scale, float? skip_if_equals, bool[] needs, int loss_kind, bool cls, int n_vis, int tuning) -> ()");
+}
+
+TORCH_LIBRARY_IMPL(mafed, CUDA, m) {
+  m.impl("step", &op_step);
+  m.impl("fwd_step", &op_fwd_step);
+  m.impl("bwd", &op_bwd);
 }

@@ -34,6 +34,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from . import cabi, node
+from . import comm as _comm
 from .comm import get_peer_comm
 
 _DTYPES = {torch.float32: cabi.F32, torch.bfloat16: cabi.BF16, torch.float16: cabi.F16}
@@ -484,6 +485,62 @@ def _step(plan: DistillPlan, attn_mask, group, teachers, mask_out, students, tic
                        peer.handle.value if peer is not None else 0, ticket, seen, cabi.active_tuning_address())
 
 
+@torch._dynamo.assume_constant_result
+def _compiled_comm(group, generation: int) -> int:
+    """The peer communicator's handle for a compiled step: 0 on one rank, -1 for the NCCL sequence.  It is a host object
+    Dynamo cannot trace, so it is read when the step is traced and becomes a constant of the graph; ``generation``
+    (``comm._generation``, which ``comm.reset()`` bumps) is read by the traced code, so Dynamo guards on it and a graph
+    is retraced rather than handed a torn-down communicator.  Tracing also puts the in-place pass back in front if the
+    caller replaced Inductor's post-grad pre-pass after the extension loaded."""
+    from . import ops
+    ops.install_graph_pass()
+    distributed, pg = resolve_group(group)
+    peer = get_peer_comm(pg) if distributed else None
+    return -1 if distributed and peer is None else (peer.handle.value if peer is not None else 0)
+
+
+def _op_step(plan: DistillPlan, attn_mask, teachers, mask_out, students, comm, tuning):
+    """One launch-sized step through the ``mafed::`` ops (``mafed_b200.ops``): what ``torch.compile`` traces."""
+    if not _native_dtypes(students, teachers):
+        students, teachers = [s.float() for s in students], [t.float() for t in teachers]
+    needs = [torch.is_grad_enabled() and s.requires_grad for s in students]
+    mask = None
+    if not plan.cls:
+        mask = attn_mask if attn_mask.dtype == torch.int64 else attn_mask.to(torch.int64)
+    want_masks = mask_out is not None and not plan.cls
+    args = (list(students), list(teachers), mask, [float(c) for c in plan.layer_coeffs],
+            None if plan.lang_weights is None else [float(c) for c in plan.lang_weights],
+            cabi.MODW_CLS if plan.cls else plan.modality_kind, float(plan.distill_coeff), plan.loss_kind,
+            bool(plan.cls), int(plan.n_vis))
+    if plan.single_pass and any(needs):
+        out, _, _, masks = torch.ops.mafed.step(*args, float(plan.assumed_grad_out), float(plan.grad_multiplier), needs,
+                                                comm, want_masks, tuning)
+    else:
+        out, _, masks = torch.ops.mafed.fwd_step(*args, float(plan.grad_multiplier), needs, comm, want_masks, tuning)
+    if not want_masks:
+        masks = None
+    elif torch.is_tensor(mask_out):
+        mask_out.copy_(masks)
+        masks = mask_out
+    return out[0], out[1:], masks
+
+
+# The NCCL sequence (a process group without a peer communicator) is host-driven: it runs eagerly, behind a graph break.
+_step_eager = torch.compiler.disable(_step)
+
+
+def _any_step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen):
+    if not torch.compiler.is_compiling():
+        return _step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
+    node.load()
+    comm = _compiled_comm(group, _comm._generation)
+    # a plain int global: Dynamo guards on it, so a step traced inside `with cabi.tuning(...)` is retraced outside it
+    tuning = cabi._active_tuning_address
+    if comm == -1:
+        return _step_eager(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
+    return _op_step(plan, attn_mask, teachers, mask_out, students, comm, tuning)
+
+
 def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tensor], attn_mask, plan: DistillPlan,
                  group=None, teachers_detached: bool = False, mask_out=None, ticket=None, seen=None,
                  return_masks: bool = False):
@@ -497,6 +554,11 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
     the result.
     ``ticket``: the token counts sent ahead of the step (``prefetch_counts``).  ``seen``: pinned float32 tensor
     that receives the upstream gradient the backward gate saw.
+
+    Under ``torch.compile`` the step runs through the ``mafed::`` ops (``mafed_b200.ops``), which Dynamo traces into the
+    caller's graph; ``ticket`` and ``seen`` are ignored there (the kernel exchanges the counts itself; nothing records
+    the upstream gradient).  A process group without a peer communicator (the NCCL sequence) is not compiled: the
+    step runs eagerly behind a graph break.
     """
     if not teachers_detached:
         teachers = [t.detach() for t in teachers]
@@ -506,7 +568,7 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
     # sides, as the reference does under autocast, distillation.py:90,244)
     n = len(students)
     if n <= cabi.MAX_LAYERS:
-        total, aux, both = _step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
+        total, aux, both = _any_step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
         if not return_masks:
             return total, aux
         return total, aux, (None if both is None else (both[0], both[1]))
@@ -520,7 +582,7 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
                           loss_kind=plan.loss_kind, cls=plan.cls, n_vis=plan.n_vis,
                           grad_multiplier=plan.grad_multiplier, single_pass=plan.single_pass,
                           assumed_grad_out=plan.assumed_grad_out)
-        part, aux, masks = _step(sub, attn_mask, group, teachers[lo:hi], mask_out if lo == 0 else None,
+        part, aux, masks = _any_step(sub, attn_mask, group, teachers[lo:hi], mask_out if lo == 0 else None,
                                  students[lo:hi], ticket, seen)
         if lo == 0:
             both = masks

@@ -37,6 +37,11 @@ except Exception:  # pragma: no cover
     _wandb = None
 
 
+def _identity(x):
+    """A plan-cache key part: plain values by value, objects by identity (Dynamo traces ``id()`` of objects only)."""
+    return x if x is None or isinstance(x, (bool, int, float, str)) else id(x)
+
+
 class _CapturedOutput:
     """Model output whose ``hidden_states`` holds only the captured (distilled) entries."""
 
@@ -259,14 +264,33 @@ class FeatureDistillation(CLStrategy):
         # `.detach()` of the reference (`_get_past_hidden_states`, distillation.py:223) is only paid for the distilled
         # layers, and only if a tensor carries a graph at all
         past_hidden_states = self._past_states(batch, layers)
-        if self.adapt_assumed_grad_out and self._gout_seen_np is not None:
+        # Under torch.compile the host-only bookkeeping is skipped, so the step traces without a graph break: no
+        # re-aiming of `assumed_grad_out` (the gate still keeps the gradients exact), no counts ticket (the kernel
+        # exchanges the counts itself), no exchange check and no W&B queue -- `record_step()` does the last two eagerly.
+        compiling = torch.compiler.is_compiling()
+        if self.adapt_assumed_grad_out and self._gout_seen_np is not None and not compiling:
             self._adapt_assumed()
         plan = self._step_plan(layers)
         hidden = output.hidden_states
         total, aux = self._launch(plan, batch, [hidden[l] for l in layers], past_hidden_states, teachers_detached=True)
-        self._record(aux, layers)
-        self.step += 1
+        if compiling:
+            # `self.step` is advanced by record_step(): an int attribute changed inside the trace would be guarded on,
+            # and every step would retrace (or feed a new int to the graph, which CUDA-graph trees re-record for)
+            self.last_layer_losses = aux
+            self.last_layers = list(layers)
+        else:
+            self._record(aux, layers)
+            self.step += 1
         return total
+
+    def record_step(self):
+        """The host side of a step that ran under ``torch.compile``: queue its per-layer losses for W&B (one
+        ``wandb.log`` per layer per step, in order, as ``distill`` does eagerly) and check the in-kernel exchange of a
+        batch-sharded run, and advance ``step``.  Call it once after every compiled step, outside the compiled region (with
+        ``mode="reduce-overhead"``, before the next replay overwrites ``last_layer_losses``)."""
+        if self.last_layer_losses is not None:
+            self._record(self.last_layer_losses, self.last_layers)
+        self.step += 1
 
     def _step_plan(self, layers) -> DistillPlan:
         """The plan of the all-layer step, rebuilt only when something it depends on changes (the host
@@ -274,13 +298,13 @@ class FeatureDistillation(CLStrategy):
         lw = self.loss_weights
         coeff = getattr(lw, "lang_coeff", None)
         key = (tuple(layers), self.distillation_coeff, self._cls_distillation, self._loss_kind, self.num_vision_tokens,
-               self.single_pass, self.assumed_grad_out, lw._modality_weighing_strategy, id(coeff),
-               getattr(coeff, "_version", None), id(lw.layer_coeffs), self.grad_multiplier, self.process_group)
+               self.single_pass, self.assumed_grad_out, lw._modality_weighing_strategy, _identity(coeff),
+               getattr(coeff, "_version", None), _identity(lw.layer_coeffs), self.grad_multiplier, self.process_group)
         if self._plan_cache is None or self._plan_cache[0] != key:
             coeffs, modality_kind, lang_weights = self._tables(layers)
             plan = self._plan(layers, coeffs, self.distillation_coeff, modality_kind, lang_weights)
-            if len(layers) <= cabi.MAX_LAYERS:
-                plan.weights()
+            if len(layers) <= cabi.MAX_LAYERS and not torch.compiler.is_compiling():
+                plan.weights()      # the ctypes tables of the eager path (the compiled ops take plain values)
             self._plan_cache = (key, plan)
         return self._plan_cache[1]
 
@@ -341,11 +365,11 @@ class FeatureDistillation(CLStrategy):
                     mask_out = True
                 else:
                     batch["lang_masks"], batch["image_masks"] = modality_masks(attn, self.num_vision_tokens)
-            if self._tickets:
+            if self._tickets and not torch.compiler.is_compiling():
                 tk = self._tickets.pop(id(attn), None)
                 if tk is not None and tk[0] is attn and tk[1] == attn._version:
                     ticket = tk[2]
-        if plan.single_pass and self._gout_seen is None:
+        if plan.single_pass and self._gout_seen is None and not torch.compiler.is_compiling():
             self._gout_seen = seen_slot()
             self._gout_seen_np = self._gout_seen.numpy()
         total, aux, masks = distill_loss(students, teachers, attn, plan, group=self.process_group,

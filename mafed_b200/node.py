@@ -1,7 +1,8 @@
 """Loader of the compiled autograd node (``csrc/torch_node.cpp`` -> ``_lib/mafed_torch_node*.so``).
 
 The extension is host C++ only: it binds the C ABI of ``libmafed_distill.so`` at run time and turns one
-``distill()`` into one call.  Like the library it is built in-tree (``python -m mafed_b200.build``) and there is
+``distill()`` into one call.  It also defines the ``mafed::`` torch.library ops that compiled callers trace
+(``mafed_b200.ops``).  Like the library it is built in-tree (``python -m mafed_b200.build``) and there is
 nothing to fall back to when it is missing.
 """
 from __future__ import annotations
@@ -39,5 +40,7 @@ def load():
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
         mod.bind(cabi.LIB_PATH)
+        from . import ops
+        ops.register()      # fake implementations and autograd of the mafed:: ops the extension defines
         _ext = mod
     return _ext
