@@ -9,6 +9,10 @@ the embedding output after dropout), entry ``L`` is the output of ``final_layer_
 
 The captured student tensors are the graph's own tensors, so gradients of the distillation loss flow into
 the model exactly as with ``output.hidden_states``.
+
+With ``stop_after_last=True`` the forward ends as soon as the highest captured entry is stored: the decoder layers
+after it, ``final_layer_norm`` (unless entry ``L`` is captured) and whatever the model computes from the decoder's output
+(the LM head and its logits) never run, and the model call returns nothing.
 """
 from __future__ import annotations
 
@@ -50,12 +54,21 @@ class HiddenStateTuple(Sequence):
         return self._states[index]
 
 
+class _StopForward(Exception):
+    """Raised by the hook of the highest captured entry to end the forward there; ``args[0]`` is the capture that
+    raised it, so that only its own ``__exit__`` suppresses it."""
+
+
 class HiddenStateCapture:
     """Context manager: ``with HiddenStateCapture(model, layers) as cap: model(**batch)`` then
-    ``cap.hidden_states[layer]``."""
+    ``cap.hidden_states[layer]``.
+
+    ``stop_after_last=True``: the hook of the highest captured entry stores it and then stops the forward (for an entry
+    ``i < L`` before decoder layer ``i`` runs, for entry ``L`` after ``final_layer_norm``).  ``__exit__`` suppresses only
+    that stop; any other exception propagates.  The model call then returns nothing, so read the states from ``cap``."""
 
     def __init__(self, model: nn.Module, layers: Iterable[int], layer_modules: Optional[nn.ModuleList] = None,
-                 final_norm: Optional[nn.Module] = None, detach: bool = False):
+                 final_norm: Optional[nn.Module] = None, detach: bool = False, stop_after_last: bool = False):
         if layer_modules is None:
             layer_modules, found_norm = find_decoder(model)
             final_norm = final_norm if final_norm is not None else found_norm
@@ -69,11 +82,14 @@ class HiddenStateCapture:
         if self.n_states - 1 in self.layers and final_norm is None:
             raise AttributeError("the last hidden state needs `final_norm=`")
         self.detach = detach
+        self._stop_at = self.layers[-1] if stop_after_last and self.layers else None
         self.states: Dict[int, torch.Tensor] = {}
         self._handles = []
 
     def _store(self, index: int, tensor: torch.Tensor):
         self.states[index] = tensor.detach() if self.detach else tensor
+        if index == self._stop_at:
+            raise _StopForward(self)
 
     def __enter__(self):
         self.states.clear()
@@ -90,11 +106,11 @@ class HiddenStateCapture:
                 self._handles.append(self.layer_modules[index].register_forward_pre_hook(pre_hook, with_kwargs=True))
         return self
 
-    def __exit__(self, *exc):
+    def __exit__(self, exc_type, exc, tb):
         for h in self._handles:
             h.remove()
         self._handles.clear()
-        return False
+        return exc_type is _StopForward and exc.args[0] is self
 
     @property
     def hidden_states(self) -> HiddenStateTuple:

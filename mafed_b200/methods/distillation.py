@@ -136,6 +136,10 @@ class FeatureDistillation(CLStrategy):
         self.teacher_dtype = kwargs.get("teacher_dtype")
         if self.teacher_dtype not in (None, torch.bfloat16, torch.float16):
             raise ValueError(f"teacher_dtype must be None, torch.bfloat16 or torch.float16, not {self.teacher_dtype!r}")
+        # stop the teacher forward after the last distilled hidden state (and the student's too when no replay loss is
+        # taken): the layers after it, the final layer norm and the LM head compute nothing the step reads.  Eager only:
+        # under torch.compile the forwards run in full (see _stop_early)
+        self.early_exit = bool(kwargs.get("early_exit", False))
         self._mem_iter = self._mem_iter_source = None
         self._mem_epoch = 0
         self._plan_cache = None
@@ -180,10 +184,14 @@ class FeatureDistillation(CLStrategy):
         if self.distillation_coeff != 0 and not self._cls_distillation:
             # batch-sharded: this rank's token counts leave for the peers now, behind the student forward
             self.prefetch_counts(batch)
+        # without a replay loss nothing reads the student's output past the last distilled hidden state
+        stop_student = not do_replay and self._stop_early()
         with torch.autocast("cuda", dtype=torch.bfloat16):
-            if self.selective_capture and self.distillation_coeff != 0:
+            if (self.selective_capture or stop_student) and self.distillation_coeff != 0:
                 # keep only the distilled entries of the hidden-state tuple alive (SURVEY 8f rank 2)
-                with HiddenStateCapture(model, self.loss_weights.get_distillation_layers()) as cap:
+                output = None       # stays None when the capture stops the forward: no logits, no loss
+                with HiddenStateCapture(model, self.loss_weights.get_distillation_layers(),
+                                        stop_after_last=stop_student) as cap:
                     output = model(**batch, compute_loss=do_replay, output_hidden_states=False, return_dict=True)
                 output = _CapturedOutput(output, cap.hidden_states)
             else:
@@ -394,13 +402,19 @@ class FeatureDistillation(CLStrategy):
         state in one dtype, so the step reads them natively instead of up-casting every layer."""
         return h if self.teacher_dtype is None or h.dtype == self.teacher_dtype else h.to(self.teacher_dtype)
 
+    def _stop_early(self) -> bool:
+        """``early_exit`` in effect: eager calls only.  A compiled step keeps the full forwards, which trace into one
+        graph; the capture's hooks and the exception that stops the forward would not."""
+        return self.early_exit and not torch.compiler.is_compiling()
+
     def _past_states(self, batch, layers):
         """Teacher hidden states of the distilled layers only (same forward and side effects as
-        ``_get_past_hidden_states``)."""
+        ``_get_past_hidden_states``; with ``early_exit`` the forward stops after the last of them)."""
+        stop = self._stop_early()
         with torch.no_grad(), self._teacher_forward(batch):
             batch.pop("labels", None)
-            if self.selective_capture:
-                with HiddenStateCapture(self.past_model, layers, detach=True) as cap:
+            if self.selective_capture or stop:
+                with HiddenStateCapture(self.past_model, layers, detach=True, stop_after_last=stop) as cap:
                     self.past_model(**batch, output_hidden_states=False, return_dict=True)
                 states = cap.hidden_states
             else:
