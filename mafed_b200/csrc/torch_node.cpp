@@ -352,7 +352,7 @@ struct DistillBackward : public Node {
 
 // ---------------------------------------------------------------- forward
 // students / teachers: the selected [B, T, D] hidden states (same shape and device; one dtype, or fp32 students with
-// bf16 / fp16 teachers -- other mixes are up-cast to fp32).  attn_mask: int64 [B, T - n_vis]
+// bf16 / fp16 teachers -- other mixes, the refused pairs, are up-cast to fp32).  attn_mask: int64 [B, T - n_vis]
 // (ignored in cls mode).  masks_out: None, an int64 [2, B, T] tensor, or True to have one allocated here; it receives
 // (lang_masks, image_masks).  comm: a mafed_comm_t* (0: single rank).  ticket: optional int64[4] from
 // prefetch_counts.  seen: optional pinned float[1].
@@ -366,8 +366,9 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
   TORCH_CHECK((int)students.size() == L && (int)teachers.size() == L, "students / teachers / plan length mismatch");
   {
     // One dtype everywhere, or fp32 students with teachers of one half-precision dtype: the kernels read the tensors
-    // as they are (a teacher pair, MAFED_DTYPE_PAIR).  Any other mix -- layers of different dtypes, a student narrower
-    // than its teacher -- is up-cast to fp32 on both sides, which is what the reference's autocast region does to
+    // as they are (a teacher pair, MAFED_DTYPE_PAIR).  distill_loss gives each dtype group of a step its own call, so
+    // any other mix arriving here is the one group of pairs the kernels refuse (a student narrower than its teacher,
+    // bf16 against fp16).  It is up-cast to fp32 on both sides, which is what the reference's autocast region does to
     // the inputs of its loss functions (distillation.py:90,244); the casts are ordinary autograd ops.
     const at::ScalarType s_type = students[0].scalar_type(), t_type = teachers[0].scalar_type();
     bool uniform = true;
@@ -531,7 +532,8 @@ std::shared_ptr<CountsTicket> prefetch_counts(const at::Tensor& attn_mask, int64
 // torch.compile can trace a step into the caller's graph (the pybind `distill` above builds its own autograd node,
 // which Dynamo cannot trace).  Their fake implementations and the autograd formula live in mafed_b200/ops.py.  The
 // plan arrives as plain values; the workspace is scratch from the caching allocator, as in `distill`.  The ops take
-// one dtype everywhere, or fp32 students with bf16 / fp16 teachers: other mixes are up-cast by the caller.
+// one dtype everywhere, or fp32 students with bf16 / fp16 teachers: the caller splits a step into dtype groups and
+// up-casts a group of refused pairs.
 
 struct OpInputs {
   std::vector<at::Tensor> students, teachers;

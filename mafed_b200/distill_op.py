@@ -44,12 +44,61 @@ _TEACHER_PAIRS = {(torch.float32, torch.bfloat16), (torch.float32, torch.float16
 
 def _native_dtypes(students, teachers) -> bool:
     """True when the kernels take these layers without an up-cast: one dtype everywhere, or fp32 students with
-    teachers of one half-precision dtype."""
+    teachers of one half-precision dtype.  ``distill_loss`` splits a step into dtype groups first
+    (``dtype_groups``), so a launch-sized step that fails this is the one group of pairs the kernels refuse (a
+    half-precision student against an fp32 teacher, bf16 against fp16): that group alone is up-cast to fp32."""
     s_types, t_types = {t.dtype for t in students}, {t.dtype for t in teachers}
     if len(s_types) != 1 or len(t_types) != 1:
         return False
     pair = (next(iter(s_types)), next(iter(t_types)))
     return pair[0] == pair[1] or pair in _TEACHER_PAIRS
+
+
+def dtype_groups(pairs: Sequence[tuple]) -> Optional[List[List[int]]]:
+    """The layers of a step partitioned by their ``(student dtype, teacher dtype)`` pair, or ``None`` when one launch
+    takes them all (every layer has the same pair).
+
+    One group per pair the kernels read as it is (one dtype, or fp32 with bf16 / fp16), in the order of each pair's
+    first layer; then, if any, one group of every layer whose pair the kernels refuse, which that step up-casts to
+    fp32.  Layer order is kept inside each group.  A single group is ``None`` as well."""
+    first = pairs[0]
+    if all(p == first for p in pairs):
+        return None
+    native, refused = {}, []
+    for i, p in enumerate(pairs):
+        if p[0] == p[1] or p in _TEACHER_PAIRS:
+            native.setdefault(p, []).append(i)
+        else:
+            refused.append(i)
+    groups = list(native.values()) + ([refused] if refused else [])
+    return groups if len(groups) > 1 else None
+
+
+def sub_steps(n: int, groups: Optional[List[List[int]]]) -> Optional[List[List[int]]]:
+    """The layer indices of each launch of a step over ``n`` layers: each dtype group (``dtype_groups``) cut into
+    chunks of at most ``MAFED_MAX_LAYERS``.  ``None``: one launch over all of them."""
+    if groups is None:
+        if n <= cabi.MAX_LAYERS:
+            return None
+        groups = [list(range(n))]
+    return [g[lo:lo + cabi.MAX_LAYERS] for g in groups for lo in range(0, len(g), cabi.MAX_LAYERS)]
+
+
+def aux_runs(steps: List[List[int]]):
+    """How to lay the sub-steps' ``aux`` vectors back out in the caller's layer order: ``(k, lo, hi)`` for each maximal
+    run of caller positions that are layers ``lo:hi`` of sub-step ``k``, in caller order."""
+    where = {}
+    for k, idx in enumerate(steps):
+        for j, i in enumerate(idx):
+            where[i] = (k, j)
+    runs = []
+    for i in range(len(where)):
+        k, j = where[i]
+        if runs and runs[-1][0] == k and runs[-1][2] == j:
+            runs[-1][2] = j + 1
+        else:
+            runs.append([k, j, j + 1])
+    return [tuple(r) for r in runs]
 
 
 @dataclass
@@ -68,6 +117,28 @@ class DistillPlan:
     assumed_grad_out: float = 1.0           # upstream gradient the one-pass step bakes in
     _weights: Optional[cabi.Weights] = field(default=None, repr=False)
     _node_plan: object = field(default=None, repr=False)
+    _splits: dict = field(default_factory=dict, repr=False)
+
+    def split(self, pairs: tuple):
+        """The launches of a step whose layers have these ``(student, teacher)`` dtype pairs: ``None`` for one
+        launch over every layer, else ``(steps, runs)`` -- ``(layer indices, sub-plan)`` per launch, and
+        ``aux_runs``.  Built once per dtype signature (a plan's host tables cost ~50 us of Python)."""
+        if pairs not in self._splits:
+            idx_lists = sub_steps(len(pairs), dtype_groups(pairs))
+            if idx_lists is None:
+                self._splits[pairs] = None
+            else:
+                steps = [(idx, self._sub_plan(idx)) for idx in idx_lists]
+                self._splits[pairs] = (steps, aux_runs(idx_lists))
+        return self._splits[pairs]
+
+    def _sub_plan(self, idx: List[int]) -> "DistillPlan":
+        return DistillPlan(layers=[self.layers[i] for i in idx], layer_coeffs=[self.layer_coeffs[i] for i in idx],
+                           distill_coeff=self.distill_coeff, modality_kind=self.modality_kind,
+                           lang_weights=None if self.lang_weights is None else [self.lang_weights[i] for i in idx],
+                           loss_kind=self.loss_kind, cls=self.cls, n_vis=self.n_vis,
+                           grad_multiplier=self.grad_multiplier, single_pass=self.single_pass,
+                           assumed_grad_out=self.assumed_grad_out)
 
     def weights(self) -> cabi.Weights:
         if self._weights is None:
@@ -232,7 +303,25 @@ def modality_masks_into(attn_mask: torch.Tensor, n_vis: int, lang: torch.Tensor,
 def token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n_vis: int) -> torch.Tensor:
     """Masked per-modality sums of the per-token L2 norms of ``len(tensors)`` ``[B, T, D]`` tensors in one
     fused pass (``distillation_loss_weights.py:122-137``).  Returns device fp64 ``[2L + 2]``:
-    ``(text sum, vision sum)`` per tensor, then ``(n_text, n_vision)``.  No host synchronisation."""
+    ``(text sum, vision sum)`` per tensor, then ``(n_text, n_vision)``.  No host synchronisation.
+
+    Tensors of several dtypes (the gradients w.r.t. a bf16 model's hidden states next to the fp32 output of its final
+    layer norm) take one pass per dtype; the per-tensor sums are laid out in the caller's order, the counts taken once."""
+    by_dtype = {}
+    for i, t in enumerate(tensors):
+        by_dtype.setdefault(t.dtype, []).append(i)
+    if len(by_dtype) == 1:
+        return _token_norm_sums(tensors, attn_mask, n_vis)
+    rows = [None] * len(tensors)
+    for idx in by_dtype.values():
+        sums = _token_norm_sums([tensors[i] for i in idx], attn_mask, n_vis)
+        for j, i in enumerate(idx):
+            rows[i] = sums[2 * j:2 * j + 2]
+    return torch.cat(rows + [sums[2 * len(idx):]])
+
+
+def _token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n_vis: int) -> torch.Tensor:
+    """``token_norm_sums`` over tensors of one dtype: one pass."""
     lib = cabi.load()
     tensors = _prepare([t.detach() for t in tensors])
     plan = DistillPlan(layers=list(range(len(tensors))), layer_coeffs=[1.0] * len(tensors), n_vis=n_vis)
@@ -554,6 +643,7 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
     the result.
     ``ticket``: the token counts sent ahead of the step (``prefetch_counts``).  ``seen``: pinned float32 tensor
     that receives the upstream gradient the backward gate saw.
+    Layers may differ in dtype: each ``(student, teacher)`` dtype group runs as its own launch (``dtype_groups``).
 
     Under ``torch.compile`` the step runs through the ``mafed::`` ops (``mafed_b200.ops``), which Dynamo traces into the
     caller's graph; ``ticket`` and ``seen`` are ignored there (the kernel exchanges the counts itself; nothing records
@@ -564,32 +654,34 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
         teachers = [t.detach() for t in teachers]
     if len(students) != len(teachers) or len(students) != len(plan.layers):
         raise ValueError("students / teachers / plan.layers length mismatch")
-    # (fp32 students with bf16 / fp16 teachers run as they are; other mixes of dtypes are up-cast to fp32 on both
-    # sides, as the reference does under autocast, distillation.py:90,244)
-    n = len(students)
-    if n <= cabi.MAX_LAYERS:
+    # Layers of several dtype pairs, or more of them than one launch carries (MAFED_MAX_LAYERS): one launch per dtype
+    # group and chunk.  Each group runs natively at its own width; only a group of pairs the kernels refuse is up-cast
+    # to fp32 on both sides (inside its step), as the reference's autocast region does to the inputs of its loss
+    # functions (distillation.py:90,244).  Every launch has its own backward gate, and across batch shards its own
+    # exchange: the groups come from the model's dtypes, so every rank runs the same sequence.  A counts ticket is only
+    # read by a step, so every launch may take it.
+    s_type, t_type = students[0].dtype, teachers[0].dtype
+    one_launch = len(students) <= cabi.MAX_LAYERS
+    for s, t in zip(students, teachers):
+        one_launch = one_launch and s.dtype == s_type and t.dtype == t_type
+    split = None if one_launch else plan.split(tuple([(s.dtype, t.dtype) for s, t in zip(students, teachers)]))
+    if split is None:
         total, aux, both = _any_step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
         if not return_masks:
             return total, aux
         return total, aux, (None if both is None else (both[0], both[1]))
-    # more selected layers than one launch carries (MAFED_MAX_LAYERS): chunk and add the partial totals
-    total, layer_losses, modal_losses, both = None, [], [], None
-    for lo in range(0, n, cabi.MAX_LAYERS):
-        hi = min(n, lo + cabi.MAX_LAYERS)
-        sub = DistillPlan(layers=plan.layers[lo:hi], layer_coeffs=plan.layer_coeffs[lo:hi],
-                          distill_coeff=plan.distill_coeff, modality_kind=plan.modality_kind,
-                          lang_weights=None if plan.lang_weights is None else plan.lang_weights[lo:hi],
-                          loss_kind=plan.loss_kind, cls=plan.cls, n_vis=plan.n_vis,
-                          grad_multiplier=plan.grad_multiplier, single_pass=plan.single_pass,
-                          assumed_grad_out=plan.assumed_grad_out)
-        part, aux, masks = _any_step(sub, attn_mask, group, teachers[lo:hi], mask_out if lo == 0 else None,
-                                 students[lo:hi], ticket, seen)
-        if lo == 0:
+    steps, runs = split
+    total, parts, both = None, [], None
+    for k, (idx, sub) in enumerate(steps):
+        part, aux, masks = _any_step(sub, attn_mask, group, [teachers[i] for i in idx], mask_out if k == 0 else None,
+                                     [students[i] for i in idx], ticket, seen)
+        if k == 0:
             both = masks
         total = part if total is None else total + part
-        layer_losses.append(aux[: hi - lo])
-        modal_losses.append(aux[hi - lo:])
-    aux = torch.cat(layer_losses + modal_losses)
+        parts.append(aux)
+    # aux in the caller's layer order: layer losses, then (text, vision) pairs
+    aux = torch.cat([parts[k][lo:hi] for k, lo, hi in runs] +
+                    [parts[k][len(steps[k][0]) + 2 * lo:len(steps[k][0]) + 2 * hi] for k, lo, hi in runs])
     if not return_masks:
         return total, aux
     return total, aux, (None if both is None else (both[0], both[1]))

@@ -9,6 +9,9 @@ per-rank gradients must equal the single-device CPU oracle on the full batch (SU
 
 ``--teacher-dtype {bf16,fp16}``: instead, fp32 student states against a teacher in that dtype (read as it is by the
 kernels); every rank's loss and gradient slice must equal the same step run on one GPU over the concatenated batch.
+
+``--mixed-layers``: instead, layers of several dtypes in one step (a bf16 model's states next to its fp32 final-layer-norm
+entry, one launch and one exchange per dtype group), with and without token counts sent ahead; compared the same way.
 """
 import argparse
 import os
@@ -26,6 +29,8 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--teacher-dtype", choices=["bf16", "fp16"], default=None,
                     help="fp32 students against a teacher in this dtype (default: today's same-dtype cases)")
+    ap.add_argument("--mixed-layers", action="store_true",
+                    help="layers of several dtypes in one step, one launch per dtype group")
     args = ap.parse_args()
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
@@ -34,6 +39,8 @@ def main():
     if args.teacher_dtype is not None:
         ok = mixed_teacher_check(rank, world, {"bf16": torch.bfloat16, "fp16": torch.float16}[args.teacher_dtype])
         finish(ok)
+    if args.mixed_layers:
+        finish(mixed_layers_check(rank, world))
     from gpu_util import Out, make_method, rel_err
     from golden_util import oracle_cfg
     from oracle import distill_oracle as O
@@ -134,6 +141,60 @@ def mixed_teacher_check(rank, world, teacher_dtype):
         ok &= good
         print(f"rank {rank}/{world} ({mode}) fp32 student, {teacher_dtype} teacher, {loss} single_pass={single_pass}: "
               f"loss err {e_loss:.2e} gradients {'equal' if same else 'DIFFER'} {'OK' if good else 'FAIL'}", flush=True)
+    return ok
+
+
+def mixed_layers_check(rank, world):
+    """Students and teachers {bf16 x 3, fp32}: one launch per dtype group, each with its own exchange, one-pass and
+    two-pass, with the token counts exchanged in the kernels or sent ahead (``prefetch_counts``, whose ticket every
+    group's launch reads).  The loss equals the one-GPU step on the concatenated batch to 1e-6 and every rank's gradient
+    slice equals it bit for bit (mse) or within 1e-6 / 2e-3 for fp32 / bf16 (cosine)."""
+    from gpu_util import Out, make_method, rel_err
+    from mafed_b200.comm import get_peer_comm
+    from oracle import distill_oracle as O
+    peer = get_peer_comm(None)
+    mode = "nccl" if peer is None else "peer-memory"
+    dtypes = [torch.bfloat16] * 3 + [torch.float32]
+    ok = True
+    for loss, single_pass, ahead in [("mse", True, False), ("cosine", True, False), ("mse", False, False),
+                                     ("cosine", False, False), ("mse", True, True), ("mse", False, True)]:
+        B = 4 * world + 2
+        st, te, am = O.make_inputs(4, B, 9, 768, n_vis=256, seed=43, mask="ragged", teacher="independent")
+        meta = dict(modality="balanced", layer_strategy="discounted", loss=loss, gamma=0.5, num_hidden_layers=4,
+                    layer=None, n_vis=256, coeff=1.0, cls=False, lang_coeff=None)
+        lo = rank * 4
+        hi = B if rank == world - 1 else lo + 4
+
+        def run(a, b, group):
+            fd = make_method(meta, single_pass=single_pass)
+            fd.grad_multiplier = 1.0
+            fd.process_group = group
+            leaves = [s[a:b].to(d).cuda().contiguous().requires_grad_(True) for s, d in zip(st, dtypes)]
+            teach = [t[a:b].to(d).cuda().contiguous() for t, d in zip(te, dtypes)]
+            fd.past_model = lambda **kw: Out(tuple(teach))
+            batch = {"attention_mask": am[a:b].cuda().contiguous()}
+            if ahead and group is None:
+                assert fd.prefetch_counts(batch) is not None or peer is None
+            loss_v = fd.distill(Out(tuple(leaves)), batch)
+            (loss_v * 0.5).backward()
+            torch.cuda.synchronize()
+            return loss_v.detach(), [l.grad for l in leaves]
+
+        loss_s, g_s = run(lo, hi, None)
+        loss_f, g_f = run(0, B, False)
+        e_loss = abs(float(loss_s) - float(loss_f)) / abs(float(loss_f))
+        pairs = [(a, b[lo:hi]) for a, b in zip(g_s, g_f)]
+        if loss == "mse":
+            same = all(a.dtype == b.dtype and torch.equal(a, b) for a, b in pairs)
+        else:
+            same = all(rel_err(a.cpu(), b.cpu()) < (1e-6 if a.dtype == torch.float32 else 2e-3) for a, b in pairs)
+        good = e_loss < 1e-6 and same
+        ok &= good
+        print(f"rank {rank}/{world} ({mode}) bf16 x 3 + fp32 layers, {loss} single_pass={single_pass} "
+              f"counts_ahead={ahead}: loss err {e_loss:.2e} gradients {'equal' if same else 'DIFFER'} "
+              f"{'OK' if good else 'FAIL'}", flush=True)
+    if peer is not None:
+        ok &= peer.status() == 0
     return ok
 
 
