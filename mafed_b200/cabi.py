@@ -217,10 +217,11 @@ def make_shape(n_layers, B, T, n_vis, D, dtype, loss_kind, cls=False, teacher_dt
 
 
 # ---- the stage combinations the path uses (one flag set each of mafed_distill_scalar_stage)
-def reduce_stage(lib, shape_ref, mask_ptr, ws_ptr, sums_ptr, stream):
-    """REDUCE|COUNTS: the rank-local sums vector before an allreduce."""
+def reduce_stage(lib, shape_ref, mask_ptr, ws_ptr, sums_ptr, stream, comm=None):
+    """REDUCE|COUNTS: the rank-local sums vector before an allreduce; with a peer communicator ``comm`` the global one,
+    the whole vector summed over the ranks' mailboxes in rank order by the same launch."""
     return lib.mafed_distill_scalar_stage(shape_ref, None, STAGE_REDUCE | STAGE_COUNTS, mask_ptr, ws_ptr, sums_ptr,
-                                          None, None, None, 0, stream)
+                                          None, None, comm, COMM_SUMS | COMM_COUNTS if comm is not None else 0, stream)
 
 
 def finalize_stage(lib, shape_ref, weights_ref, sums_ptr, out_ptr, bwd_scale_ptr, stream):

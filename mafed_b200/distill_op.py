@@ -300,28 +300,43 @@ def modality_masks_into(attn_mask: torch.Tensor, n_vis: int, lang: torch.Tensor,
                    "mafed_distill_modality_masks")
 
 
-def token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n_vis: int) -> torch.Tensor:
+def token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n_vis: int, group=False) -> torch.Tensor:
     """Masked per-modality sums of the per-token L2 norms of ``len(tensors)`` ``[B, T, D]`` tensors in one
     fused pass (``distillation_loss_weights.py:122-137``).  Returns device fp64 ``[2L + 2]``:
     ``(text sum, vision sum)`` per tensor, then ``(n_text, n_vision)``.  No host synchronisation.
 
     Tensors of several dtypes (the gradients w.r.t. a bf16 model's hidden states next to the fp32 output of its final
-    layer norm) take one pass per dtype; the per-tensor sums are laid out in the caller's order, the counts taken once."""
+    layer norm) take one pass per dtype; the per-tensor sums are laid out in the caller's order, the counts taken once.
+
+    ``group``: ``False`` (the default) returns this process's vector.  Otherwise (``None``: the default process group;
+    see ``resolve_group``) the tensors are this rank's batch shard and every rank gets the vector of the whole batch,
+    identical on every rank; every rank of the group must make the call.  With a peer-memory communicator the pass's
+    reduce launch sums the vector over the ranks in rank order (no extra launch, no NCCL call); without one
+    (``MAFED_B200_DIST=nccl``, ranks on several hosts) the vector is allreduced.  Tensors of several dtypes are exchanged
+    once, as the assembled vector, by the allreduce: the reduce launch exchanges the vector of its own pass only."""
+    distributed, pg = resolve_group(group)
     by_dtype = {}
     for i, t in enumerate(tensors):
         by_dtype.setdefault(t.dtype, []).append(i)
     if len(by_dtype) == 1:
-        return _token_norm_sums(tensors, attn_mask, n_vis)
+        peer = get_peer_comm(pg) if distributed else None
+        sums = _token_norm_sums(tensors, attn_mask, n_vis, peer)
+        if distributed and peer is None:
+            allreduce_sums(sums, pg)
+        return sums
     rows = [None] * len(tensors)
     for idx in by_dtype.values():
         sums = _token_norm_sums([tensors[i] for i in idx], attn_mask, n_vis)
         for j, i in enumerate(idx):
             rows[i] = sums[2 * j:2 * j + 2]
-    return torch.cat(rows + [sums[2 * len(idx):]])
+    sums = torch.cat(rows + [sums[2 * len(idx):]])
+    if distributed:
+        allreduce_sums(sums, pg)
+    return sums
 
 
-def _token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n_vis: int) -> torch.Tensor:
-    """``token_norm_sums`` over tensors of one dtype: one pass."""
+def _token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n_vis: int, peer=None) -> torch.Tensor:
+    """``token_norm_sums`` over tensors of one dtype: one pass (summed over the ranks of ``peer``, a ``PeerComm``)."""
     lib = cabi.load()
     tensors = _prepare([t.detach() for t in tensors])
     plan = DistillPlan(layers=list(range(len(tensors))), layer_coeffs=[1.0] * len(tensors), n_vis=n_vis)
@@ -333,8 +348,8 @@ def _token_norm_sums(tensors: Sequence[torch.Tensor], attn_mask: torch.Tensor, n
         sums = torch.empty(2 * L + 2, dtype=torch.float64, device=dev)
         cabi.check(lib.mafed_distill_token_norm_sums(ln.shape_ref, ln.s_ptrs, ln.mask_ptr, ws.data_ptr(), stream),
                    "mafed_distill_token_norm_sums")
-        cabi.check(cabi.reduce_stage(lib, ln.shape_ref, ln.mask_ptr, ws.data_ptr(), sums.data_ptr(), stream),
-                   "mafed_distill_scalar_stage(reduce)")
+        cabi.check(cabi.reduce_stage(lib, ln.shape_ref, ln.mask_ptr, ws.data_ptr(), sums.data_ptr(), stream,
+                                     peer.handle if peer is not None else None), "mafed_distill_scalar_stage(reduce)")
     return sums
 
 

@@ -140,6 +140,10 @@ class FeatureDistillation(CLStrategy):
         # taken): the layers after it, the final layer norm and the LM head compute nothing the step reads.  Eager only:
         # under torch.compile the forwards run in full (see _stop_early)
         self.early_exit = bool(kwargs.get("early_exit", False))
+        # `adaptive` weights of a batch-sharded run: compute the importances over the union of the ranks' task loaders,
+        # the same on every rank (one exchange per task), instead of each rank's own shard.  Off by default: each rank
+        # then keeps its own importances, as naive DDP over the reference does
+        self.global_importances = bool(kwargs.get("global_importances", False))
         self._mem_iter = self._mem_iter_source = None
         self._mem_epoch = 0
         self._plan_cache = None
@@ -152,8 +156,29 @@ class FeatureDistillation(CLStrategy):
     def update(self, dataset, model, dataloader, mask=None, **kwargs):
         self._update_model(model)
         self._update_memory(dataset)
-        self.loss_weights.update_weights(model, dataloader, self.task_id)
+        if self.global_importances:
+            self.loss_weights.update_weights(model, dataloader, self.task_id, process_group=self.process_group)
+            self.check_importances()
+        else:
+            self.loss_weights.update_weights(model, dataloader, self.task_id)
         self.task_id += 1
+
+    def check_importances(self):
+        """``global_importances``: raise unless every rank of the group holds rank 0's ``adaptive`` language weights
+        (compared bit for bit, one all-gather of the L-float host table).  Ranks whose kernels read different weights
+        would each compute a different "global" loss, and DDP would average gradients of no single computation."""
+        distributed, pg = resolve_group(self.process_group)
+        if not distributed or self.loss_weights._modality_weighing_strategy != "adaptive":
+            return
+        dist = torch.distributed
+        bits = torch.tensor(self.loss_weights._adaptive_host_table(), dtype=torch.float32).view(torch.int32).tolist()
+        every = [None] * dist.get_world_size(pg)
+        dist.all_gather_object(every, bits, group=pg)
+        differ = [r if pg is None else dist.get_global_rank(pg, r) for r, b in enumerate(every) if b != every[0]]
+        if differ:
+            raise cabi.MafedDistillError(
+                f"the adaptive language weights of rank(s) {differ} differ from rank 0's after the importance exchange: "
+                "every rank must compute them over the same process group")
 
     def compute_loss(self, model, loss, batch, **kwargs):
         return loss

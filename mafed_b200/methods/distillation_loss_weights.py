@@ -138,28 +138,48 @@ class DistillationWeights:
         return self._lang_coeff_host
 
     # ------------------------------------------------------------------ adaptive importances
-    def update_weights(self, model, dataloader, task_id):
-        """Running average over tasks of the gradient-based language importance (reference :62-69)."""
+    def update_weights(self, model, dataloader, task_id, process_group=False):
+        """Running average over tasks of the gradient-based language importance (reference :62-69).
+        ``process_group``: see ``gradient_norm_sums``."""
         if self._modality_weighing_strategy != "adaptive":
             return
-        fresh = self.compute_adaptive_weights(model, dataloader)
+        fresh = self.compute_adaptive_weights(model, dataloader, process_group=process_group)
         if task_id < 1:
             self.lang_coeff = fresh
         else:
             self.lang_coeff = (fresh + task_id * self.lang_coeff) / (task_id + 1)
         self._lang_coeff_host = None
 
-    def compute_adaptive_weights(self, model, dataloader):
+    def compute_adaptive_weights(self, model, dataloader, process_group=False):
         """Per-layer share of the LM-loss gradient norm that falls on text tokens (reference :91-146).
 
         For every batch: gradient of the LM loss w.r.t. each selected hidden state, per-token L2
         norm, masked sums per modality; finally ``lang / (lang + image)`` of the per-token means.
+        ``process_group``: see ``gradient_norm_sums``.
         """
-        from mafed_b200.distill_op import modality_masks as device_masks, token_norm_sums
+        L = len(self.get_distillation_layers())
+        running = self.gradient_norm_sums(model, dataloader, process_group=process_group)
+        sums = running[: 2 * L].reshape(L, 2)
+        lang_imp = (sums[:, 0] / running[2 * L]).float()
+        image_imp = (sums[:, 1] / running[2 * L + 1]).float()
+        return lang_imp / (lang_imp + image_imp)
+
+    def gradient_norm_sums(self, model, dataloader, process_group=False):
+        """The totals behind ``compute_adaptive_weights``: device fp64 ``[2L + 2]``, per selected layer the sums of the
+        per-token L2 norms of the LM-loss gradient over text and over vision tokens, then the two token counts, added
+        over the batches of ``dataloader``.
+
+        ``process_group``: ``False`` (the default) keeps them this process's own.  Otherwise (``None``: the default
+        group, when one is initialised with more than one rank) the ranks' loaders are taken as the shards of one
+        dataset: each rank adds its own batches, then the totals are exchanged once (an fp64 SUM-allreduce, the same
+        on every rank), so every rank gets those of the union of the shards.  Every rank of the group must make the
+        call (the exchange is a collective).  A ``DistributedSampler`` pads the last shard with repeated samples: the totals are then those of the
+        padded union, which is what the ranks' loaders yield.
+        """
+        from mafed_b200.distill_op import allreduce_sums, modality_masks as device_masks, resolve_group, token_norm_sums
 
         model.eval()
         layers = self.get_distillation_layers()
-        L = len(layers)
         n_vis = self.num_vision_tokens
         running = None  # device fp64 [2L + 2]: per layer (text, vision) norm sums, then token counts
         for batch in dataloader:
@@ -174,11 +194,12 @@ class DistillationWeights:
             # one fused pass over all L gradients instead of L x (norm, 2 masked sums)
             now = token_norm_sums(grads, attn, n_vis)
             running = now if running is None else running + now
-        sums = running[: 2 * L].reshape(L, 2)
-        lang_imp = (sums[:, 0] / running[2 * L]).float()
-        image_imp = (sums[:, 1] / running[2 * L + 1]).float()
         model.zero_grad()
-        return lang_imp / (lang_imp + image_imp)
+        # the pass is additive over batches: one exchange of the totals, not one per batch
+        distributed, pg = resolve_group(process_group)
+        if distributed:
+            allreduce_sums(running, pg)
+        return running
 
 
 def modality_masks(attention_mask: torch.Tensor, num_vision_tokens: int):

@@ -12,6 +12,10 @@ kernels); every rank's loss and gradient slice must equal the same step run on o
 
 ``--mixed-layers``: instead, layers of several dtypes in one step (a bf16 model's states next to its fp32 final-layer-norm
 entry, one launch and one exchange per dtype group), with and without token counts sent ahead; compared the same way.
+
+``--adaptive``: instead, the ``adaptive`` importances computed over the ranks' shards of a task loader
+(``FeatureDistillation(global_importances=True)``) on the tiny VL model, against one GPU over all the batches, and the
+sharded ``replay()`` step that follows; and ``token_norm_sums(..., group=None)`` on a batch shard.
 """
 import argparse
 import os
@@ -31,6 +35,8 @@ def main():
                     help="fp32 students against a teacher in this dtype (default: today's same-dtype cases)")
     ap.add_argument("--mixed-layers", action="store_true",
                     help="layers of several dtypes in one step, one launch per dtype group")
+    ap.add_argument("--adaptive", action="store_true",
+                    help="adaptive importances over the ranks' loader shards, then a sharded replay() step")
     args = ap.parse_args()
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
@@ -41,6 +47,9 @@ def main():
         finish(ok)
     if args.mixed_layers:
         finish(mixed_layers_check(rank, world))
+    if args.adaptive:
+        ok = shard_norm_sums_check(rank, world)
+        finish(adaptive_check(rank, world) and ok)
     from gpu_util import Out, make_method, rel_err
     from golden_util import oracle_cfg
     from oracle import distill_oracle as O
@@ -195,6 +204,153 @@ def mixed_layers_check(rank, world):
               f"{'OK' if good else 'FAIL'}", flush=True)
     if peer is not None:
         ok &= peer.status() == 0
+    return ok
+
+
+def _max_rel(a, b):
+    a, b = a.double().cpu(), b.double().cpu()
+    return float(((a - b).abs() / b.abs().clamp_min(1e-300)).max())
+
+
+def _all_equal(t):
+    """True when ``t`` holds the same bits on every rank."""
+    every = [torch.empty_like(t) for _ in range(dist.get_world_size())]
+    dist.all_gather(every, t.contiguous())
+    return all(torch.equal(e, every[0]) for e in every)
+
+
+def shard_norm_sums_check(rank, world):
+    """``token_norm_sums(..., group=None)`` on uneven ragged batch shards, one dtype (with a communicator: the exchange
+    inside the reduce launch) and bf16 x 3 + fp32 (one pass per dtype, one allreduce of the assembled vector): the same
+    bits on every rank, equal to the ranks' own vectors added in rank order to 1e-12, and to one GPU's pass over the
+    whole batch to 1e-6 (its per-CTA fp32 partials group the tokens differently)."""
+    from mafed_b200.comm import get_peer_comm
+    from mafed_b200.distill_op import token_norm_sums
+    mode = "nccl" if get_peer_comm(None) is None else "peer-memory"
+    g = torch.Generator().manual_seed(71)
+    B, n_vis, txt, D = 3 * world + 1, 256, 9, 768
+    full = [torch.randn(B, n_vis + txt, D, generator=g) * (0.5 + l) for l in range(4)]
+    am = torch.ones(B, txt, dtype=torch.int64)
+    for b in range(B):
+        am[b, : (2 * b) % txt] = 0
+    lo = 3 * rank
+    hi = B if rank == world - 1 else lo + 3
+    ok = True
+    for name, dtypes in (("fp32", [torch.float32] * 4), ("bf16 x 3 + fp32", [torch.bfloat16] * 3 + [torch.float32])):
+        shard = [t[lo:hi].to(d).cuda().contiguous() for t, d in zip(full, dtypes)]
+        mask = am[lo:hi].cuda().contiguous()
+        mine = token_norm_sums(shard, mask, n_vis)
+        every = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(every, mine)
+        in_order = every[0].clone()
+        for e in every[1:]:
+            in_order = in_order + e
+        glob = token_norm_sums(shard, mask, n_vis, group=None)
+        one = token_norm_sums([t.to(d).cuda().contiguous() for t, d in zip(full, dtypes)], am.cuda(), n_vis)
+        torch.cuda.synchronize()
+        same, e_ranks, e_one = _all_equal(glob), _max_rel(glob, in_order), _max_rel(glob, one)
+        good = same and e_ranks < 1e-12 and e_one < 1e-6
+        ok &= good
+        print(f"rank {rank}/{world} ({mode}) token_norm_sums on a shard, {name}: same on all ranks {same}, "
+              f"vs ranks' vectors {e_ranks:.1e}, vs one GPU {e_one:.1e} {'OK' if good else 'FAIL'}", flush=True)
+    return ok
+
+
+def adaptive_check(rank, world):
+    """``adaptive`` importances of a batch-sharded run (``FeatureDistillation(global_importances=True)``), the tiny VL
+    model, every rank on its shard of a seeded task loader of uneven length (``update()``, then a second task):
+    (a) ``lang_coeff`` is bit-identical on every rank; (b) the exchanged fp64 totals, and the importances formed from them
+    in fp64, equal one GPU's pass over all the batches to 1e-12 (only the order of the additions over batches differs),
+    and ``lang_coeff`` (the fp32 running average over the tasks) equals that GPU's to 1e-6; (c) the sharded ``replay()`` step that follows (no replay
+    loss, so the loss is the global one) gives the same loss on every rank, and parameter gradients summed over the
+    ranks equal the one-GPU step on the concatenated memory batch within the fp32 tolerance (1e-5).  The model runs in
+    fp32 (``fp32_island``): under bf16 autocast the ranks' weight gradients come out of bf16 products, and their sum
+    differed from the full-batch product by 2.4e-3 here, with the loss bit-identical."""
+    import copy
+
+    from gpu_util import rel_err
+    from mafed_b200.comm import get_peer_comm
+    from mafed_b200.methods import CLMethod, DistillationWeights
+    from tiny_vl import TinyVL, make_batch
+    mode = "nccl" if get_peer_comm(None) is None else "peer-memory"
+    n_vis, L = 8, 3
+
+    class Opts:
+        tasks = ["a", "b", "c"]; batch_size = 4; seed = 1; pin_mem = False; accumulate_grad_batches = 1
+
+    def strategy(group, global_importances):
+        fd = CLMethod["featdistill"](memory_size=8, opts=Opts(), model_type="vlpythia",
+                                     distillation_modality_weighing_strategy="adaptive",
+                                     distillation_layer_weighing_strategy="discounted", distillation_layer=None,
+                                     num_hidden_layers=L, gamma=0.5, replay_coeff=0.0, distillation_coeff=2.0,
+                                     process_group=group, grad_multiplier=1.0, global_importances=global_importances)
+        fd.num_vision_tokens = fd.loss_weights.num_vision_tokens = n_vis
+        fd.data_hooks = (None, lambda loader: loader)
+        return fd
+
+    def ratio64(t):
+        lang, image = t[0:2 * L:2] / t[2 * L], t[1:2 * L:2] / t[2 * L + 1]
+        return lang / (lang + image)
+
+    torch.manual_seed(0)
+    model = TinyVL(n_vis=n_vis, fp32_island=True).cuda()
+    model.gpt_neox.config._attn_implementation = "eager"    # SDPA's memory-efficient backward adds with atomics
+    tasks = [[make_batch(bsz=3 + i % 3, seed=100 * t + i, device="cuda") for i in range(2 * world + 1)] for t in (1, 2)]
+    fd = strategy(None, True)
+    one = DistillationWeights("adaptive", "discounted", num_hidden_layers=L, distillation_layer=None,
+                              num_vision_tokens=n_vis)
+    ok = True
+    for k, batches in enumerate(tasks):
+        fd.update(list(range(16)), model, [dict(b) for b in batches[rank::world]])
+        glob = fd.loss_weights.gradient_norm_sums(model, [dict(b) for b in batches[rank::world]], process_group=None)
+        tot1 = one.gradient_norm_sums(model, [dict(b) for b in batches])
+        one.update_weights(model, [dict(b) for b in batches], k)
+        torch.cuda.synchronize()
+        coeff = fd.loss_weights.lang_coeff
+        same = _all_equal(coeff) and _all_equal(glob)
+        e_tot, e_imp = _max_rel(glob, tot1), _max_rel(ratio64(glob), ratio64(tot1))
+        e_coeff = _max_rel(coeff, one.lang_coeff)
+        good = same and e_tot < 1e-12 and e_imp < 1e-12 and e_coeff < 1e-6
+        ok &= good
+        print(f"rank {rank}/{world} ({mode}) adaptive importances, task {k}: lang_coeff {coeff.tolist()} "
+              f"same on all ranks {same}; vs one GPU: totals {e_tot:.1e}, fp64 importances {e_imp:.1e}, "
+              f"lang_coeff {e_coeff:.1e} {'OK' if good else 'FAIL'}", flush=True)
+
+    # the sharded replay() step against one GPU on the concatenated memory batch, with these weights
+    torch.manual_seed(1)
+    with torch.no_grad():
+        for p in model.parameters():
+            p.add_(0.02 * torch.randn_like(p))                       # the student has moved away from the teacher
+    single = copy.deepcopy(model)
+    mem = make_batch(bsz=2 * world + 1, seed=300, device="cuda")
+    lo = 2 * rank
+    hi = mem["input_ids"].shape[0] if rank == world - 1 else lo + 2
+    fd.mem_dataloader = [{k: v[lo:hi].contiguous() for k, v in mem.items()}]
+    loss, n_ex = fd.replay(model)
+    loss.backward()
+    grads = [p.grad if p.grad is not None else torch.zeros_like(p) for p in model.parameters()]
+    for g in grads:
+        dist.all_reduce(g)
+    ref = strategy(False, False)
+    ref.past_model, ref.task_id = fd.past_model, fd.task_id
+    ref.loss_weights.lang_coeff = fd.loss_weights.lang_coeff.clone()
+    ref.mem_dataloader = [dict(mem)]
+    loss1, _ = ref.replay(single)
+    loss1.backward()
+    want = [p.grad if p.grad is not None else torch.zeros_like(p) for p in single.parameters()]
+    torch.cuda.synchronize()
+    same = _all_equal(loss.detach().reshape(1))
+    e_loss = abs(float(loss) - float(loss1)) / abs(float(loss1))
+    e_grad = max(rel_err(a.cpu(), b.cpu()) for a, b in zip(grads, want) if b.abs().sum() > 0)
+    good = same and n_ex == hi - lo and e_loss < 1e-5 and e_grad < 1e-5
+    ok &= good
+    print(f"rank {rank}/{world} ({mode}) sharded replay() with the global importances: loss same on all ranks {same}, "
+          f"vs one GPU: loss {e_loss:.1e} parameter gradients {e_grad:.1e} {'OK' if good else 'FAIL'}", flush=True)
+    peer = get_peer_comm(None)
+    if peer is not None:
+        ok &= peer.status() == 0
+    if os.environ.get("MAFED_B200_DIST", "peer") == "peer":
+        ok &= peer is not None
     return ok
 
 
