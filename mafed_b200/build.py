@@ -4,6 +4,9 @@
   units: ``distill_abi.cu`` (whole-program compiled: every ordinary launch) and ``distill_gate.cu`` (relocatable
   device code, device-linked with cudadevrt: the gated backward whose 1-CTA gate starts the real kernel from the
   device).  No torch anywhere in it.
+* ``_lib/libmafed_teacher_gather.so`` -- the teacher-cache gather kernel (``csrc/teacher_gather.cu``) behind its own
+  C ABI (``include/mafed_teacher_gather.h``), bound by ``mafed_b200.teacher_cache``.  A unit of its own, so the
+  distillation library and its export list stay as they are.
 * ``_lib/mafed_torch_node*.so`` -- the torch extension (``csrc/torch_node.cpp``, host C++ only): the autograd node
   that turns one ``distill()`` into one call of the C ABI without Python on the hot path.
 """
@@ -24,6 +27,11 @@ HEADERS = [os.path.join(CSRC, n) for n in
            ("distill_common.cuh", "distill_ldg.cuh", "distill_tma.cuh", "distill_epilogue.cuh",
             "distill_comm.cuh", "distill_host.cuh", "distill_dispatch.cuh", "distill_gate.h")] + \
           [os.path.join(ROOT, "include", "mafed_distill.h")]
+
+GATHER_SOURCE = os.path.join(CSRC, "teacher_gather.cu")
+GATHER_HEADER = os.path.join(ROOT, "include", "mafed_teacher_gather.h")
+GATHER_LIB_PATH = os.path.join(LIB_DIR, "libmafed_teacher_gather.so")
+GATHER_STAMP_PATH = os.path.join(LIB_DIR, "gather.stamp")
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", *ARCH, "-lineinfo", "-Xcompiler", "-fPIC"]
@@ -96,6 +104,20 @@ def build(force=False, verbose=False):
     return LIB_PATH
 
 
+def build_teacher_gather(force=False, verbose=False):
+    """Compile libmafed_teacher_gather.so for sm_100a if missing or older than its source."""
+    fp = _fingerprint([GATHER_SOURCE, GATHER_HEADER], NVCC_FLAGS)
+    if not force and not _stale(GATHER_LIB_PATH, GATHER_STAMP_PATH, fp):
+        return GATHER_LIB_PATH
+    os.makedirs(LIB_DIR, exist_ok=True)
+    extra = ["-Xptxas=-v"] if verbose else []
+    _run([[_nvcc(), *NVCC_FLAGS, *extra, "-I", os.path.join(ROOT, "include"), "-shared", GATHER_SOURCE,
+           "-o", GATHER_LIB_PATH]], verbose)
+    with open(GATHER_STAMP_PATH, "w") as f:
+        f.write(fp)
+    return GATHER_LIB_PATH
+
+
 def build_torch_ext(force=False, verbose=False):
     """Compile the torch extension (host C++ against the torch headers; it dlopens libmafed_distill.so)."""
     from torch.utils import cpp_extension as ce
@@ -124,5 +146,6 @@ if __name__ == "__main__":
     import sys
     force, verbose = "--force" in sys.argv, "-v" in sys.argv
     print(build(force=force, verbose=verbose))
+    print(build_teacher_gather(force=force, verbose=verbose))
     if "--no-ext" not in sys.argv:
         print(build_torch_ext(force=force, verbose=verbose))

@@ -54,7 +54,11 @@ class _CapturedOutput:
 
 
 class FeatureDistillation(CLStrategy):
-    """Feature distillation with separate vision / language weights (MAFED)."""
+    """Feature distillation with separate vision / language weights (MAFED).
+
+    ``teacher_cache=True`` computes the teacher's distilled hidden states of the whole episodic memory once per task
+    (in ``update()``) and gathers each replay step's rows from them instead of running the teacher (INTEGRATION.md:
+    the text rows' targets change).  Under ``torch.compile`` the option does not apply: the teacher forward runs."""
 
     def __init__(
         self,
@@ -144,6 +148,11 @@ class FeatureDistillation(CLStrategy):
         # the same on every rank (one exchange per task), instead of each rank's own shard.  Off by default: each rank
         # then keeps its own importances, as naive DDP over the reference does
         self.global_importances = bool(kwargs.get("global_importances", False))
+        # serve replay steps' teacher states from a per-task cache of the episodic memory (mafed_b200.teacher_cache)
+        # instead of a teacher forward: built in update(), gathered by one kernel per step.  Eager only, as early_exit
+        self.teacher_cache = bool(kwargs.get("teacher_cache", False))
+        self._teacher_cache = None          # the TeacherCache of the current task (None: built on the next replay)
+        self._memory_index = None           # memory indices of the batch replay() drew, for _past_states
         self._mem_iter = self._mem_iter_source = None
         self._mem_epoch = 0
         self._plan_cache = None
@@ -156,6 +165,8 @@ class FeatureDistillation(CLStrategy):
     def update(self, dataset, model, dataloader, mask=None, **kwargs):
         self._update_model(model)
         self._update_memory(dataset)
+        if self.teacher_cache:
+            self._build_teacher_cache()
         if self.global_importances:
             self.loss_weights.update_weights(model, dataloader, self.task_id, process_group=self.process_group)
             self.check_importances()
@@ -203,6 +214,8 @@ class FeatureDistillation(CLStrategy):
         """Memory batch -> student forward (hidden states kept) -> replay LM loss + distillation loss.
         Returns ``(loss, n_examples)`` like ``distillation.py:84-103``."""
         batch = self._next_memory_batch()
+        if self.teacher_cache:
+            self._memory_index = batch.pop("memory_index", None)
         n_ex = batch["input_ids"].size(0)
         do_replay = self.replay_coeff > 0 and self.task_id > 0
         loss = None
@@ -435,6 +448,9 @@ class FeatureDistillation(CLStrategy):
     def _past_states(self, batch, layers):
         """Teacher hidden states of the distilled layers only (same forward and side effects as
         ``_get_past_hidden_states``; with ``early_exit`` the forward stops after the last of them)."""
+        if self.teacher_cache and not torch.compiler.is_compiling():
+            batch.pop("labels", None)
+            return self._cached_past_states(batch, layers)
         stop = self._stop_early()
         with torch.no_grad(), self._teacher_forward(batch):
             batch.pop("labels", None)
@@ -447,6 +463,25 @@ class FeatureDistillation(CLStrategy):
         # no per-tensor `.detach()` (distillation.py:223): these come out of a no_grad forward, and the node never builds
         # a graph edge to a teacher tensor whatever its flags are
         return [self._as_teacher_dtype(states[l]) for l in layers]
+
+    def _cached_past_states(self, batch, layers):
+        """``teacher_cache``: the distilled layers' teacher states of the batch ``replay()`` drew, gathered from the cache
+        (built here if ``load_state_dict`` left none) -- no teacher forward."""
+        idx, self._memory_index = self._memory_index, None
+        if idx is None:
+            raise cabi.MafedDistillError(
+                "teacher_cache: the batch has no memory_index (replay() takes it from the memory loader, which yields it "
+                "with teacher_cache=True)")
+        if self._teacher_cache is None:
+            if self.past_model is None:
+                raise cabi.MafedDistillError("teacher_cache: there is no teacher (past_model) to build the cache from")
+            self._build_teacher_cache()
+        return self._teacher_cache.gather(idx, batch["attention_mask"].shape[1] + self.num_vision_tokens, layers)
+
+    def _build_teacher_cache(self):
+        from mafed_b200 import teacher_cache
+        self._teacher_cache = None              # the previous task's cache goes before the new one is allocated
+        self._teacher_cache = teacher_cache.build(self)
 
     def _get_past_hidden_states(self, batch):
         with torch.no_grad(), self._teacher_forward(batch):
@@ -577,6 +612,7 @@ class FeatureDistillation(CLStrategy):
             self.loss_weights.lang_coeff = coeff
             self.loss_weights._lang_coeff_host = None
         self._plan_cache = None
+        self._teacher_cache = None      # not saved: rebuilt on the first replay, from the restored memory and teacher
         if datasets is not None:
             from torch.utils.data import Subset
             self.datasets = [Subset(ds, idx) for ds, idx in zip(datasets, state["memory_indices"])]
@@ -614,7 +650,12 @@ class FeatureDistillation(CLStrategy):
         distributed = dist.is_available() and dist.is_initialized()
         sampler = DistributedSampler(memory) if distributed else RandomSampler(memory)
         collate, prefetch = self._data_hooks()
-        loader = DataLoader(memory, sampler=sampler, num_workers=self.num_workers, batch_size=self.batch_size,
+        data = memory
+        if self.teacher_cache:
+            # each batch also carries its samples' memory indices (a host list), which select their cached teacher rows
+            from mafed_b200.teacher_cache import IndexedCollate, IndexedDataset
+            data, collate = IndexedDataset(memory), IndexedCollate(collate)
+        loader = DataLoader(data, sampler=sampler, num_workers=self.num_workers, batch_size=self.batch_size,
                             collate_fn=collate)
         self.mem_dataloader = prefetch(loader)
         self.mem_sampler = sampler

@@ -37,6 +37,8 @@ def main():
                     help="layers of several dtypes in one step, one launch per dtype group")
     ap.add_argument("--adaptive", action="store_true",
                     help="adaptive importances over the ranks' loader shards, then a sharded replay() step")
+    ap.add_argument("--teacher-cache", action="store_true",
+                    help="replay() steps with teacher_cache=True, sharded, against one GPU on the concatenated batch")
     args = ap.parse_args()
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
@@ -47,6 +49,8 @@ def main():
         finish(ok)
     if args.mixed_layers:
         finish(mixed_layers_check(rank, world))
+    if args.teacher_cache:
+        finish(teacher_cache_check(rank, world))
     if args.adaptive:
         ok = shard_norm_sums_check(rank, world)
         finish(adaptive_check(rank, world) and ok)
@@ -205,6 +209,78 @@ def mixed_layers_check(rank, world):
     if peer is not None:
         ok &= peer.status() == 0
     return ok
+
+
+def teacher_cache_check(rank, world):
+    """``teacher_cache=True`` on a batch-sharded run: every rank builds the same cache over the whole memory, with no
+    exchange, and a sharded cached ``replay()`` step without a replay loss (its loss is the global-batch distillation
+    loss) equals one GPU's cached step on the concatenated batch: loss to 1e-5, the ranks' summed parameter gradients to
+    1e-4 (fp32 model: the sums run in another order).  The shards are padded to the global batch's text length, so the
+    student sees the same tokens as in the one-GPU batch."""
+    import copy
+    from torch.utils.data import ConcatDataset
+    from gpu_util import rel_err
+    from mafed_b200.methods import CLMethod
+    from mafed_b200.teacher_cache import repad_left
+    from tiny_vl import TinyVL
+    from vl_memory import VLSamples, collate
+
+    class Opts:
+        tasks = ["a", "b"]; batch_size = 4; seed = 1; pin_mem = False; accumulate_grad_batches = 1
+
+    torch.manual_seed(0)
+    teacher = TinyVL(fp32_island=True).cuda()
+    student = copy.deepcopy(teacher)
+    with torch.no_grad():
+        for p in student.parameters():
+            p.add_(0.02 * torch.randn_like(p))
+
+    def strategy(group):
+        fd = CLMethod["featdistill"](memory_size=32, opts=Opts(), model_type="vlpythia",
+                                     distillation_modality_weighing_strategy="balanced",
+                                     distillation_layer_weighing_strategy="discounted", distillation_layer=None,
+                                     num_hidden_layers=3, replay_coeff=0.0, teacher_cache=True, process_group=group,
+                                     grad_multiplier=1.0)
+        fd.num_vision_tokens, fd.num_workers = 8, 0
+        fd.data_hooks = (collate, lambda loader: loader)
+        fd.update(dataset=VLSamples(64, seed=3, max_txt=9), model=teacher, dataloader=None)
+        return fd
+
+    def step(fd, idx, text_len):
+        memory = ConcatDataset(fd.datasets)
+        batch = repad_left(collate([memory[i] for i in idx]), text_len)
+        batch.pop("labels")
+        batch = {k: v.cuda() if torch.is_tensor(v) else v for k, v in batch.items()}
+        batch["memory_index"] = list(idx)
+        fd.mem_dataloader = [batch]
+        model = copy.deepcopy(student)
+        loss, n_ex = fd.replay(model)
+        loss.backward()
+        torch.cuda.synchronize()
+        return loss.detach(), n_ex, [p.grad for p in model.parameters()]
+
+    sharded, full = strategy(None), strategy(False)
+    same_cache = all(_all_equal(s) for s in sharded._teacher_cache.states)
+    B = 4 * world + 2
+    idx = [(5 * i) % 32 for i in range(B)]
+    memory = ConcatDataset(full.datasets)
+    text_len = max(len(memory[i]["input_ids"]) for i in idx)
+    lo = rank * 4
+    hi = B if rank == world - 1 else lo + 4
+    loss_s, n_s, g_s = step(sharded, idx[lo:hi], text_len)
+    loss_f, n_f, g_f = step(full, idx, text_len)
+    e_loss = abs(float(loss_s) - float(loss_f)) / abs(float(loss_f))
+    e_grad = 0.0
+    for a, b in zip(g_s, g_f):
+        if b is None:
+            e_grad = e_grad if a is None else float("inf")
+            continue
+        dist.all_reduce(a)
+        e_grad = max(e_grad, rel_err(a, b))
+    good = same_cache and n_s == hi - lo and n_f == B and e_loss < 1e-5 and e_grad < 1e-4
+    print(f"rank {rank}/{world} teacher cache: caches equal on every rank {same_cache}, loss err {e_loss:.2e}, "
+          f"summed gradient err {e_grad:.2e} {'OK' if good else 'FAIL'}", flush=True)
+    return good
 
 
 def _max_rel(a, b):
