@@ -58,7 +58,10 @@ class FeatureDistillation(CLStrategy):
 
     ``teacher_cache=True`` computes the teacher's distilled hidden states of the whole episodic memory once per task
     (in ``update()``) and gathers each replay step's rows from them instead of running the teacher (INTEGRATION.md:
-    the text rows' targets change).  Under ``torch.compile`` the option does not apply: the teacher forward runs."""
+    the text rows' targets change).  Under ``torch.compile`` the option does not apply: the teacher forward runs.
+    ``shard_teacher_cache=True`` on top of it splits the cache across the ranks of the process group (one process per
+    GPU of one host): each rank builds and holds its share, and a step gathers each sample's rows from whichever GPU
+    holds them, with the same numbers as the replicated cache."""
 
     def __init__(
         self,
@@ -151,7 +154,13 @@ class FeatureDistillation(CLStrategy):
         # serve replay steps' teacher states from a per-task cache of the episodic memory (mafed_b200.teacher_cache)
         # instead of a teacher forward: built in update(), gathered by one kernel per step.  Eager only, as early_exit
         self.teacher_cache = bool(kwargs.get("teacher_cache", False))
+        # split the cache across the ranks of the process group (teacher_cache.build_sharded) instead of a whole copy
+        # per rank: HBM held for the task traded against NVLink reads per step.  On one rank the cache is replicated
+        self.shard_teacher_cache = bool(kwargs.get("shard_teacher_cache", False))
+        if self.shard_teacher_cache and not self.teacher_cache:
+            raise ValueError("shard_teacher_cache=True needs teacher_cache=True")
         self._teacher_cache = None          # the TeacherCache of the current task (None: built on the next replay)
+        self._retired_cache = None          # a sharded cache load_state_dict dropped: released by the next build
         self._memory_index = None           # memory indices of the batch replay() drew, for _past_states
         self._mem_iter = self._mem_iter_source = None
         self._mem_epoch = 0
@@ -480,8 +489,23 @@ class FeatureDistillation(CLStrategy):
 
     def _build_teacher_cache(self):
         from mafed_b200 import teacher_cache
+        if self.shard_teacher_cache:
+            self._build_sharded_teacher_cache()
+            return
         self._teacher_cache = None              # the previous task's cache goes before the new one is allocated
         self._teacher_cache = teacher_cache.build(self)
+
+    def _build_sharded_teacher_cache(self):
+        """``shard_teacher_cache``: release the previous shards (collective: a peer's gather may still read this rank's
+        shard until every rank has synchronised), then build this task's across the group, or the replicated cache
+        when there is no group to shard over."""
+        from mafed_b200 import teacher_cache
+        old, self._teacher_cache, self._retired_cache = self._teacher_cache or self._retired_cache, None, None
+        if isinstance(old, teacher_cache.ShardedTeacherCache):
+            old.release()
+        del old
+        distributed, group = resolve_group(self.process_group)
+        self._teacher_cache = teacher_cache.build_sharded(self, group) if distributed else teacher_cache.build(self)
 
     def _get_past_hidden_states(self, batch):
         with torch.no_grad(), self._teacher_forward(batch):
@@ -612,6 +636,8 @@ class FeatureDistillation(CLStrategy):
             self.loss_weights.lang_coeff = coeff
             self.loss_weights._lang_coeff_host = None
         self._plan_cache = None
+        if self.shard_teacher_cache:     # its shards are released collectively, by the rebuild
+            self._retired_cache = self._teacher_cache or self._retired_cache
         self._teacher_cache = None      # not saved: rebuilt on the first replay, from the restored memory and teacher
         if datasets is not None:
             from torch.utils.data import Subset

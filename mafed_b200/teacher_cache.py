@@ -10,6 +10,12 @@ Layout: ``T_c = n_vis + the longest text of the memory set``; every sample is co
 that length, as the collate pads a batch.  A batch at length ``T <= T_c`` takes the visual rows ``t < n_vis`` from the
 start of its samples' cache rows and the text rows from their right-aligned end.
 
+Sharded (``shard_teacher_cache=True``, one process per GPU of one box): ``build_sharded`` runs only this rank's share of
+the same build batches into one device buffer per rank (``ShardedTeacherCache``), maps every peer's buffer through CUDA
+IPC, and a step's gather reads each sample's rows from whichever GPU holds them, in the same single launch per dtype.
+Build batch ``k`` (the ``k``-th batch of ``batch_size`` samples of the memory, in order) belongs to rank ``k % N``
+(``shard_owners``), so every row is computed by the same batch as in ``build`` and is bit for bit the replicated row.
+
 Sample identity: the memory loader yields ``batch["memory_index"]``, a Python list of the samples' indices into the
 memory ``ConcatDataset`` (``IndexedDataset`` + ``IndexedCollate``); a list is left on the host by the prefetch loader,
 so a step never reads a device tensor back.
@@ -19,8 +25,9 @@ from __future__ import annotations
 import ctypes
 import logging
 import os
+import socket
 import threading
-from typing import Dict, List, Sequence
+from typing import Dict, List, Sequence, Tuple
 
 import torch
 
@@ -28,7 +35,9 @@ from mafed_b200.cabi import MafedDistillError
 
 _log = logging.getLogger(__name__)
 
-ABI_VERSION = 1
+ABI_VERSION = 2
+MAX_RANKS = 16
+_ALIGN = 256                    # byte alignment of each layer's block in a shard
 _DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib", "libmafed_teacher_gather.so")
 
@@ -55,10 +64,29 @@ def load():
             lib.mafed_teacher_gather.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p),
                                                  ctypes.POINTER(ctypes.c_int64), i32, i32, ctypes.c_int64, i32, i32,
                                                  i32, i32, i32, ctypes.c_void_p]
+            vp, i64 = ctypes.c_void_p, ctypes.c_int64
+            lib.mafed_teacher_gather_sharded.restype = i32
+            lib.mafed_teacher_gather_sharded.argtypes = [ctypes.POINTER(vp), ctypes.POINTER(vp), i32,
+                                                         ctypes.POINTER(i64), ctypes.POINTER(ctypes.c_int32),
+                                                         ctypes.POINTER(i64), i32, i32, i64, i32, i32, i32, i32, i32, vp]
+            lib.mafed_teacher_shard_handle_bytes.restype = i32
+            lib.mafed_teacher_shard_create.restype = i32
+            lib.mafed_teacher_shard_create.argtypes = [i32, i32, i64, ctypes.c_char_p, ctypes.POINTER(vp)]
+            lib.mafed_teacher_shard_connect.restype = i32
+            lib.mafed_teacher_shard_connect.argtypes = [vp, ctypes.c_char_p]
+            lib.mafed_teacher_shard_base.restype = i32
+            lib.mafed_teacher_shard_base.argtypes = [vp, i32, ctypes.POINTER(vp)]
+            lib.mafed_teacher_shard_destroy.restype = i32
+            lib.mafed_teacher_shard_destroy.argtypes = [vp]
             if lib.mafed_teacher_gather_abi_version() != ABI_VERSION:
                 raise MafedDistillError("libmafed_teacher_gather.so ABI version mismatch; rebuild")
             _lib = lib
     return _lib
+
+
+def _check(rc, what):
+    if rc != 0:
+        raise MafedDistillError(f"{what} failed: {load().mafed_teacher_gather_error_string(rc).decode()} (code {rc})")
 
 
 def gather_raw(out_ptrs, cache_ptrs, idx, B, M, T, T_c, n_vis, D, dtype_code, stream):
@@ -68,9 +96,22 @@ def gather_raw(out_ptrs, cache_ptrs, idx, B, M, T, T_c, n_vis, D, dtype_code, st
     rc = lib.mafed_teacher_gather((ctypes.c_void_p * n)(*out_ptrs), (ctypes.c_void_p * len(cache_ptrs))(*cache_ptrs),
                                   (ctypes.c_int64 * len(idx))(*idx) if idx is not None else None, n, B, M, T, T_c,
                                   n_vis, D, dtype_code, stream)
-    if rc != 0:
-        raise MafedDistillError(f"mafed_teacher_gather failed: {lib.mafed_teacher_gather_error_string(rc).decode()} "
-                                f"(code {rc})")
+    _check(rc, "mafed_teacher_gather")
+
+
+def _array(ctype, values):
+    return (ctype * len(values))(*values) if values is not None else None
+
+
+def gather_sharded_raw(out_ptrs, bases, layer_off, src_rank, slot, B, slots, T, T_c, n_vis, D, dtype_code, stream):
+    """``mafed_teacher_gather_sharded`` as it is (plain ints and pointers; ``None`` passes NULL); raise
+    ``MafedDistillError`` on a non-zero code."""
+    lib = load()
+    rc = lib.mafed_teacher_gather_sharded(
+        _array(ctypes.c_void_p, out_ptrs), _array(ctypes.c_void_p, bases), len(bases) if bases is not None else 0,
+        _array(ctypes.c_int64, layer_off), _array(ctypes.c_int32, src_rank), _array(ctypes.c_int64, slot),
+        len(out_ptrs if out_ptrs is not None else layer_off), B, slots, T, T_c, n_vis, D, dtype_code, stream)
+    _check(rc, "mafed_teacher_gather_sharded")
 
 
 def gather(cache: Sequence[torch.Tensor], idx: Sequence[int], T: int, n_vis: int) -> List[torch.Tensor]:
@@ -165,36 +206,46 @@ class TeacherCache:
         return gather(self.states, idx, T, self.n_vis)
 
 
-def build(strategy) -> TeacherCache:
-    """Run ``strategy.past_model`` once over the whole episodic memory (``strategy.datasets``) and cache its distilled
-    hidden states, as ``replay()`` would hand them to the step: the same bf16 autocast region, ``teacher_dtype``
-    autocast and rounding, and a forward that stops after the last distilled entry."""
+def _build_batches(strategy):
+    """The build batches: the memory ``ConcatDataset`` in order, in batches of ``strategy.batch_size`` (host inputs,
+    each with its ``memory_index``), the longest text of the whole memory, and M."""
     from torch.utils.data import ConcatDataset, DataLoader
-
-    from mafed_b200.capture import HiddenStateCapture
 
     memory = ConcatDataset(strategy.datasets)
     collate, _ = strategy._data_hooks()
     loader = DataLoader(IndexedDataset(memory), batch_size=strategy.batch_size, shuffle=False, num_workers=0,
                         collate_fn=IndexedCollate(collate))
     batches = list(loader)                   # host inputs, kept: for ~500 samples a few hundred MB
+    return batches, max(b["input_ids"].shape[1] for b in batches), len(memory)
+
+
+def _teacher_states(strategy, batch, text_len, layers, device):
+    """One build batch through the teacher at ``text_len`` text tokens: ``(memory indices, [B, T_c, D] per layer)``."""
+    from mafed_b200.capture import HiddenStateCapture
+
+    model = strategy.past_model
+    idx = batch.pop("memory_index")
+    batch.pop("labels", None)
+    batch = {k: v.to(device, non_blocking=True) if torch.is_tensor(v) else v
+             for k, v in repad_left(batch, text_len).items()}
+    with torch.no_grad(), torch.autocast(device.type, dtype=torch.bfloat16), strategy._teacher_forward(batch):
+        with HiddenStateCapture(model, layers, detach=True, stop_after_last=True) as cap:
+            model(**batch, output_hidden_states=False, return_dict=True)
+    return idx, [strategy._as_teacher_dtype(cap.hidden_states[l]) for l in layers]
+
+
+def build(strategy) -> TeacherCache:
+    """Run ``strategy.past_model`` once over the whole episodic memory (``strategy.datasets``) and cache its distilled
+    hidden states, as ``replay()`` would hand them to the step: the same bf16 autocast region, ``teacher_dtype``
+    autocast and rounding, and a forward that stops after the last distilled entry."""
+    batches, text_len, M = _build_batches(strategy)
     n_vis = strategy.num_vision_tokens
-    text_len = max(b["input_ids"].shape[1] for b in batches)
     T_c = n_vis + text_len
     layers = strategy.loss_weights.get_distillation_layers()
-    model = strategy.past_model
-    device = next(model.parameters()).device
-    M = len(memory)
+    device = next(strategy.past_model.parameters()).device
     states = None
     for batch in batches:
-        idx = batch.pop("memory_index")
-        batch.pop("labels", None)
-        batch = {k: v.to(device, non_blocking=True) if torch.is_tensor(v) else v
-                 for k, v in repad_left(batch, text_len).items()}
-        with torch.no_grad(), torch.autocast(device.type, dtype=torch.bfloat16), strategy._teacher_forward(batch):
-            with HiddenStateCapture(model, layers, detach=True, stop_after_last=True) as cap:
-                model(**batch, output_hidden_states=False, return_dict=True)
-        hs = [strategy._as_teacher_dtype(cap.hidden_states[l]) for l in layers]
+        idx, hs = _teacher_states(strategy, batch, text_len, layers, device)
         if states is None:
             need = sum(M * T_c * h.shape[-1] * h.element_size() for h in hs)
             _log.info("teacher cache: %d samples x %d layers x T_c %d x D %d = %d bytes", M, len(layers), T_c,
@@ -209,3 +260,165 @@ def build(strategy) -> TeacherCache:
         for s, h in zip(states, hs):
             s.index_copy_(0, rows, h)
     return TeacherCache(layers, states, T_c, n_vis)
+
+
+# ---------------------------------------------------------------- the cache sharded across the ranks of one box
+def shard_owners(M: int, batch_size: int, world: int) -> Tuple[List[int], List[int], List[int]]:
+    """Where each memory sample lives in a sharded cache: ``(rank[i], slot[i], count[r])``.  Build batch
+    ``k = i // batch_size`` belongs to rank ``k % world``; a rank's batches fill its slots in order, so sample ``i``
+    takes slot ``(k // world) * batch_size + i % batch_size``.  A pure function of its arguments: every rank computes
+    it with no exchange.  A rank with no build batch (fewer batches than ranks) holds no sample."""
+    if M < 0 or batch_size < 1 or world < 1:
+        raise ValueError(f"shard_owners needs M >= 0, batch_size >= 1 and world >= 1, not {M}, {batch_size}, {world}")
+    rank = [(i // batch_size) % world for i in range(M)]
+    slot = [(i // batch_size // world) * batch_size + i % batch_size for i in range(M)]
+    count = [0] * world
+    for r in rank:
+        count[r] += 1
+    return rank, slot, count
+
+
+def shard_layout(capacity: int, T_c: int, D: int, element_sizes: Sequence[int]) -> Tuple[List[int], int]:
+    """Byte offset of each layer's ``[capacity, T_c, D]`` block in a shard (each 256-byte aligned) and the shard's
+    size.  The same on every rank: every rank allocates the largest share."""
+    offsets, at = [], 0
+    for e in element_sizes:
+        offsets.append(at)
+        at += -(-capacity * T_c * D * e // _ALIGN) * _ALIGN
+    return offsets, max(at, _ALIGN)
+
+
+class _DeviceMemory:
+    """A raw device range as a torch tensor (``__cuda_array_interface__``); the memory stays the shard's."""
+
+    def __init__(self, ptr: int, nbytes: int):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+
+class ShardedTeacherCache:
+    """This rank's share of the teacher cache, with every peer's share mapped (``build_sharded``).  Same surface as
+    ``TeacherCache``: ``layers``, ``T_c``, ``n_vis`` and ``gather``, which reads each sample's rows from the GPU that
+    holds them (one launch per dtype of the layers).  ``local_states[k]`` is ``[count, T_c, D]``: this rank's samples
+    (``owner``/``slot`` map memory indices to ranks and slots).  ``nbytes`` is this rank's shard.  ``release()`` is a
+    collective of the group the cache was built over."""
+
+    def __init__(self, layers, dtypes, T_c, n_vis, M, D, owner, slot, count, capacity, offsets, nbytes, handle, group,
+                 rank, device):
+        self.layers, self.dtypes, self.T_c, self.n_vis, self.M, self.D = list(layers), list(dtypes), T_c, n_vis, M, D
+        self.owner, self.slot, self.count, self.capacity = owner, slot, count, capacity
+        self.offsets, self.nbytes, self.group, self.rank, self.device = offsets, nbytes, group, rank, device
+        self._handle = handle
+        lib = load()
+        self.bases = []
+        for r in range(len(count)):
+            base = ctypes.c_void_p()
+            _check(lib.mafed_teacher_shard_base(handle, r, ctypes.byref(base)), "mafed_teacher_shard_base")
+            self.bases.append(base.value)
+        raw = torch.as_tensor(_DeviceMemory(self.bases[rank], nbytes), device=device)
+        self._slots = [raw[o:o + capacity * T_c * D * torch.empty((), dtype=d).element_size()].view(d)
+                       .view(capacity, T_c, D) for o, d in zip(offsets, self.dtypes)]
+        self.local_states = [s[: count[rank]] for s in self._slots]
+
+    def gather(self, idx: Sequence[int], T: int, layers: Sequence[int]) -> List[torch.Tensor]:
+        if list(layers) != self.layers:
+            raise MafedDistillError(f"the teacher cache holds layers {self.layers}, the step distils {list(layers)}")
+        if self._handle is None:
+            raise MafedDistillError("the sharded teacher cache has been released")
+        idx = [int(i) for i in idx]
+        bad = [i for i in idx if not 0 <= i < self.M]
+        if bad:
+            raise MafedDistillError(f"memory index {bad[0]} out of range for a teacher cache of {self.M} samples")
+        if not self.n_vis <= T <= self.T_c:
+            raise MafedDistillError(f"a batch of {T} tokens does not fit the teacher cache (n_vis = {self.n_vis}, "
+                                    f"T_c = {self.T_c}): the memory set changed since the cache was built")
+        out = [torch.empty((len(idx), T, self.D), dtype=d, device=self.device) for d in self.dtypes]
+        ranks, slots = [self.owner[i] for i in idx], [self.slot[i] for i in idx]
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        for dtype in dict.fromkeys(self.dtypes):
+            pick = [k for k, d in enumerate(self.dtypes) if d == dtype]
+            gather_sharded_raw([out[k].data_ptr() for k in pick], self.bases, [self.offsets[k] for k in pick], ranks,
+                               slots, len(idx), self.capacity, T, self.T_c, self.n_vis, self.D, _DTYPES[dtype], stream)
+        return out
+
+    def release(self):
+        """Free the shards, collectively over the cache's group: wait for this device's work and for every rank
+        (a peer may still be gathering from this shard), then unmap the peers' shards and free this one."""
+        if self._handle is None:
+            return
+        torch.cuda.synchronize(self.device)
+        torch.distributed.barrier(group=self.group)
+        self.local_states, self._slots = [], []
+        load().mafed_teacher_shard_destroy(self._handle)
+        self._handle = None
+
+
+def build_sharded(strategy, group=None) -> ShardedTeacherCache:
+    """``build`` split across the ranks of ``group`` (the default group if None), one process per GPU of one host:
+    rank ``r`` runs the build batches ``k % N == r`` (the same inputs at the same ``T_c`` as ``build``) into its own
+    shard, and maps every peer's shard through CUDA IPC.  Collective: every rank of the group calls it."""
+    dist = torch.distributed
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    if world > MAX_RANKS:
+        raise MafedDistillError(f"a sharded teacher cache spans at most {MAX_RANKS} ranks, the group has {world}")
+    lib = load()
+    batches, text_len, M = _build_batches(strategy)
+    n_vis = strategy.num_vision_tokens
+    T_c = n_vis + text_len
+    layers = strategy.loss_weights.get_distillation_layers()
+    device = next(strategy.past_model.parameters()).device
+    owner, slot, count = shard_owners(M, strategy.batch_size, world)
+    mine = batches[rank::world]
+    # this rank's first batch gives the layers' width and dtypes (rank 0 always has one)
+    first = _teacher_states(strategy, mine[0], text_len, layers, device) if mine else None
+    spec = None if first is None else (first[1][0].shape[-1], [str(h.dtype) for h in first[1]])
+    every = [None] * world
+    dist.all_gather_object(every, (socket.gethostname(), spec), group=group)
+    hosts = sorted({h for h, _ in every})
+    if len(hosts) != 1:
+        raise MafedDistillError(f"shard_teacher_cache needs every rank of the group on one host (CUDA IPC over "
+                                f"NVLink); the ranks run on {hosts}")
+    D, names = every[0][1]
+    if any(sp is not None and sp != every[0][1] for _, sp in every):
+        raise MafedDistillError(f"the ranks' teachers give different hidden-state widths or dtypes: {[sp for _, sp in every]}")
+    dtypes = [getattr(torch, n.split(".")[-1]) for n in names]
+    capacity = max(count)
+    offsets, nbytes = shard_layout(capacity, T_c, D, [torch.empty((), dtype=d).element_size() for d in dtypes])
+    _log.info("sharded teacher cache: rank %d/%d holds %d of %d samples (capacity %d) x %d layers x T_c %d x D %d = "
+              "%d bytes", rank, world, count[rank], M, capacity, len(layers), T_c, D, nbytes)
+
+    handle = ctypes.c_void_p()
+    hbytes = ctypes.create_string_buffer(lib.mafed_teacher_shard_handle_bytes())
+    rc = lib.mafed_teacher_shard_create(world, rank, nbytes, hbytes, ctypes.byref(handle))
+    every = [None] * world
+    dist.all_gather_object(every, (rc, hbytes.raw), group=group)
+    if any(r != 0 for r, _ in every):
+        lib.mafed_teacher_shard_destroy(handle)
+        failed = [r for r, (c, _) in enumerate(every) if c != 0]
+        raise MafedDistillError(f"rank(s) {failed} could not allocate a teacher-cache shard of {nbytes} bytes "
+                                f"({capacity} samples x {len(layers)} layers x T_c {T_c} x D {D}): "
+                                f"{lib.mafed_teacher_gather_error_string(every[failed[0]][0]).decode()}")
+    rc = lib.mafed_teacher_shard_connect(handle, b"".join(h for _, h in every))
+    flags = [None] * world
+    dist.all_gather_object(flags, rc, group=group)
+    if any(flags):
+        lib.mafed_teacher_shard_destroy(handle)
+        raise MafedDistillError(f"rank(s) {[r for r, c in enumerate(flags) if c]} could not map the peers' teacher-cache "
+                                "shards")
+    cache = ShardedTeacherCache(layers, dtypes, T_c, n_vis, M, D, owner, slot, count, capacity, offsets, nbytes,
+                                handle, group, rank, device)
+    for k, batch in enumerate(mine):
+        idx, hs = first if k == 0 else _teacher_states(strategy, batch, text_len, layers, device)
+        lo = slot[idx[0]]
+        for s, h in zip(cache._slots, hs):
+            s[lo:lo + len(idx)].copy_(h)
+    first = None
+    # every row is written before any peer reads it
+    torch.cuda.synchronize(device)
+    dist.barrier(group=group)
+    every = [None] * world
+    mine_spec = (M, T_c, layers, D, names)
+    dist.all_gather_object(every, mine_spec, group=group)
+    if any(e != mine_spec for e in every):
+        cache.release()
+        raise MafedDistillError(f"the ranks' teacher caches differ in (M, T_c, layers, D, dtypes): {every}")
+    return cache

@@ -16,6 +16,11 @@ entry, one launch and one exchange per dtype group), with and without token coun
 ``--adaptive``: instead, the ``adaptive`` importances computed over the ranks' shards of a task loader
 (``FeatureDistillation(global_importances=True)``) on the tiny VL model, against one GPU over all the batches, and the
 sharded ``replay()`` step that follows; and ``token_norm_sums(..., group=None)`` on a batch shard.
+
+``--teacher-cache-sharded``: instead, ``shard_teacher_cache=True``: each rank's shard against the replicated cache, and
+a sharded cached ``replay()`` step whose every rank's batch draws rows from every rank's shard, against the
+``teacher_cache=True`` step (bit for bit) and one GPU on the concatenated batch; then a second ``update()`` that
+releases and rebuilds the shards.
 """
 import argparse
 import os
@@ -39,6 +44,8 @@ def main():
                     help="adaptive importances over the ranks' loader shards, then a sharded replay() step")
     ap.add_argument("--teacher-cache", action="store_true",
                     help="replay() steps with teacher_cache=True, sharded, against one GPU on the concatenated batch")
+    ap.add_argument("--teacher-cache-sharded", action="store_true",
+                    help="shard_teacher_cache=True against the replicated cache and one GPU on the concatenated batch")
     args = ap.parse_args()
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
@@ -51,6 +58,8 @@ def main():
         finish(mixed_layers_check(rank, world))
     if args.teacher_cache:
         finish(teacher_cache_check(rank, world))
+    if args.teacher_cache_sharded:
+        finish(teacher_cache_sharded_check(rank, world))
     if args.adaptive:
         ok = shard_norm_sums_check(rank, world)
         finish(adaptive_check(rank, world) and ok)
@@ -280,6 +289,104 @@ def teacher_cache_check(rank, world):
     good = same_cache and n_s == hi - lo and n_f == B and e_loss < 1e-5 and e_grad < 1e-4
     print(f"rank {rank}/{world} teacher cache: caches equal on every rank {same_cache}, loss err {e_loss:.2e}, "
           f"summed gradient err {e_grad:.2e} {'OK' if good else 'FAIL'}", flush=True)
+    return good
+
+
+def teacher_cache_sharded_check(rank, world):
+    """``shard_teacher_cache=True``: every rank's ``local_states`` equal the replicated cache's rows of its samples and
+    its ``nbytes`` is its shard; a sharded cached ``replay()`` step in which every rank's batch holds a sample of every
+    rank's shard equals the replicated-cache step on the same ranks bit for bit (loss, every parameter gradient, the
+    batch masks) and one GPU's step on the concatenated batch within ``teacher_cache_check``'s tolerances; a second
+    ``update()`` releases the first task's shards and builds the next ones."""
+    import copy
+    from torch.utils.data import ConcatDataset
+    from gpu_util import rel_err
+    from mafed_b200 import teacher_cache as TC
+    from mafed_b200.methods import CLMethod
+    from tiny_vl import TinyVL
+    from vl_memory import VLSamples, collate
+
+    class Opts:
+        tasks = ["a", "b", "c"]; batch_size = 4; seed = 1; pin_mem = False; accumulate_grad_batches = 1
+
+    torch.manual_seed(0)
+    teacher = TinyVL(fp32_island=True).cuda()
+    student = copy.deepcopy(teacher)
+    with torch.no_grad():
+        for p in student.parameters():
+            p.add_(0.02 * torch.randn_like(p))
+
+    def strategy(group, shard):
+        fd = CLMethod["featdistill"](memory_size=64, opts=Opts(), model_type="vlpythia",
+                                     distillation_modality_weighing_strategy="balanced",
+                                     distillation_layer_weighing_strategy="discounted", distillation_layer=None,
+                                     num_hidden_layers=3, replay_coeff=0.0, teacher_cache=True,
+                                     shard_teacher_cache=shard, process_group=group, grad_multiplier=1.0)
+        fd.num_vision_tokens, fd.num_workers = 8, 0
+        fd.data_hooks = (collate, lambda loader: loader)
+        fd.update(dataset=VLSamples(64, seed=3, max_txt=9), model=teacher, dataloader=None)
+        return fd
+
+    def step(fd, idx, text_len):
+        memory = ConcatDataset(fd.datasets)
+        batch = TC.repad_left(collate([memory[i] for i in idx]), text_len)
+        batch.pop("labels")
+        batch = {k: v.cuda() if torch.is_tensor(v) else v for k, v in batch.items()}
+        batch["memory_index"] = list(idx)
+        fd.mem_dataloader = [batch]
+        model = copy.deepcopy(student)
+        loss, n_ex = fd.replay(model)
+        loss.backward()
+        torch.cuda.synchronize()
+        return loss.detach(), n_ex, [p.grad for p in model.parameters()], batch
+
+    sharded, replicated, full = strategy(None, True), strategy(None, False), strategy(False, False)
+    cache, whole = sharded._teacher_cache, replicated._teacher_cache
+    ok = isinstance(cache, TC.ShardedTeacherCache)
+    mine = [i for i in range(cache.M) if cache.owner[i] == rank]
+    ok &= all(torch.equal(a, b[mine]) for a, b in zip(cache.local_states, whole.states))
+    sizes = [s.element_size() for s in whole.states]
+    ok &= cache.nbytes == TC.shard_layout(max(cache.count), cache.T_c, cache.D, sizes)[1]
+    ok &= cache.count[rank] == len(mine)
+    # rank r's batch: one sample of build batch (r + j) % world -- held by rank (r + j) % world -- per j, and one more
+    n_batches = -(-cache.M // 4)
+    per_rank = [[((r + j) % world % n_batches) * 4 + (r + j) % 4 for j in range(world)] + [(3 * r + 1) % cache.M]
+                for r in range(world)]
+    idx = per_rank[rank]
+    every = [i for r in per_rank for i in r]
+    memory = ConcatDataset(full.datasets)
+    text_len = max(len(memory[i]["input_ids"]) for i in every)
+    remote = sum(cache.owner[i] != rank for i in idx)
+    loss_s, n_s, g_s, b_s = step(sharded, idx, text_len)
+    loss_r, n_r, g_r, b_r = step(replicated, idx, text_len)
+    same = torch.equal(loss_s, loss_r) and n_s == n_r == len(idx)
+    same &= all((a is None) == (b is None) and (a is None or torch.equal(a, b)) for a, b in zip(g_s, g_r))
+    same &= all(torch.equal(b_s[k], b_r[k]) for k in ("lang_masks", "image_masks"))
+    loss_f, n_f, g_f, _ = step(full, every, text_len)
+    e_loss = abs(float(loss_s) - float(loss_f)) / abs(float(loss_f))
+    e_grad = 0.0
+    for a, b in zip(g_s, g_f):
+        if b is None:
+            e_grad = e_grad if a is None else float("inf")
+            continue
+        a = a.clone()
+        dist.all_reduce(a)
+        e_grad = max(e_grad, rel_err(a, b))
+    close = n_f == len(every) and e_loss < 1e-5 and e_grad < 1e-4
+    # the next task: update() releases these shards (collectively) before it builds the new ones
+    first = cache
+    sharded.update(dataset=VLSamples(64, seed=4, max_txt=9), model=teacher, dataloader=None)
+    second = sharded._teacher_cache
+    rebuilt = first._handle is None and isinstance(second, TC.ShardedTeacherCache) and second.M == 2 * first.M
+    replicated.update(dataset=VLSamples(64, seed=4, max_txt=9), model=teacher, dataloader=None)
+    mine2 = [i for i in range(second.M) if second.owner[i] == rank]
+    rebuilt &= all(torch.equal(a, b[mine2]) for a, b in zip(second.local_states, replicated._teacher_cache.states))
+    second.release()
+    good = ok and same and close and rebuilt and remote >= world - 1
+    print(f"rank {rank}/{world} sharded teacher cache: {len(mine)} of {cache.M} samples, {cache.nbytes} bytes "
+          f"(replicated {whole.nbytes}), shard rows equal {ok}, step of {len(idx)} samples ({remote} from peers) "
+          f"bit-identical to the replicated cache {same}, against one GPU: loss err {e_loss:.2e} summed gradient err "
+          f"{e_grad:.2e}, released and rebuilt {rebuilt} {'OK' if good else 'FAIL'}", flush=True)
     return good
 
 
