@@ -7,6 +7,10 @@
 * ``_lib/libmafed_teacher_gather.so`` -- the teacher-cache gather kernel (``csrc/teacher_gather.cu``) behind its own
   C ABI (``include/mafed_teacher_gather.h``), bound by ``mafed_b200.teacher_cache``.  A unit of its own, so the
   distillation library and its export list stay as they are.
+* ``_lib/libmafed_cached_step.so`` -- the one-pass step that reads a replay batch's teacher rows straight from the
+  teacher cache (``csrc/cached_step.cu``, the TMA-ring kernels of the distillation library with the cache's
+  addressing) behind its own C ABI (``include/mafed_cached_step.h``), bound lazily by the torch extension.  A unit of
+  its own for the same reason.
 * ``_lib/mafed_torch_node*.so`` -- the torch extension (``csrc/torch_node.cpp``, host C++ only): the autograd node
   that turns one ``distill()`` into one call of the C ABI without Python on the hot path.
 """
@@ -32,6 +36,11 @@ GATHER_SOURCE = os.path.join(CSRC, "teacher_gather.cu")
 GATHER_HEADER = os.path.join(ROOT, "include", "mafed_teacher_gather.h")
 GATHER_LIB_PATH = os.path.join(LIB_DIR, "libmafed_teacher_gather.so")
 GATHER_STAMP_PATH = os.path.join(LIB_DIR, "gather.stamp")
+
+CACHED_SOURCE = os.path.join(CSRC, "cached_step.cu")
+CACHED_HEADER = os.path.join(ROOT, "include", "mafed_cached_step.h")
+CACHED_LIB_PATH = os.path.join(LIB_DIR, "libmafed_cached_step.so")
+CACHED_STAMP_PATH = os.path.join(LIB_DIR, "cached_step.stamp")
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", *ARCH, "-lineinfo", "-Xcompiler", "-fPIC"]
@@ -118,6 +127,20 @@ def build_teacher_gather(force=False, verbose=False):
     return GATHER_LIB_PATH
 
 
+def build_cached_step(force=False, verbose=False):
+    """Compile libmafed_cached_step.so for sm_100a if missing or older than its source or the kernel headers."""
+    fp = _fingerprint([CACHED_SOURCE, CACHED_HEADER] + HEADERS, NVCC_FLAGS)
+    if not force and not _stale(CACHED_LIB_PATH, CACHED_STAMP_PATH, fp):
+        return CACHED_LIB_PATH
+    os.makedirs(LIB_DIR, exist_ok=True)
+    extra = ["-Xptxas=-v"] if verbose else []
+    _run([[_nvcc(), *NVCC_FLAGS, *extra, "-I", os.path.join(ROOT, "include"), "-I", CSRC, "-shared", CACHED_SOURCE,
+           "-o", CACHED_LIB_PATH]], verbose)
+    with open(CACHED_STAMP_PATH, "w") as f:
+        f.write(fp)
+    return CACHED_LIB_PATH
+
+
 def build_torch_ext(force=False, verbose=False):
     """Compile the torch extension (host C++ against the torch headers; it dlopens libmafed_distill.so)."""
     from torch.utils import cpp_extension as ce
@@ -129,7 +152,8 @@ def build_torch_ext(force=False, verbose=False):
     libdir = ce.library_paths()[0]
     flags = CXX_FLAGS + [f"-D_GLIBCXX_USE_CXX11_ABI={int(torch.compiled_with_cxx11_abi())}",
                          f"-DTORCH_EXTENSION_NAME={EXT_NAME}", "-DTORCH_API_INCLUDE_EXTENSION_H"]
-    fp = _fingerprint([EXT_SOURCE, os.path.join(ROOT, "include", "mafed_distill.h")], flags + [torch.__version__])
+    fp = _fingerprint([EXT_SOURCE, os.path.join(ROOT, "include", "mafed_distill.h"), CACHED_HEADER],
+                      flags + [torch.__version__])
     if not force and not _stale(EXT_PATH, EXT_STAMP_PATH, fp):
         return EXT_PATH
     os.makedirs(LIB_DIR, exist_ok=True)
@@ -147,5 +171,6 @@ if __name__ == "__main__":
     force, verbose = "--force" in sys.argv, "-v" in sys.argv
     print(build(force=force, verbose=verbose))
     print(build_teacher_gather(force=force, verbose=verbose))
+    print(build_cached_step(force=force, verbose=verbose))
     if "--no-ext" not in sys.argv:
         print(build_torch_ext(force=force, verbose=verbose))

@@ -83,14 +83,34 @@ __device__ __forceinline__ void named_bar_sync(int id, int n_threads) {
   asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(n_threads) : "memory");
 }
 
+// ---------------------------------------------------------------- teacher-row addressing
+// Where the producer finds the teacher row of row (b, t) of layer l.
+//  * DenseTeacher: the [B, T, D] tensors of an ordinary step, t[l] + row * t_row_pitch.
+//  * CacheTeacher: the per-task teacher cache (include/mafed_cached_step.h), one contiguous [M, T_c, D] tensor per
+//    layer at t[l]; sample b is memory sample idx[b], its visual rows t < n_vis at the start of the sample's T_c rows
+//    and its text rows right-aligned at their end -- the mapping of the teacher-cache gather, so that the step reads
+//    the rows a gathered tensor would hold.  The table travels in the kernel parameters (__grid_constant__).
+struct DenseTeacher {
+  static constexpr bool kCache = false;
+};
+
+constexpr int kCacheMaxSamples = 2048;
+struct CacheTeacher {
+  static constexpr bool kCache = true;
+  int32_t idx[kCacheMaxSamples];   // memory index of each sample, in [0, M)
+  long long T_c;                   // cache rows of one sample
+  long long shift;                 // T_c - T: offset of the text rows past n_vis
+  float* gout_seen;                // backward fix-up: receives the upstream gradient it saw (optional)
+};
+
 // ---------------------------------------------------------------- producer
 // All 32 lanes of the producer warp run this; lane r owns row r of every stage.  The backward walks its tiles
 // last-to-first, so that it starts on the rows the forward left in L2.  A stage holds its rows' student bytes, then
 // their teacher bytes (TT: the teacher's element type; its rows are row_bytes >> TeacherChunk::kShift long).
-template <typename T, typename TT>
+template <typename T, typename TT, typename TA = DenseTeacher>
 __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom& geo, unsigned char* data,
                                              uint64_t* full, uint64_t* empty, TmaStageMeta* meta, int lane,
-                                             bool for_backward) {
+                                             bool for_backward, const TA& ta = TA()) {
   const long long tiles_per_layer = (p.n_rows + geo.rows - 1) / geo.rows;
   const long long total = tiles_per_layer * p.n_layers;
   const uint32_t row_bytes = (uint32_t)p.n_chunks * 16u;
@@ -103,10 +123,12 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
   // The row weights of a tile come from the attention mask (an L2 round trip).  They are fetched one tile ahead, so
   // that the trip overlaps the wait for a free slot: a run of padded tiles (long, half-empty text) is otherwise paced
   // by this warp's load latency instead of by the zero-fill's bandwidth.
-  struct Tile { int l, n_rows, m; long long row0; float w; };
+  // trow: the lane's teacher row in the cache (CacheTeacher only)
+  struct Tile { int l, n_rows, m; long long row0; float w; long long trow; };
   // (layer, tile in layer) of this CTA's tiles advance by gridDim.x per step: kept incrementally, no 64-bit division
   // on the per-tile path; the row -> (sample, position) split is a 32-bit division whenever the row count allows it
-  const bool rows32 = p.n_rows <= 0x7fffffffLL;
+  // (always for the cache, whose host side admits at most 2^31 - 1 rows)
+  const bool rows32 = TA::kCache || p.n_rows <= 0x7fffffffLL;
   int f_l = (int)((long long)blockIdx.x / tiles_per_layer);
   long long f_til = (long long)blockIdx.x - (long long)f_l * tiles_per_layer;
   auto fetch = [&]() {
@@ -116,6 +138,7 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
     x.n_rows = (int)min((long long)geo.rows, p.n_rows - x.row0);
     x.m = 1;
     x.w = 0.f;
+    if constexpr (TA::kCache) x.trow = 0;
     if (lane < x.n_rows) {
       if (rows32) {
         const unsigned row = (unsigned)x.row0 + (unsigned)lane;
@@ -123,6 +146,7 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
         const int t = (int)(row - bb * (unsigned)p.T);
         if (t < p.n_vis) x.w = 1.f;
         else { x.m = 0; x.w = (float)__ldg(p.mask + (long long)bb * p.txt + (t - p.n_vis)); }
+        if constexpr (TA::kCache) x.trow = (long long)ta.idx[bb] * ta.T_c + t + (t < p.n_vis ? 0 : ta.shift);
       } else {
         x.w = row_weight(p, x.row0 + lane, x.m);
       }
@@ -168,14 +192,36 @@ __device__ __forceinline__ void tma_producer(const PathParams& p, const TmaGeom&
     const char* sb = reinterpret_cast<const char*>(p.s[l]) + row0 * row_pitch;
     const char* tb = reinterpret_cast<const char*>(p.t[l]) + row0 * t_row_pitch;
     const unsigned all = (n_rows >= 32) ? 0xffffffffu : ((1u << n_rows) - 1u);
-    if (contiguous && valid == all) {
-      // whole tile live: one bulk copy per tensor
-      if (lane == 0) bulk_g2s(s_dst, sb, (uint32_t)n_rows * row_bytes, bar);
-      if (lane == 1 && both) bulk_g2s(t_dst, tb, (uint32_t)n_rows * t_row_bytes, bar);
-    } else if (w != 0.f) {
-      // ragged tile: only live rows are fetched (padded text rows cost no bandwidth)
-      bulk_g2s(s_dst + (uint32_t)lane * row_bytes, sb + (long long)lane * row_pitch, row_bytes, bar);
-      if (both) bulk_g2s(t_dst + (uint32_t)lane * t_row_bytes, tb + (long long)lane * t_row_pitch, t_row_bytes, bar);
+    if constexpr (TA::kCache) {
+      // the lane's teacher row in the cache (a sample's rows are two runs there: visual prefix, text block)
+      const char* tr = reinterpret_cast<const char*>(p.t[l]) + cur.trow * (long long)t_row_bytes;
+      if (contiguous && valid == all) {
+        if (lane == 0) bulk_g2s(s_dst, sb, (uint32_t)n_rows * row_bytes, bar);
+        // one bulk copy per contiguous run of teacher rows: a lane starts a run unless its row follows the previous
+        // lane's in memory (same bytes in flight as a single copy: expect_tx is unchanged)
+        const unsigned long long a = reinterpret_cast<unsigned long long>(tr);
+        const unsigned long long prev = __shfl_up_sync(0xffffffffu, a, 1);
+        const bool start = lane < n_rows && (lane == 0 || a != prev + t_row_bytes);
+        const unsigned starts = __ballot_sync(0xffffffffu, start);
+        if (start && both) {
+          const unsigned later = starts & (0xfffffffeu << lane);   // the runs that start after this lane
+          const int end = later ? __ffs(later) - 1 : n_rows;
+          bulk_g2s(t_dst + (uint32_t)lane * t_row_bytes, tr, (uint32_t)(end - lane) * t_row_bytes, bar);
+        }
+      } else if (w != 0.f) {
+        bulk_g2s(s_dst + (uint32_t)lane * row_bytes, sb + (long long)lane * row_pitch, row_bytes, bar);
+        if (both) bulk_g2s(t_dst + (uint32_t)lane * t_row_bytes, tr, t_row_bytes, bar);
+      }
+    } else {
+      if (contiguous && valid == all) {
+        // whole tile live: one bulk copy per tensor
+        if (lane == 0) bulk_g2s(s_dst, sb, (uint32_t)n_rows * row_bytes, bar);
+        if (lane == 1 && both) bulk_g2s(t_dst, tb, (uint32_t)n_rows * t_row_bytes, bar);
+      } else if (w != 0.f) {
+        // ragged tile: only live rows are fetched (padded text rows cost no bandwidth)
+        bulk_g2s(s_dst + (uint32_t)lane * row_bytes, sb + (long long)lane * row_pitch, row_bytes, bar);
+        if (both) bulk_g2s(t_dst + (uint32_t)lane * t_row_bytes, tb + (long long)lane * t_row_pitch, t_row_bytes, bar);
+      }
     }
     if (++stage == geo.stages) { stage = 0; phase ^= 1u; }
   }
@@ -433,9 +479,10 @@ __device__ __forceinline__ float cosine_row_unrolled(uint32_t sa, uint32_t ta, i
 
 // MODE = kBackward: gradients only.  MODE = kFused: the consumers also accumulate the forward's loss
 // sums from the rows they already hold in shared memory (one pass over student and teacher per step).
-template <typename T, int LOSS, int MODE, typename TT = T>
-__global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
-k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo) {
+// TA: the teacher-row addressing (k_bwd_tma: DenseTeacher; k_bwd_tma_cached: CacheTeacher); only the producer
+// reads it, so the consumers' arithmetic is the same for both.
+template <typename T, int LOSS, int MODE, typename TT, typename TA>
+__device__ __forceinline__ void bwd_tma_body(const PathParams& p, const TmaGeom& geo, const TA& ta) {
   constexpr int NE = Pack<T>::kPer16;
   constexpr bool FUSED = MODE == kFused;
   // a half-precision teacher under an fp32 student: no unrolled short-row cosine forms (general two-sweep loop)
@@ -453,10 +500,13 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     gout = p.fixed_gout;
   } else {
     gout = (p.grad_out ? __ldg(p.grad_out) : 1.f) * p.gout_scale;
+    if constexpr (TA::kCache) {
+      if (ta.gout_seen != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *ta.gout_seen = gout;
+    }
     if (p.skip_if_gout_equals && gout == p.fixed_gout) return;  // fix-up launch with nothing to fix
   }
   if (warp == kTmaConsumerWarps) {
-    tma_producer<T, TT>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, !FUSED);
+    tma_producer<T, TT, TA>(p, geo, dyn_smem, sm.full, sm.empty, sm.meta, lane, !FUSED, ta);
     return;
   }
   // Scale table in shared memory.  One-pass step with the prologue folded in: while the producer's first
@@ -683,6 +733,20 @@ k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom 
     cta_sums_store(sums, p.ws, p.n_layers, 0, kTmaConsumerThreads);
     if (p.tail_done != nullptr) tma_tail<kTmaConsumerThreads>(p, p.inline_scale ? s_counts : p.tail_counts_in, counts_epoch);
   }
+}
+
+template <typename T, int LOSS, int MODE, typename TT = T>
+__global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
+k_bwd_tma(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo) {
+  bwd_tma_body<T, LOSS, MODE, TT>(p, geo, DenseTeacher());
+}
+
+// The same kernel reading the teacher rows straight from the per-task cache (mafed_cached_step.h).
+template <typename T, int LOSS, int MODE, typename TT = T>
+__global__ void __launch_bounds__(kTmaConsumerThreads + 32, 1)
+k_bwd_tma_cached(const __grid_constant__ PathParams p, const __grid_constant__ TmaGeom geo,
+                 const __grid_constant__ CacheTeacher c) {
+  bwd_tma_body<T, LOSS, MODE, TT>(p, geo, c);
 }
 
 }  // namespace MAFED_NS

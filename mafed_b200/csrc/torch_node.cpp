@@ -24,6 +24,7 @@
 #include <tuple>
 #include <vector>
 
+#include "mafed_cached_step.h"
 #include "mafed_distill.h"
 
 namespace {
@@ -75,6 +76,53 @@ const Api& api() {
   TORCH_CHECK(g_api.bound, "mafed_torch_node: bind(<path of libmafed_distill.so>) has not been called");
   return g_api;
 }
+
+// The step that reads the teacher straight from the teacher cache (include/mafed_cached_step.h): a library of its
+// own, bound on first use (`bind_cached(path)`, mafed_b200.node.load_cached).
+struct CachedApi {
+  decltype(&mafed_cached_step_abi_version) abi_version = nullptr;
+  decltype(&mafed_cached_step_error_string) error_string = nullptr;
+  decltype(&mafed_cached_step_supported) supported = nullptr;
+  decltype(&mafed_cached_step) step = nullptr;
+  decltype(&mafed_cached_step_bwd) bwd = nullptr;
+  bool bound = false;
+};
+CachedApi g_cached;
+
+template <typename F>
+void load_cached_symbol(void* lib, const char* name, F& fn) {
+  fn = reinterpret_cast<F>(dlsym(lib, name));
+  TORCH_CHECK(fn != nullptr, "libmafed_cached_step.so does not export ", name, ": rebuild it (python -m mafed_b200.build)");
+}
+
+void bind_cached(const std::string& path) {
+  void* lib = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
+  TORCH_CHECK(lib != nullptr, "cannot load ", path, " (", dlerror(),
+              "): build it with `python -m mafed_b200.build` -- the cached step has no eager fallback");
+  CachedApi a;
+  load_cached_symbol(lib, "mafed_cached_step_abi_version", a.abi_version);
+  load_cached_symbol(lib, "mafed_cached_step_error_string", a.error_string);
+  load_cached_symbol(lib, "mafed_cached_step_supported", a.supported);
+  load_cached_symbol(lib, "mafed_cached_step", a.step);
+  load_cached_symbol(lib, "mafed_cached_step_bwd", a.bwd);
+  TORCH_CHECK(a.abi_version() == MAFED_CACHED_ABI_VERSION, "libmafed_cached_step.so ABI version ", a.abi_version(),
+              " != ", MAFED_CACHED_ABI_VERSION, "; rebuild");
+  a.bound = true;
+  g_cached = a;
+}
+
+const CachedApi& cached_api() {
+  TORCH_CHECK(g_cached.bound, "mafed_torch_node: bind_cached(<path of libmafed_cached_step.so>) has not been called");
+  return g_cached;
+}
+
+// A step whose teacher rows come from the teacher cache: the teacher table holds the [M, T_c, D] cache tensors and
+// sample b reads memory sample idx[b].
+struct CacheRef {
+  std::vector<int64_t> idx;
+  int64_t M = 0;
+  int32_t T_c = 0;
+};
 
 void check_rc(int rc, const char* what) {
   TORCH_CHECK(rc == 0, what, " failed: ", api().error_string(rc), " (code ", rc, ")");
@@ -277,6 +325,24 @@ void launch_bwd(const mafed_shape_t& shape, const Tables& tb, const at::Tensor& 
            "mafed_distill_bwd");
 }
 
+void launch_cached_step(const mafed_shape_t& shape, const Tables& tb, const CacheRef& c, const at::Tensor& mask,
+                        const mafed_weights_t& w, float fixed, const Scratch& sc, float* out, float* bwd_scale,
+                        int64_t* lang, int64_t* image, cudaStream_t stream) {
+  const CachedApi& a = cached_api();
+  const int rc = a.step(&shape, tb.s, tb.t, c.M, c.T_c, c.idx.data(), tb.g, mask.defined() ? mask.data_ptr<int64_t>() : nullptr,
+                        &w, fixed, sc.ws, out, bwd_scale, sc.sums, lang, image, stream);
+  TORCH_CHECK(rc == 0, "mafed_cached_step failed: ", a.error_string(rc), " (code ", rc, ")");
+}
+
+void launch_cached_bwd(const mafed_shape_t& shape, const Tables& tb, const CacheRef& c, const at::Tensor& mask,
+                       const float* bwd_scale, const at::Tensor& g, float grad_out_scale, const float* skip, float* seen,
+                       cudaStream_t stream) {
+  const CachedApi& a = cached_api();
+  const int rc = a.bwd(&shape, tb.s, tb.t, c.M, c.T_c, c.idx.data(), tb.g, mask.defined() ? mask.data_ptr<int64_t>() : nullptr,
+                       bwd_scale, g.data_ptr<float>(), grad_out_scale, skip, seen, stream);
+  TORCH_CHECK(rc == 0, "mafed_cached_step_bwd failed: ", a.error_string(rc), " (code ", rc, ")");
+}
+
 // The upstream gradient as the kernels read it: fp32, contiguous, on `device`.
 at::Tensor upstream(at::Tensor g, c10::Device device) {
   if (g.scalar_type() != at::kFloat || g.device() != device) g = g.to(device, at::kFloat);
@@ -300,8 +366,9 @@ struct DistillBackward : public Node {
   float* seen = nullptr;           // pinned host word that receives the upstream gradient (kept alive by `seen_owner`)
   at::Tensor seen_owner;
   bool released = false;
+  std::shared_ptr<CacheRef> cache;  // a step read from the teacher cache: `teachers` are the cache tensors
 
-  std::string name() const override { return "MafedDistillBackward"; }
+  std::string name() const override { return cache ? "MafedCachedDistillBackward" : "MafedDistillBackward"; }
 
   void release_variables() override {
     for (auto& s : students) s.reset_data();
@@ -343,8 +410,12 @@ struct DistillBackward : public Node {
     for (size_t i = 0, j = 0; i < n; ++i)
       if (needs[i]) out[i] = std::move(views[j++]);
     const float fixed = plan->fixed();
-    launch_bwd(shape, tb, m, bwd_scale, g, (float)plan->grad_multiplier, gate ? &fixed : nullptr, gate ? seen : nullptr,
-               stream);
+    if (cache)   // the full-grid fix-up (libmafed_cached_step.so starts nothing from the device)
+      launch_cached_bwd(shape, tb, *cache, m, bwd_scale, g, (float)plan->grad_multiplier, gate ? &fixed : nullptr,
+                        gate ? seen : nullptr, stream);
+    else
+      launch_bwd(shape, tb, m, bwd_scale, g, (float)plan->grad_multiplier, gate ? &fixed : nullptr,
+                 gate ? seen : nullptr, stream);
     grad_buf.reset();   // handed to autograd: a second backward (retain_graph) recomputes into a fresh buffer
     return out;
   }
@@ -358,13 +429,15 @@ struct DistillBackward : public Node {
 // prefetch_counts.  seen: optional pinned float[1].
 // Returns (total, aux, masks): the 0-dim fp32 loss with the node attached, the [3L] layer / (text, vision) losses,
 // and the [2, B, T] mask tensor (None if not requested).
-std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
+// cache: a one-pass step whose teachers are the [M, T_c, D] tensors of the teacher cache (distill_cached).
+std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill_impl(
     const std::shared_ptr<Plan>& plan, std::vector<at::Tensor> students, std::vector<at::Tensor> teachers,
     const c10::optional<at::Tensor>& attn_mask, const py::object& masks_out, int64_t comm,
-    const std::shared_ptr<CountsTicket>& ticket, const c10::optional<at::Tensor>& seen, int64_t tuning_addr) {
+    const std::shared_ptr<CountsTicket>& ticket, const c10::optional<at::Tensor>& seen, int64_t tuning_addr,
+    const std::shared_ptr<CacheRef>& cache) {
   const int L = plan->n_layers;
   TORCH_CHECK((int)students.size() == L && (int)teachers.size() == L, "students / teachers / plan length mismatch");
-  {
+  if (!cache) {
     // One dtype everywhere, or fp32 students with teachers of one half-precision dtype: the kernels read the tensors
     // as they are (a teacher pair, MAFED_DTYPE_PAIR).  distill_loss gives each dtype group of a step its own call, so
     // any other mix arriving here is the one group of pairs the kernels refuse (a student narrower than its teacher,
@@ -393,14 +466,22 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
   for (int i = 0; i < L; ++i) {
     at::Tensor& s = students[i];
     at::Tensor& t = teachers[i];
-    TORCH_CHECK_VALUE(s.sizes() == s0.sizes() && t.sizes() == s0.sizes(),
-                      "all selected hidden states must share one [B, T, D] shape");
+    if (cache) {
+      TORCH_CHECK_VALUE(s.sizes() == s0.sizes() && t.dim() == 3 && t.size(0) == cache->M && t.size(1) == cache->T_c &&
+                            t.size(2) == s0.size(2) && t.is_contiguous(),
+                        "the teacher cache must hold one contiguous [M, T_c, D] tensor per selected layer");
+    } else {
+      TORCH_CHECK_VALUE(s.sizes() == s0.sizes() && t.sizes() == s0.sizes(),
+                        "all selected hidden states must share one [B, T, D] shape");
+    }
     TORCH_CHECK_VALUE(s.scalar_type() == s0.scalar_type() && t.scalar_type() == teachers[0].scalar_type() &&
                           s.device() == device && t.device() == device,
                       "student / teacher dtype or device mismatch");
     needs[i] = grad_mode && s.requires_grad();
     any_need = any_need || needs[i];
   }
+  TORCH_CHECK(!cache || (plan->single_pass && any_need && comm == 0 && ticket == nullptr && !plan->cls),
+              "distill_cached runs the one-pass step of one rank with gradients (single_pass, no CLS)");
   // collect the graph edges before the tensors are replaced by contiguous copies
   torch::autograd::edge_list edges;
   if (any_need) edges = torch::autograd::collect_next_edges(students);
@@ -450,8 +531,12 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
   if (plan->single_pass && any_need) {
     grad_buf = alloc_grads(count_needs(needs), s0, plan->cls);
     fill_grad_ptrs(grad_buf, needs, tb);
-    launch_step(shape, tb, mask, plan->w, plan->fixed(), sc, out.data_ptr<float>(), bwd_scale, lang, image, comm,
-                ticket_ptr, stream);
+    if (cache)
+      launch_cached_step(shape, tb, *cache, mask, plan->w, plan->fixed(), sc, out.data_ptr<float>(), bwd_scale, lang,
+                         image, stream);
+    else
+      launch_step(shape, tb, mask, plan->w, plan->fixed(), sc, out.data_ptr<float>(), bwd_scale, lang, image, comm,
+                  ticket_ptr, stream);
   } else {
     launch_fwd_step(shape, tb, mask, plan->w, sc, out.data_ptr<float>(), bwd_scale, lang, image, comm, stream);
   }
@@ -482,6 +567,7 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
     node->bwd_scale = bwd_scale;
     node->grad_buf = grad_buf;
     node->needs = needs;
+    node->cache = cache;
     if (seen.has_value() && seen->defined()) {
       // must be device-accessible host memory (a pinned tensor): the gate kernel stores into it
       TORCH_CHECK_VALUE(seen->scalar_type() == at::kFloat && seen->device().is_cpu(), "seen must be a pinned float32 tensor");
@@ -491,6 +577,62 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
     torch::autograd::set_history(total, node);
   }
   return std::make_tuple(std::move(total), std::move(aux), std::move(masks));
+}
+
+std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill(
+    const std::shared_ptr<Plan>& plan, std::vector<at::Tensor> students, std::vector<at::Tensor> teachers,
+    const c10::optional<at::Tensor>& attn_mask, const py::object& masks_out, int64_t comm,
+    const std::shared_ptr<CountsTicket>& ticket, const c10::optional<at::Tensor>& seen, int64_t tuning_addr) {
+  return distill_impl(plan, std::move(students), std::move(teachers), attn_mask, masks_out, comm, ticket, seen,
+                      tuning_addr, nullptr);
+}
+
+// The one-pass step of one rank with the teacher rows read straight from the teacher cache: `cache` holds one
+// contiguous [M, T_c, D] tensor per selected layer, `idx` the B memory indices of the batch (each in [0, M)).  Same
+// result and node as `distill` on the gathered teachers; the node keeps the cache tensors (version-checked) and runs the
+// library's full-grid fix-up as its backward.  The caller asks `cached_supported` first.
+std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> distill_cached(
+    const std::shared_ptr<Plan>& plan, std::vector<at::Tensor> students, std::vector<at::Tensor> cache,
+    std::vector<int64_t> idx, int64_t T_c, const c10::optional<at::Tensor>& attn_mask, const py::object& masks_out,
+    const c10::optional<at::Tensor>& seen, int64_t tuning_addr) {
+  cached_api();
+  TORCH_CHECK_VALUE(!cache.empty() && cache[0].dim() == 3, "the teacher cache must hold [M, T_c, D] tensors");
+  TORCH_CHECK_VALUE(!students.empty() && students[0].dim() == 3 && (int64_t)idx.size() == students[0].size(0),
+                    "one memory index per sample of the batch");
+  auto ref = std::make_shared<CacheRef>();
+  ref->idx = std::move(idx);
+  ref->M = cache[0].size(0);
+  ref->T_c = (int32_t)T_c;
+  return distill_impl(plan, std::move(students), std::move(cache), attn_mask, masks_out, 0, nullptr, seen, tuning_addr,
+                      ref);
+}
+
+// Does libmafed_cached_step.so take this step (mafed_cached_step_supported)?  False for dtype mixes it has no kernel
+// for; the caller then gathers the teacher rows and runs `distill`.
+bool cached_supported(const std::shared_ptr<Plan>& plan, const std::vector<at::Tensor>& students,
+                      const std::vector<at::Tensor>& cache, int64_t T_c, int64_t tuning_addr) {
+  const CachedApi& a = cached_api();
+  const int L = plan->n_layers;
+  if ((int)students.size() != L || (int)cache.size() != L || plan->cls) return false;
+  const at::Tensor& s0 = students[0];
+  const at::Tensor& c0 = cache[0];
+  if (s0.dim() != 3 || c0.dim() != 3 || !s0.is_cuda()) return false;
+  const auto st = s0.scalar_type(), ct = c0.scalar_type();
+  const bool native = st == ct || (st == at::kFloat && (ct == at::kBFloat16 || ct == at::kHalf));
+  if (!native || (st != at::kFloat && st != at::kBFloat16 && st != at::kHalf)) return false;
+  Tables tb;
+  for (int i = 0; i < L; ++i) {
+    const at::Tensor& s = students[i];
+    const at::Tensor& c = cache[i];
+    if (s.sizes() != s0.sizes() || s.scalar_type() != st || !s.is_contiguous() || s.device() != s0.device() ||
+        c.sizes() != c0.sizes() || c.scalar_type() != ct || !c.is_contiguous() || c.device() != s0.device() ||
+        c.size(2) != s0.size(2) || c.size(1) != T_c)
+      return false;
+    tb.s[i] = s.data_ptr();
+    tb.t[i] = c.data_ptr();
+  }
+  const mafed_shape_t shape = make_shape(s0, c0, L, plan->loss_kind, false, plan->n_vis, tuning_addr);
+  return a.supported(&shape, tb.s, tb.t, c0.size(0), (int32_t)T_c) == 1;
 }
 
 // Token counts ahead of the step (mafed_distill_prefetch_counts): launches on the side stream, returns the ticket.
@@ -687,6 +829,12 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
       .def("data_ptr", [](CountsTicket& t) { return (uint64_t)(uintptr_t)t.tensor.data_ptr(); });
   m.def("distill", &distill, py::arg("plan"), py::arg("students"), py::arg("teachers"), py::arg("attn_mask"),
         py::arg("masks_out"), py::arg("comm"), py::arg("ticket"), py::arg("seen"), py::arg("tuning"));
+  m.def("bind_cached", &bind_cached, "dlopen libmafed_cached_step.so and resolve its C ABI");
+  m.def("cached_bound", [] { return g_cached.bound; });
+  m.def("distill_cached", &distill_cached, py::arg("plan"), py::arg("students"), py::arg("cache"), py::arg("idx"),
+        py::arg("T_c"), py::arg("attn_mask"), py::arg("masks_out"), py::arg("seen"), py::arg("tuning"));
+  m.def("cached_supported", &cached_supported, py::arg("plan"), py::arg("students"), py::arg("cache"), py::arg("T_c"),
+        py::arg("tuning"));
   m.def("prefetch_counts", &prefetch_counts, py::arg("attn_mask"), py::arg("n_vis"), py::arg("comm"), py::arg("tuning"));
 }
 

@@ -675,28 +675,72 @@ def distill_loss(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tens
     # functions (distillation.py:90,244).  Every launch has its own backward gate, and across batch shards its own
     # exchange: the groups come from the model's dtypes, so every rank runs the same sequence.  A counts ticket is only
     # read by a step, so every launch may take it.
+    split = _split(plan, students, teachers)
+    if split is None:
+        total, aux, both = _any_step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
+    else:
+        steps, runs = split
+        total, aux, both = _joined(steps, runs, [
+            _any_step(sub, attn_mask, group, [teachers[i] for i in idx], mask_out if k == 0 else None,
+                      [students[i] for i in idx], ticket, seen) for k, (idx, sub) in enumerate(steps)])
+    if not return_masks:
+        return total, aux
+    return total, aux, (None if both is None else (both[0], both[1]))
+
+
+def _split(plan: DistillPlan, students, teachers):
+    """``None`` when one launch takes every layer, else ``plan.split`` of the layers' dtype pairs."""
     s_type, t_type = students[0].dtype, teachers[0].dtype
     one_launch = len(students) <= cabi.MAX_LAYERS
     for s, t in zip(students, teachers):
         one_launch = one_launch and s.dtype == s_type and t.dtype == t_type
-    split = None if one_launch else plan.split(tuple([(s.dtype, t.dtype) for s, t in zip(students, teachers)]))
-    if split is None:
-        total, aux, both = _any_step(plan, attn_mask, group, teachers, mask_out, students, ticket, seen)
-        if not return_masks:
-            return total, aux
-        return total, aux, (None if both is None else (both[0], both[1]))
-    steps, runs = split
-    total, parts, both = None, [], None
-    for k, (idx, sub) in enumerate(steps):
-        part, aux, masks = _any_step(sub, attn_mask, group, [teachers[i] for i in idx], mask_out if k == 0 else None,
-                                     [students[i] for i in idx], ticket, seen)
-        if k == 0:
-            both = masks
+    return None if one_launch else plan.split(tuple([(s.dtype, t.dtype) for s, t in zip(students, teachers)]))
+
+
+def _joined(steps, runs, results):
+    """``(total, aux, masks)`` of a step run as several launches (``results``: each launch's ``(total, aux, masks)``),
+    with ``aux`` in the caller's layer order: layer losses, then (text, vision) pairs."""
+    total, parts = None, []
+    for part, aux, _ in results:
         total = part if total is None else total + part
         parts.append(aux)
-    # aux in the caller's layer order: layer losses, then (text, vision) pairs
     aux = torch.cat([parts[k][lo:hi] for k, lo, hi in runs] +
                     [parts[k][len(steps[k][0]) + 2 * lo:len(steps[k][0]) + 2 * hi] for k, lo, hi in runs])
+    return total, aux, results[0][2]
+
+
+def cached_distill_loss(students: Sequence[torch.Tensor], cache: Sequence[torch.Tensor], idx: Sequence[int], T_c: int,
+                        attn_mask, plan: DistillPlan, mask_out=None, seen=None, return_masks: bool = False):
+    """``distill_loss`` of one rank's one-pass step whose teacher rows come straight from the teacher cache: ``cache``
+    holds one contiguous ``[M, T_c, D]`` tensor per selected layer (``TeacherCache.step_inputs``) and sample ``b`` of
+    the batch is memory sample ``idx[b]``.  The step's kernels read the rows where they are, so no ``[B, T, D]`` copy
+    of the teacher is made; the loss, gradients, masks and ``aux`` are bit-identical to ``distill_loss`` on the
+    gathered teachers (``teacher_cache.gather``).
+
+    Returns ``None``, having launched nothing, when some launch of the step is not one ``libmafed_cached_step.so``
+    takes (``mafed_cached_step_supported``; a launch without gradients, i.e. the two-pass form; a dtype group the
+    kernels refuse): the caller then gathers and calls ``distill_loss``, so a step never mixes the two libraries.
+    The same ``dtype_groups`` split as ``distill_loss``; CLS, the two-pass form, batch sharding and ``torch.compile``
+    are the caller's to route to ``distill_loss``."""
+    if len(students) != len(cache) or len(students) != len(plan.layers):
+        raise ValueError("students / cache / plan.layers length mismatch")
+    if plan.cls or not plan.single_pass or not torch.is_grad_enabled():
+        return None
+    ext = node.load_cached()
+    tuning = cabi.active_tuning_address()
+    split = _split(plan, students, cache)
+    steps = [(None, plan)] if split is None else split[0]
+    launches = []
+    for lidx, sub in steps:
+        s = list(students) if lidx is None else [students[i] for i in lidx]
+        c = list(cache) if lidx is None else [cache[i] for i in lidx]
+        if not any(x.requires_grad for x in s) or not ext.cached_supported(sub.node_plan(), s, c, T_c, tuning):
+            return None
+        launches.append((sub, s, c))
+    idx = [int(i) for i in idx]
+    results = [ext.distill_cached(sub.node_plan(), s, c, idx, T_c, attn_mask, mask_out if k == 0 else None, seen, tuning)
+               for k, (sub, s, c) in enumerate(launches)]
+    total, aux, both = results[0] if split is None else _joined(split[0], split[1], results)
     if not return_masks:
         return total, aux
     return total, aux, (None if both is None else (both[0], both[1]))

@@ -27,7 +27,8 @@ import torch
 from mafed_b200 import cabi
 from mafed_b200 import comm as _comm
 from mafed_b200.capture import HiddenStateCapture, HiddenStateTuple
-from mafed_b200.distill_op import DistillPlan, distill_loss, modality_masks, resolve_group, seen_slot
+from mafed_b200.distill_op import (DistillPlan, cached_distill_loss, distill_loss, modality_masks, resolve_group,
+                                   seen_slot)
 from mafed_b200.methods.base import CLStrategy
 from mafed_b200.methods.distillation_loss_weights import DistillationWeights
 
@@ -315,19 +316,35 @@ class FeatureDistillation(CLStrategy):
         """Sum over the selected layers of ``layer_coeff * distillation_coeff * layer_loss``
         (``distillation.py:105-122``) -- as one fused launch instead of a Python loop."""
         layers = self.loss_weights.get_distillation_layers()
-        # the teacher's states come out of a no_grad forward and the node never differentiates them: the per-tensor
-        # `.detach()` of the reference (`_get_past_hidden_states`, distillation.py:223) is only paid for the distilled
-        # layers, and only if a tensor carries a graph at all
-        past_hidden_states = self._past_states(batch, layers)
         # Under torch.compile the host-only bookkeeping is skipped, so the step traces without a graph break: no
         # re-aiming of `assumed_grad_out` (the gate still keeps the gradients exact), no counts ticket (the kernel
         # exchanges the counts itself), no exchange check and no W&B queue -- `record_step()` does the last two eagerly.
         compiling = torch.compiler.is_compiling()
+        cached = None
+        if self.teacher_cache and not compiling:
+            # the cached teacher rows of this batch: read straight from the cache by the step where it takes them,
+            # otherwise gathered (as _past_states does)
+            batch.pop("labels", None)
+            cached = self._cache_step(batch, layers)
+            past_hidden_states = None
+        else:
+            # the teacher's states come out of a no_grad forward and the node never differentiates them: the
+            # per-tensor `.detach()` of the reference (`_get_past_hidden_states`, distillation.py:223) is only paid for
+            # the distilled layers, and only if a tensor carries a graph at all
+            past_hidden_states = self._past_states(batch, layers)
         if self.adapt_assumed_grad_out and self._gout_seen_np is not None and not compiling:
             self._adapt_assumed()
         plan = self._step_plan(layers)
         hidden = output.hidden_states
-        total, aux = self._launch(plan, batch, [hidden[l] for l in layers], past_hidden_states, teachers_detached=True)
+        students = [hidden[l] for l in layers]
+        result = None
+        if cached is not None:
+            result = self._launch_cached(plan, batch, students, *cached)
+            if result is None:
+                cache, idx, T = cached
+                past_hidden_states = cache.gather(idx, T, layers)
+        total, aux = result if result is not None else self._launch(plan, batch, students, past_hidden_states,
+                                                                    teachers_detached=True)
         if compiling:
             # `self.step` is advanced by record_step(): an int attribute changed inside the trace would be guarded on,
             # and every step would retrace (or feed a new int to the graph, which CUDA-graph trees re-record for)
@@ -434,6 +451,32 @@ class FeatureDistillation(CLStrategy):
             batch["lang_masks"], batch["image_masks"] = masks
         return total, aux
 
+    def _launch_cached(self, plan: DistillPlan, batch, students, cache, idx, T):
+        """The step with the teacher rows read straight from a replicated teacher cache (``cached_distill_loss``), or
+        ``None`` (nothing launched) where the gather + step takes it: a sharded cache, a step across ranks, the
+        two-pass form, CLS, or a launch ``libmafed_cached_step.so`` does not take."""
+        from mafed_b200 import teacher_cache
+        if (not isinstance(cache, teacher_cache.TeacherCache) or resolve_group(self.process_group)[0] or
+                not plan.single_pass or plan.cls):
+            return None
+        states, idx, T, T_c = cache.step_inputs(idx, T, plan.layers)
+        attn, mask_out = batch["attention_mask"], None
+        if self.populate_batch_masks and attn.is_cuda and attn.dtype == torch.int64 and attn.is_contiguous():
+            mask_out = True
+        if self._gout_seen is None:
+            self._gout_seen = seen_slot()
+            self._gout_seen_np = self._gout_seen.numpy()
+        res = cached_distill_loss(students, states, idx, T_c, attn, plan, mask_out=mask_out, seen=self._gout_seen,
+                                  return_masks=True)
+        if res is None:
+            return None
+        total, aux, masks = res
+        if masks is not None:
+            batch["lang_masks"], batch["image_masks"] = masks
+        elif self.populate_batch_masks:
+            batch["lang_masks"], batch["image_masks"] = modality_masks(attn, self.num_vision_tokens)
+        return total, aux
+
     def _teacher_forward(self, batch):
         """Autocast region of the teacher forward.  A snapshot held in ``teacher_dtype`` runs under an autocast of that
         dtype: inside replay's bf16 region an fp16 snapshot would otherwise get bf16 out of its linears next to fp16 out
@@ -476,6 +519,12 @@ class FeatureDistillation(CLStrategy):
     def _cached_past_states(self, batch, layers):
         """``teacher_cache``: the distilled layers' teacher states of the batch ``replay()`` drew, gathered from the cache
         (built here if ``load_state_dict`` left none) -- no teacher forward."""
+        cache, idx, T = self._cache_step(batch, layers)
+        return cache.gather(idx, T, layers)
+
+    def _cache_step(self, batch, layers):
+        """``(cache, memory indices, T)`` of the batch ``replay()`` drew: takes its ``memory_index`` and builds the cache
+        if ``load_state_dict`` left none."""
         idx, self._memory_index = self._memory_index, None
         if idx is None:
             raise cabi.MafedDistillError(
@@ -485,7 +534,7 @@ class FeatureDistillation(CLStrategy):
             if self.past_model is None:
                 raise cabi.MafedDistillError("teacher_cache: there is no teacher (past_model) to build the cache from")
             self._build_teacher_cache()
-        return self._teacher_cache.gather(idx, batch["attention_mask"].shape[1] + self.num_vision_tokens, layers)
+        return self._teacher_cache, idx, batch["attention_mask"].shape[1] + self.num_vision_tokens
 
     def _build_teacher_cache(self):
         from mafed_b200 import teacher_cache

@@ -18,6 +18,8 @@ EXT_NAME = "mafed_torch_node"
 EXT_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib",
                         EXT_NAME + (sysconfig.get_config_var("EXT_SUFFIX") or ".so"))
 
+CACHED_LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib", "libmafed_cached_step.so")
+
 _ext = None
 _lock = threading.Lock()
 
@@ -44,3 +46,16 @@ def load():
         ops.register()      # fake implementations and autograd of the mafed:: ops the extension defines
         _ext = mod
     return _ext
+
+
+def load_cached():
+    """The extension with ``libmafed_cached_step.so`` bound as well (the step that reads the teacher straight from the
+    teacher cache); bound on first use, raise if the library is absent."""
+    ext = load()
+    if not ext.cached_bound():
+        with _lock:
+            if not ext.cached_bound():
+                if not os.path.exists(CACHED_LIB_PATH):
+                    raise cabi.MafedDistillError(f"{CACHED_LIB_PATH} not found: build it with `python -m mafed_b200.build`")
+                ext.bind_cached(CACHED_LIB_PATH)
+    return ext

@@ -4,7 +4,9 @@ The teacher (``past_model``) and the memory are both fixed for a task, and every
 memory, so the teacher forward of a replay step recomputes hidden states it has computed before.  ``build`` runs the
 teacher once per task over the whole memory and keeps, per distilled layer, one ``[M, T_c, D]`` tensor; a replay step
 then gathers its samples' rows from it (``TeacherCache.gather``: one launch of ``libmafed_teacher_gather.so`` per dtype
-of the cached layers, ``include/mafed_teacher_gather.h``) instead of running the teacher.
+of the cached layers, ``include/mafed_teacher_gather.h``) instead of running the teacher -- or, where the one-pass step
+takes the shape, has the step's kernels read the rows straight from the cache (``TeacherCache.step_inputs``,
+``libmafed_cached_step.so``, ``include/mafed_cached_step.h``), with no gathered copy at all.
 
 Layout: ``T_c = n_vis + the longest text of the memory set``; every sample is computed with its text left-padded to
 that length, as the collate pads a batch.  A batch at length ``T <= T_c`` takes the visual rows ``t < n_vis`` from the
@@ -114,10 +116,8 @@ def gather_sharded_raw(out_ptrs, bases, layer_off, src_rank, slot, B, slots, T, 
     _check(rc, "mafed_teacher_gather_sharded")
 
 
-def gather(cache: Sequence[torch.Tensor], idx: Sequence[int], T: int, n_vis: int) -> List[torch.Tensor]:
-    """``[B, T, D]`` teacher states of the memory samples ``idx`` from ``[M, T_c, D]`` cache tensors (one kernel launch
-    per dtype among them), stream-ordered on the current stream."""
-    M, T_c, D = cache[0].shape
+def _checked(idx: Sequence[int], T: int, M: int, T_c: int, n_vis: int) -> List[int]:
+    """The memory indices of a step as ints, after the range and length checks every read of the cache makes."""
     idx = [int(i) for i in idx]
     bad = [i for i in idx if not 0 <= i < M]
     if bad:
@@ -125,6 +125,14 @@ def gather(cache: Sequence[torch.Tensor], idx: Sequence[int], T: int, n_vis: int
     if not n_vis <= T <= T_c:
         raise MafedDistillError(f"a batch of {T} tokens does not fit the teacher cache (n_vis = {n_vis}, T_c = {T_c}): "
                                 "the memory set changed since the cache was built")
+    return idx
+
+
+def gather(cache: Sequence[torch.Tensor], idx: Sequence[int], T: int, n_vis: int) -> List[torch.Tensor]:
+    """``[B, T, D]`` teacher states of the memory samples ``idx`` from ``[M, T_c, D]`` cache tensors (one kernel launch
+    per dtype among them), stream-ordered on the current stream."""
+    M, T_c, D = cache[0].shape
+    idx = _checked(idx, T, M, T_c, n_vis)
     out = [torch.empty((len(idx), T, D), dtype=c.dtype, device=c.device) for c in cache]
     stream = torch.cuda.current_stream(cache[0].device).cuda_stream
     for dtype in dict.fromkeys(c.dtype for c in cache):
@@ -204,6 +212,13 @@ class TeacherCache:
         if list(layers) != self.layers:
             raise MafedDistillError(f"the teacher cache holds layers {self.layers}, the step distils {list(layers)}")
         return gather(self.states, idx, T, self.n_vis)
+
+    def step_inputs(self, idx: Sequence[int], T: int, layers: Sequence[int]):
+        """What a step that reads the teacher rows straight from the cache needs instead of ``gather``'s tensors:
+        ``(states, idx, T, T_c)`` with ``idx`` checked as ``gather`` checks it (``distill_op.cached_distill_loss``)."""
+        if list(layers) != self.layers:
+            raise MafedDistillError(f"the teacher cache holds layers {self.layers}, the step distils {list(layers)}")
+        return self.states, _checked(idx, T, self.states[0].shape[0], self.T_c, self.n_vis), T, self.T_c
 
 
 def _build_batches(strategy):
